@@ -2,6 +2,7 @@
 """bench.py -- warped images/s of the attention-guided warp hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c4|c5] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input:
   c2 (default; BASELINE.json configs[1]): 256 x 336^2 RGB uint8 + bf16 attention
@@ -20,6 +21,9 @@ checksums.  Rank 0 prints ONE JSON line.
             HBM copy peak (MEASURED_PEAKS.json).
 `cpu_baseline`: the oracle port of the reference CPU path on this box's host cores (bounded sample).
 `--impl reference`: only the CPU arm, same metric/config, `"impl": "reference"`.
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the last timed step of each workload returned to
+            its caller as DIR/<workload>_<array>.npy (float32; a fixed, seeded sample of the elements of an array
+            larger than DUMP_ELEMENTS).  Inputs are seeded, so two builds can be compared output for output.
 """
 
 from __future__ import annotations
@@ -102,6 +106,45 @@ def ncu_traffic(kernel, workload):
             return json.load(f).get(workload, {}).get(kernel)
     except Exception:
         return None
+
+
+# ------------------------------------------------------------------------------------------
+# --dump-outputs
+# ------------------------------------------------------------------------------------------
+DUMP_ELEMENTS = 4_000_000          # per array: 16 MB of float32; a run of all workloads writes < 64 MB
+DUMP_BYTES_MAX = 64 * 10**6
+
+
+def dump_sample(tensors, n=DUMP_ELEMENTS, seed=0):
+    """float32 host copy of the elements of `tensors` (flattened and concatenated in order): all of them when
+    there are at most n, else n of them at sorted positions drawn with a fixed seed (the same positions in every
+    run of the same workload, whatever the build)."""
+    import numpy as np
+    import torch
+    sizes = [t.numel() for t in tensors]
+    total = sum(sizes)
+    if total <= n:
+        return torch.cat([t.reshape(-1).float() for t in tensors]).cpu().numpy()
+    idx = np.sort(np.random.default_rng(seed).integers(0, total, n))
+    starts = np.cumsum([0] + sizes)
+    parts = []
+    for t, lo, hi, start in zip(tensors, np.searchsorted(idx, starts[:-1]), np.searchsorted(idx, starts[1:]),
+                                starts[:-1]):
+        if hi > lo:
+            parts.append(t.reshape(-1)[torch.from_numpy(idx[lo:hi] - start).to(t.device)].float())
+    return torch.cat(parts).cpu().numpy()
+
+
+def write_dumps(path, dumps):
+    """dumps: {workload: {array name: float32 ndarray}} -> path/<workload>_<array>.npy"""
+    import numpy as np
+    total = sum(a.nbytes for d in dumps.values() for a in d.values())
+    if total > DUMP_BYTES_MAX:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed {DUMP_BYTES_MAX}")
+    os.makedirs(path, exist_ok=True)
+    for wl_key, d in dumps.items():
+        for name, a in d.items():
+            np.save(os.path.join(path, f"{wl_key}_{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------
@@ -532,23 +575,24 @@ def bench_uniform(ctx, wl_key, with_clocks=True):
     if rank == 0 and with_clocks:
         sampler.start()
     elapsed_ms, launches = timed_steps(ctx, step, args.steps, args.warmup, fork, join)
-    # the same steps again, for >= 120 ms: the contract's K steps last a couple of milliseconds, too short for more
-    # than one NVML clock sample; this region reports the sustained rate and gives the sampler its samples
-    sus_steps = int(min(max(args.steps, 0.12e3 / max(elapsed_ms / args.steps, 1e-3)), 4000))
-    sus_ms, _ = timed_steps(ctx, step, sus_steps, args.warmup + args.steps, fork, join)
     clocks = sampler.stop() if (rank == 0 and with_clocks) else None
     lib.attwarp_set_sm_share(1)
 
-    n_done = args.warmup + args.steps + sus_steps
-    chk = sharding.checksum64(sets[(n_done - 1) % R]["out"][:8])
+    last = sets[(args.warmup + args.steps - 1) % R]
+    dump = None
+    if args.dump_outputs and rank == 0:
+        dump = {"out": dump_sample([last["out"]])}
+        if wl["has_attention"]:
+            dump["tokens"] = dump_sample([last["aux"][0]])
+        dump.update(map_x=dump_sample([last["aux"][1]]), map_y=dump_sample([last["aux"][2]]))
+    chk = sharding.checksum64(last["out"][:8])
     stats = sharding.gather_stats(elapsed_ms, B * args.steps, chk, dev)
-    sus_stats = sharding.gather_stats(sus_ms, B * sus_steps, 0, dev)
     value = sharding.aggregate_throughput(stats)
     worst_ms = max(s[0] for s in stats)
 
     # single-stream figure (one batch at a time: nothing of another step to overlap with)
-    one_ms, _ = timed_steps(ctx, lambda i: (run_step_single(i), launches_per_step)[1], max(args.steps, 20), 0)
-    one_stats = sharding.gather_stats(one_ms, B * max(args.steps, 20), 0, dev)
+    one_ms, _ = timed_steps(ctx, lambda i: (run_step_single(i), launches_per_step)[1], args.steps, 0)
+    one_stats = sharding.gather_stats(one_ms, B * args.steps, 0, dev)
 
     # ---- per-kernel durations, outside the timed region ---------------------------------------------
     # each kernel alone, launched back to back over the rotating sets (the launch of kernel n+1 overlaps
@@ -639,7 +683,7 @@ def bench_uniform(ctx, wl_key, with_clocks=True):
             pipe = HostTokenPipeline(chunk, (grid, grid), (side, side, C), device=dev)
             api = "attwarp_b200.batched.HostTokenPipeline.run (pinned host in/out)"
         probe = HostCopyProbe(pipe)
-        ke = max(3, min(args.steps, 10))
+        ke = args.steps
 
         def time_e2e(fn):
             for _ in range(2):
@@ -696,10 +740,8 @@ def bench_uniform(ctx, wl_key, with_clocks=True):
 
     res = {"value": value, "ms_per_step": worst_ms / args.steps, "per_rank_ms": [s[0] for s in stats],
            "launches": launches * world, "kernels": kernels, "roofline": roofline, "e2e": e2e, "clocks": clocks,
-           "driver_flow": driver_flow,
-           "sustained": {"steps": sus_steps, "ms_per_step": max(s[0] for s in sus_stats) / sus_steps,
-                         "value": sharding.aggregate_throughput(sus_stats)},
-           "single_stream": {"ms_per_step": max(s[0] for s in one_stats) / max(args.steps, 20),
+           "driver_flow": driver_flow, "dump": dump,
+           "single_stream": {"ms_per_step": max(s[0] for s in one_stats) / args.steps,
                              "value": sharding.aggregate_throughput(one_stats),
                              "note": "one batch at a time on one stream (no overlap between steps)"},
            "run": {"rotate": R, "streams": n_streams, "sm_share": sm_share,
@@ -760,6 +802,7 @@ def bench_ragged(ctx):
     for i in range(args.warmup):
         step(i)
     elapsed_ms, launches = timed_steps(ctx, step, steps, 0)
+    dump = {"out": dump_sample(outs)} if args.dump_outputs and rank == 0 else None
     stats = sharding.gather_stats(elapsed_ms, len(mine) * steps, 0, dev)
     bstats = sharding.gather_stats(elapsed_ms, my_bytes // 1024, 0, dev)
     value = sharding.aggregate_throughput(stats)
@@ -803,7 +846,7 @@ def bench_ragged(ctx):
                         "achieved": gbs, "peak": ctx.peak, "unit": "GB/s", "frac": gbs / ctx.peak, "traffic": None,
                         "peak_source": ctx.peak_src, "algorithmic_bytes_per_launch": total_bytes // world,
                         "note": "per GPU: the slowest rank's step time over its share of the bytes"},
-           "check": check, "e2e": None,
+           "check": check, "e2e": None, "dump": dump,
            "run": {"launch": "one maps launch + one resample launch per class of images (grouped by the consumer warps "
                              "their strips need, 3..16, and by whether their rows are 4-byte aligned; classes fan out "
                              "over three streams) per step over the rank's shard; descriptor table planned once per "
@@ -866,11 +909,11 @@ def bench_pdf(ctx):
     if rank == 0:
         sampler.start()
     elapsed_ms, launches = timed_steps(ctx, step, args.steps, args.warmup, fork, join)
-    sus_steps = int(min(max(args.steps, 0.12e3 / max(elapsed_ms / args.steps, 1e-3)), 2000))
-    sus_ms, _ = timed_steps(ctx, step, sus_steps, args.warmup + args.steps, fork, join)
     clocks = sampler.stop() if rank == 0 else None
+    dump = None
+    if args.dump_outputs and rank == 0:
+        dump = {"out": dump_sample([sets[(args.warmup + args.steps - 1) % R]["out"]])}
     stats = sharding.gather_stats(elapsed_ms, B * args.steps, 0, dev)
-    sus_stats = sharding.gather_stats(sus_ms, B * sus_steps, 0, dev)
     value = sharding.aggregate_throughput(stats)
     worst_ms = max(s[0] for s in stats)
     by = B * C * side * side * 4 * 2
@@ -902,9 +945,7 @@ def bench_pdf(ctx):
                                                           "maps": "maps of rand^3 24x24 token grids"}}
     hard = max(kernels, key=lambda k: kernels[k]["ms"])
     res = {"value": value, "ms_per_step": worst_ms / args.steps, "per_rank_ms": [s[0] for s in stats],
-           "launches": launches * world, "kernels": kernels, "clocks": clocks, "e2e": None,
-           "sustained": {"steps": sus_steps, "ms_per_step": max(s[0] for s in sus_stats) / sus_steps,
-                         "value": sharding.aggregate_throughput(sus_stats)},
+           "launches": launches * world, "kernels": kernels, "clocks": clocks, "e2e": None, "dump": dump,
            "roofline": {"bound": "hbm", "kernel": "remap_f32_stream_kernel", "achieved": kernels[hard]["achieved_gbs"],
                         "peak": ctx.peak, "unit": "GB/s", "frac": kernels[hard]["frac"],
                         "traffic": ncu_traffic("remap_f32_stream_kernel", "c5"), "peak_source": ctx.peak_src,
@@ -936,15 +977,17 @@ def run_gpu(args, rank, local_rank, world):
         head = bench_pdf(ctx)
     else:
         head = bench_uniform(ctx, head_key)
+    dumps = {head_key: head["dump"]}
     extra = {}
     if args.workload == "all":
         for key in ("c3", "c4"):
             r = bench_uniform(ctx, key, with_clocks=False) if key == "c3" else bench_ragged(ctx)
+            dumps[key] = r["dump"]
             entry = {"metric": METRIC, "unit": UNIT, "value": r["value"], "ms_per_step": r["ms_per_step"],
                      "scaling": "strong" if key == "c4" else "weak", "dtype": DTYPES[key],
                      "config": workload_config(key, world), "roofline": r["roofline"], "e2e": r["e2e"],
                      "per_rank_ms": r["per_rank_ms"], "gpu_launches": r["launches"], "run": r["run"]}
-            for k in ("kernels", "sustained", "single_stream", "driver_flow", "images_per_rank", "shard_imbalance", "check", "steps"):
+            for k in ("kernels", "single_stream", "driver_flow", "images_per_rank", "shard_imbalance", "check", "steps"):
                 if k in r:
                     entry[k] = r[k]
             extra[key] = entry
@@ -953,13 +996,15 @@ def run_gpu(args, rank, local_rank, world):
         dist.destroy_process_group()
     if rank != 0:
         return 0
+    if args.dump_outputs:
+        write_dumps(args.dump_outputs, dumps)
     line = {"metric": METRIC, "value": head["value"], "unit": UNIT, "n_gpus": world,
             "steps": head.get("steps", args.steps), "warmup": args.warmup, "ms_per_step": head["ms_per_step"],
             "higher_is_better": True, "scaling": "strong" if wl.get("ragged") else "weak", "vs_baseline": None,
             "dtype": DTYPES[head_key], "data": "synthetic", "config": workload_config(head_key, world),
             "run": head["run"], "clocks": head.get("clocks"), "e2e": head["e2e"], "gpu_launches": head["launches"],
             "roofline": head["roofline"], "cpu_baseline": cpu_info, "per_rank_ms": head["per_rank_ms"]}
-    for k in ("kernels", "sustained", "single_stream", "driver_flow", "images_per_rank", "shard_imbalance", "check"):
+    for k in ("kernels", "single_stream", "driver_flow", "images_per_rank", "shard_imbalance", "check"):
         if k in head:
             line[k] = head[k]
     if extra:
@@ -981,15 +1026,19 @@ def main():
     ap.add_argument("--streams", type=int, default=0, help="CUDA streams consecutive steps alternate over (default 4 with attention, else 3)")
     ap.add_argument("--sm-share", type=int, default=0, help="attwarp_set_sm_share for the overlapped steps (default 2 with attention and several streams, else 1)")
     ap.add_argument("--e2e-chunk", type=int, default=0, help="images per host-pipeline chunk (default 64 at 336^2, 16 at 1344^2)")
-    ap.add_argument("--c4-steps", type=int, default=0, help="steps of the c4 workload (default: min(--steps, 10))")
+    ap.add_argument("--c4-steps", type=int, default=0, help="steps of the c4 workload (default: --steps)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch the kernels eagerly instead of by graph replay")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step returned as DIR/<workload>_<array>.npy")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 10 if args.workload == "c4" else 200
-    if args.c4_steps <= 0:
-        args.c4_steps = min(args.steps, 10)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm; --impl reference has none")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
     # stdout carries the ONE JSON line and nothing else: NCCL's own logging (its version banner, NCCL_DEBUG

@@ -1,5 +1,6 @@
 """CPU: the host-side pieces of bench.py that do not need a GPU -- workload table, the stdout guard used
-around NCCL initialisation, and the clock sampler degrading to None when neither NVML nor nvidia-smi exists."""
+around NCCL initialisation, the --dump-outputs sampler, and the clock sampler degrading to None when neither
+NVML nor nvidia-smi exists."""
 
 import importlib.util
 import os
@@ -38,6 +39,22 @@ def test_stdout_guard_sends_library_output_to_stderr():
     assert r.returncode == 0, r.stderr
     assert r.stdout.split() == ["line-1", "line-2"]
     assert "banner from a C library" in r.stderr
+
+
+def test_dump_sample_is_a_fixed_sample_of_the_concatenated_outputs(tmp_path):
+    import numpy as np
+    import torch
+    b = _bench()
+    g = torch.Generator().manual_seed(0)
+    ts = [torch.randint(0, 256, (s, s + 1, 3), dtype=torch.uint8, generator=g) for s in (3, 40, 7)]
+    flat = np.concatenate([t.numpy().reshape(-1) for t in ts]).astype(np.float32)
+    assert np.array_equal(b.dump_sample(ts, flat.size), flat)
+    got = b.dump_sample(ts, 500)
+    assert got.dtype == np.float32 and got.size == 500
+    assert np.array_equal(got, b.dump_sample(ts, 500))                  # the same positions in every run
+    assert np.array_equal(got, flat[np.sort(np.random.default_rng(0).integers(0, flat.size, 500))])
+    b.write_dumps(str(tmp_path), {"c4": {"out": got}})
+    assert np.array_equal(np.load(tmp_path / "c4_out.npy"), got)
 
 
 def test_clock_sampler_without_a_gpu_is_none_not_an_error():

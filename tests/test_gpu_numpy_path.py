@@ -102,7 +102,7 @@ def test_large_image_end_to_end_vs_oracle():
         assert diff.max() <= 1 and (diff != 0).mean() <= 1e-3
 
 
-def test_error_behaviour():
+def test_error_behaviour(tmp_path):
     need_gpu()
     from attwarp_b200 import new_method
     img = np.zeros((8, 9, 3), np.uint8)
@@ -111,8 +111,9 @@ def test_error_behaviour():
     with pytest.raises(TypeError):
         new_method.warp_image_by_attention(img.astype(np.int32), np.zeros((8, 9)), 9, 8)
     assert new_method.set_transform_function("nope") == "identity"
-    assert new_method.save_warped_image("/nonexistent.png", np.zeros((4, 4)), None, None,
-                                        "/tmp/x.png") is False
+    out = tmp_path / "x.png"
+    assert new_method.save_warped_image("/nonexistent.png", np.zeros((4, 4)), None, None, str(out)) is False
+    assert not out.exists()
 
 
 @pytest.mark.parametrize("H,W", [(1, 16), (63, 336), (64, 336), (65, 1024), (200, 1040), (130, 1344), (70, 2064)])
