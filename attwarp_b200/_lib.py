@@ -76,7 +76,10 @@ SIGNATURES = {
     "attwarp_ragged_workspace_bytes": (_sz, [_vp, _i]),
     "attwarp_ragged_last_launches": (_i, []),
     "attwarp_warp_ragged_from_tokens": (_i, [_vp, _i, _i, _i, _vp, _i, _tp, _vp, _sz, _vp]),
-    "attwarp_warp_image_host": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _i, _i, _tp, _vp,
+    "attwarp_png_max_bytes": (_sz, [_i, _i, _i]),
+    "attwarp_png_workspace_bytes": (_sz, [_vp, _i]),
+    "attwarp_encode_png": (_i, [_vp, _i, _vp, _sz, _vp, _sz, _vp, _vp]),
+    "attwarp_warp_image_host":(_i, [_vp, _i, _i, _i, _i, _vp, _i, _i, _i, _tp, _vp,
                                      C.POINTER(_i)]),
     "attwarp_safe_softmax": (_i, [_vp, _i, _i, _f, _vp, _vp]),
     "attwarp_mix_with_uniform": (_i, [_vp, _i, _i, _f, _vp, _vp]),

@@ -38,6 +38,10 @@ int launch_maps_from_mask(const uint8_t* mask, int B, int h, int w, int H, int W
                           const attwarp_transform_params& tp, void* ws, size_t ws_bytes, float* map_x, float* map_y,
                           cudaStream_t st);
 int launch_strictly_increasing(const float* F, int B, int N, float eps, float* out, cudaStream_t st);
+size_t png_max_bytes_impl(int H, int W, int C);
+size_t png_workspace_bytes_impl(const attwarp_png_image* images, int n);
+int launch_encode_png(const attwarp_png_image* images, int n, void* ws, uint8_t* out, int64_t* offsets,
+                      cudaStream_t st);
 int launch_interp_linear_rows(const float* F, int B, int N, int L, float* out, cudaStream_t st);
 
 static thread_local char g_err[512] = "";
@@ -441,6 +445,44 @@ int attwarp_warp_ragged_from_tokens(const float* tok, int n, int gh, int gw,
 }
 
 int attwarp_ragged_last_launches(void) { return g_ragged_last_launches; }
+
+// ---------------------------------------------------------------------------------------------
+static bool png_shape_ok(int H, int W, int C) {
+    return H > 0 && W > 0 && (C == 1 || C == 3 || C == 4) && (int64_t)W * C < ((int64_t)1 << 30);
+}
+
+size_t attwarp_png_max_bytes(int H, int W, int C) { return png_shape_ok(H, W, C) ? png_max_bytes_impl(H, W, C) : 0; }
+
+size_t attwarp_png_workspace_bytes(const attwarp_png_image* images, int n) {
+    if (images == nullptr || n <= 0) return 0;
+    for (int i = 0; i < n; ++i)
+        if (!png_shape_ok(images[i].H, images[i].W, images[i].C)) return 0;
+    return png_workspace_bytes_impl(images, n);
+}
+
+int attwarp_encode_png(const attwarp_png_image* images, int n, void* workspace, size_t workspace_bytes, void* out,
+                       size_t out_capacity, int64_t* offsets, void* stream) {
+    AW_REQUIRE(images && out && offsets, "encode_png: NULL pointer");
+    AW_REQUIRE(n > 0, "encode_png: n must be positive (got %d)", n);
+    size_t need_out = 0;
+    for (int i = 0; i < n; ++i) {
+        const attwarp_png_image& im = images[i];
+        AW_REQUIRE(im.src, "encode_png: image %d: NULL pointer", i);
+        AW_REQUIRE(im.C == 1 || im.C == 3 || im.C == 4, "encode_png: image %d: C must be 1, 3 or 4 (got %d)", i, im.C);
+        AW_REQUIRE(png_shape_ok(im.H, im.W, im.C), "encode_png: image %d: sizes must be positive and W*C below 2^30", i);
+        need_out += png_max_bytes_impl(im.H, im.W, im.C);
+    }
+    AW_REQUIRE(out_capacity >= need_out, "encode_png: output buffer too small (%zu < %zu)", out_capacity, need_out);
+    const size_t need = png_workspace_bytes_impl(images, n);
+    if (workspace == nullptr || workspace_bytes < need)
+        return fail(ATTWARP_ERR_WORKSPACE, "encode_png: workspace too small (%zu < %zu)", workspace_bytes, need);
+    cudaStream_t st = as_stream(stream);
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    AW_CUDA(cudaStreamIsCapturing(st, &cap));
+    if (cap != cudaStreamCaptureStatusNone)
+        return fail(ATTWARP_ERR_UNSUPPORTED, "encode_png: cannot be captured into a CUDA graph (host-side descriptor table)");
+    return launch_encode_png(images, n, workspace, static_cast<uint8_t*>(out), offsets, st);
+}
 
 static int warp_image_host_impl(const void* image_host, int img_dtype, int C, int H, int W,
                                 const void* att_host, int att_dtype, int Wo, int Ho,

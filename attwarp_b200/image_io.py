@@ -15,9 +15,23 @@ batches the rest:
   reproduce the reference's pixels.  Anything that is not a JPEG (PNG, ...) is decoded on the host, exactly.
 * ``encode_png_batch(images, paths)`` device tensors -> PNG files: device -> pinned host copy, then
   ``cv2.imwrite`` in a thread pool -- the reference's own encoder, so the files decode to the same bytes.
-  (A GPU PNG/deflate encoder is out of scope until its output is pinned; PNG is lossless, so only speed is at stake.)
+  ``on_device=True`` encodes on the GPU instead (``encode_png_device``, ``ops.encode_png``: two launches for the
+  whole mixed-size list) and only the compressed bytes cross PCIe.  Like ``decode_jpeg_batch(exact=...)`` the
+  keyword trades byte identity for speed, here of the FILE bytes only: PNG is lossless and the pixels are the
+  same.  What the device encoder's files satisfy:
+    1. ``cv2.imdecode(buf, cv2.IMREAD_UNCHANGED)`` returns the input array exactly (Pillow: the same pixels in
+       RGB(A) order): HWC BGR is stored as RGB (colour type 2), BGRA as RGBA (6), [H, W] / [H, W, 1] as grey (0);
+       bit depth 8, no interlace -- the IHDR cv2.imencode writes.
+    2. Signature, IHDR, IDAT chunks, IEND with a correct CRC-32 each; the IDAT payloads are one zlib stream
+       (78 01, deflate blocks, Adler-32) of the filtered scanlines.
+    3. A file's bytes depend only on its pixels (not on the batch, the position in it, the stream or the run).
+    4. Sizes: every row Sub-filtered, like cv2 4.13; the stream cut into 32 KiB segments, each one deflate block of
+       distance-1 matches (zlib's Z_RLE, what cv2 evidently uses at level 1) under its own dynamic Huffman code, or
+       stored when that is not smaller.  Measured on the CPU with the encoder's own block builder against
+       cv2.imencode 4.13: 0.998x on photo-like, 1.000-1.003x on smooth gradients, 0.999x on noise (336^2, 500^2,
+       1344^2); noise never exceeds the stored size plus 17 bytes per 32 KiB and 75 bytes per file.
 * ``warp_files(...)``                the driver loop of main_batched.py:243-287 for a whole list of files: decode
-  -> one ragged launch per stage -> encode.
+  -> one ragged launch per stage -> encode (``on_device_png=True``: the device encoder above).
 """
 
 from __future__ import annotations
@@ -76,12 +90,42 @@ def decode_jpeg_batch(sources: Sequence, device=None, exact: bool = False) -> Li
     return out  # type: ignore[return-value]
 
 
-def encode_png_batch(images: Sequence[torch.Tensor], paths: Sequence[str], workers: int = 8) -> List[bool]:
+def encode_png_device(images) -> List[bytes]:
+    """uint8 device images ([H, W] or [H, W, C], C in {1, 3, 4}, mixed shapes; or a [B, H, W, C] tensor) -> the
+    bytes of their PNG files, encoded on the GPU (``ops.encode_png``).  The offsets come to the host first, then
+    the files in one copy to pinned memory; blocks until they are there."""
+    payload, offsets = ops.encode_png(images)
+    offs = offsets.cpu().tolist()                    # synchronises: the encode has run
+    total = offs[-1]
+    host = torch.empty(total, dtype=torch.uint8, pin_memory=True)
+    if total:
+        host.copy_(payload[:total], non_blocking=True)
+        torch.cuda.current_stream(payload.device).synchronize()
+    buf = host.numpy()
+    return [buf[offs[k]:offs[k + 1]].tobytes() for k in range(len(offs) - 1)]
+
+
+def _write_file(path, data: bytes) -> bool:
+    try:
+        with open(os.fspath(path), "wb") as f:
+            f.write(data)
+        return True
+    except OSError:
+        return False
+
+
+def encode_png_batch(images: Sequence[torch.Tensor], paths: Sequence[str], workers: int = 8,
+                     on_device: bool = False) -> List[bool]:
     """uint8 [H, W, 3] (BGR) or [H, W] device tensors -> PNG files with ``cv2.imwrite`` (the reference's encoder,
     new_method.py:491).  The device -> host copies are enqueued first (pinned staging), the encodes run in a
-    thread pool (OpenCV releases the GIL).  Returns cv2.imwrite's result per file."""
-    import cv2
+    thread pool (OpenCV releases the GIL).  Returns cv2.imwrite's result per file.
+    ``on_device=True``: the files are encoded on the GPU (``encode_png_device``; also [H, W, 1] and BGRA [H, W, 4])
+    and written with plain file writes; False for a file that cannot be written, like cv2.imwrite.  Same pixels,
+    different file bytes (module docstring)."""
     assert len(images) == len(paths)
+    if on_device:
+        return [_write_file(p, b) for p, b in zip(paths, encode_png_device(list(images)))]
+    import cv2
     host = []
     for t in images:
         h = torch.empty(t.shape, dtype=t.dtype, pin_memory=True)
@@ -101,7 +145,7 @@ def encode_png_batch(images: Sequence[torch.Tensor], paths: Sequence[str], worke
 
 def warp_files(image_sources: Sequence, tok: torch.Tensor, output_paths: Sequence[str], out_sizes=None,
                transform: str = "identity", exp_scale: float = 1.0, exp_divisor: float = 1.0,
-               apply_inverse: bool = False, device=None, workers: int = 8) -> List[bool]:
+               apply_inverse: bool = False, device=None, workers: int = 8, on_device_png: bool = False) -> List[bool]:
     """The per-image loop of the batched driver (main_batched.py:243-287: ``save_warped_image(image, mask, ...,
     width, height, "identity")`` per sample) for a list of image files and their token maps: GPU decode -> stages
     2-5 for the whole (mixed-resolution) list in one launch per stage -> PNG files.
@@ -111,11 +155,12 @@ def warp_files(image_sources: Sequence, tok: torch.Tensor, output_paths: Sequenc
                 sample's own size, main_batched.py:276-287)
     The attention the reference warps with in this flow is ``blend_mask``'s image-size uint8 mask; use
     ``ops.mota_mask`` + ``ops.maps_from_attention`` when that exact quantisation is wanted -- this entry point warps
-    with the token map index-upsampled on the fly (BASELINE configs[3])."""
+    with the token map index-upsampled on the fly (BASELINE configs[3]).
+    on_device_png  encode the files on the GPU (``encode_png_batch(on_device=True)``): same pixels, other bytes"""
     if len(image_sources) == 0:
         return []
     imgs = decode_jpeg_batch(image_sources, device)
     dev = imgs[0].device
     outs = ops.warp_ragged_from_tokens(tok.to(dev), imgs, out_sizes, transform=transform, exp_scale=exp_scale,
                                        exp_divisor=exp_divisor, apply_inverse=apply_inverse)
-    return encode_png_batch(outs, output_paths, workers)
+    return encode_png_batch(outs, output_paths, workers, on_device=on_device_png)

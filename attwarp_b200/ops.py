@@ -507,3 +507,58 @@ class RaggedBatch:
                                                       ptr(self._ws), self._ws.numel(), current_stream(self.device)))
             self.launches = int(lib.attwarp_ragged_last_launches())      # kernels this call enqueued
         return self.outs
+
+
+# --------------------------------------------------------------------------------------------
+# PNG encode (the warped images' way to disk)
+# --------------------------------------------------------------------------------------------
+# attwarp_png_image (include/attwarp.h)
+_PNG_DTYPE = np.dtype([("src", np.uint64), ("H", np.int32), ("W", np.int32), ("C", np.int32), ("pad", np.int32)])
+
+
+def encode_png(images):
+    """PNG files of n uint8 device images of any shapes, in two launches on the current stream (nothing
+    synchronises).
+
+    images  a sequence of uint8 CUDA tensors [H, W] or [H, W, C] with C in {1, 3, 4} -- channel order as
+            cv2.imwrite takes it: BGR(A) is stored as RGB(A), one channel as grey -- or a [B, H, W, C] tensor
+    Returns (payload, offsets): uint8 [capacity] and int64 [n + 1] device tensors; file i is
+    payload[offsets[i]:offsets[i + 1]].  A file's bytes depend only on its image's pixels; they are not cv2's
+    bytes, the decoded pixels are the same (every row Sub-filtered, deflate of run-length matches in 32 KiB
+    segments, within a few per mille of cv2's sizes on photo-like, smooth and noise images)."""
+    lib = load()
+    if isinstance(images, torch.Tensor):
+        if images.dim() != 4:
+            raise ValueError(f"encode_png: a tensor argument must be [B, H, W, C], got {tuple(images.shape)}")
+        images = list(images.unbind(0))
+    elif not isinstance(images, (list, tuple)):
+        raise ValueError(f"encode_png: expected a sequence of image tensors or a [B, H, W, C] tensor, got {type(images)}")
+    imgs = []
+    for k, t in enumerate(images):
+        if (not isinstance(t, torch.Tensor) or t.dtype != torch.uint8 or not t.is_cuda or t.dim() not in (2, 3)
+                or (t.dim() == 3 and t.shape[2] not in (1, 3, 4)) or t.numel() == 0):
+            desc = f"{t.dtype} {tuple(t.shape)} on {t.device}" if isinstance(t, torch.Tensor) else type(t).__name__
+            raise ValueError(f"encode_png: image {k} must be a non-empty uint8 CUDA tensor [H, W] or [H, W, C] with "
+                             f"C in (1, 3, 4), got {desc}")
+        imgs.append(t.contiguous())
+    n = len(imgs)
+    dev = imgs[0].device if n else torch.device("cuda", torch.cuda.current_device())
+    if any(t.device != dev for t in imgs):
+        raise ValueError("encode_png: all images must be on one device")
+    if n == 0:
+        return torch.empty(0, dtype=torch.uint8, device=dev), torch.zeros(1, dtype=torch.int64, device=dev)
+    table = np.zeros(n, dtype=_PNG_DTYPE)
+    table["src"] = [t.data_ptr() for t in imgs]
+    table["H"] = [t.shape[0] for t in imgs]
+    table["W"] = [t.shape[1] for t in imgs]
+    table["C"] = [t.shape[2] if t.dim() == 3 else 1 for t in imgs]
+    table_p = table.ctypes.data_as(C.c_void_p)           # `table` stays alive until the call returns
+    cap = sum(int(lib.attwarp_png_max_bytes(int(h), int(w), int(c))) for h, w, c in zip(table["H"], table["W"], table["C"]))
+    payload = torch.empty(cap, dtype=torch.uint8, device=dev)
+    offsets = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    wsb = lib.attwarp_png_workspace_bytes(table_p, n)
+    ws = _workspace(wsb, dev)
+    with torch.cuda.device(dev):
+        check(lib.attwarp_encode_png(table_p, n, ptr(ws), ws.numel(), ptr(payload), cap, ptr(offsets),
+                                     current_stream(dev)))
+    return payload, offsets

@@ -262,6 +262,36 @@ int attwarp_warp_image_host(const void* image_host, int img_dtype, int C, int H,
                             const attwarp_transform_params* tp, void* out_host,
                             int* used_fallback);
 
+/* ---------------------------------------------------------------------------------------------
+ * PNG encode of n uint8 images of any shapes in two launches (the warped images' way to disk;
+ * the reference writes each with cv2.imwrite, AGW/new_method.py:491).
+ *
+ * images : HOST array of n descriptors; src is a DEVICE pointer to a dense [H][W][C] uint8 image,
+ *          C = 1 (stored as grey), 3 (BGR, stored as RGB) or 4 (BGRA, stored as RGBA), as
+ *          cv2.imwrite stores them.  src must stay valid until the stream has run the call.
+ * Each file: signature, IHDR (bit depth 8, no interlace), IDAT chunks whose payloads are one zlib
+ * stream (78 01, deflate, Adler-32), IEND.  Every row has the Sub filter; the stream is coded in
+ * independent segments of 32 KiB (distance-1 matches under a dynamic Huffman code, or stored).
+ * A file's bytes depend only on its image's pixels.  The bytes differ from cv2's encoder; the
+ * decoded pixels are the same.
+ * attwarp_png_max_bytes       : the largest file an H x W x C image can give (host arithmetic)
+ * attwarp_png_workspace_bytes : device scratch one call over `images` needs
+ * out      : device buffer of out_capacity >= sum over images of attwarp_png_max_bytes bytes;
+ *            receives the files back to back
+ * offsets  : device int64 [n + 1]: file i is out[offsets[i] .. offsets[i + 1])
+ * The call uploads its descriptor table from host memory: ATTWARP_ERR_UNSUPPORTED on a stream
+ * that is being captured into a CUDA graph.
+ */
+typedef struct attwarp_png_image {
+    const void* src;
+    int32_t H, W, C;
+} attwarp_png_image;
+
+size_t attwarp_png_max_bytes(int H, int W, int C);
+size_t attwarp_png_workspace_bytes(const attwarp_png_image* images_host, int n);
+int attwarp_encode_png(const attwarp_png_image* images_host, int n, void* workspace, size_t workspace_bytes,
+                       void* out, size_t out_capacity, int64_t* offsets, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Stages 2-3, torch path (all float32 [B][N] row-major unless noted).
  */
