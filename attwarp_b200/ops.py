@@ -87,13 +87,40 @@ class GraphedCall:
 # --------------------------------------------------------------------------------------------
 # stage 1
 # --------------------------------------------------------------------------------------------
+def _token_window(name, tok_start, B, K, T, device):
+    """Check that every image's token window [start, start + T) lies inside its row of K tokens and return
+    ``tok_start`` as a contiguous int32 tensor on ``device`` (None stays None).  The kernels read the window
+    through raw pointers, so a window past the row reads another row, another image or past the tensor.
+    A CUDA ``tok_start`` is not copied back to be checked: only its length is, its values are the caller's."""
+    if T < 1:
+        raise ValueError(f"{name}: the token window must hold at least one token, got T={T}")
+    if tok_start is None:
+        if T > K:
+            raise ValueError(f"{name}: T={T} tokens requested from rows of K={K} (pass tok_start for a window)")
+        return None
+    starts = torch.as_tensor(tok_start)        # list / CPU tensor / CUDA tensor of per-sample offsets
+    if starts.numel() != B:
+        raise ValueError(f"{name}: tok_start holds {starts.numel()} values for a batch of {B}")
+    if not starts.is_cuda and B > 0:
+        lo, hi = int(starts.min()), int(starts.max())
+        if lo < 0 or hi > K - T:
+            raise ValueError(f"{name}: tok_start values in [{lo}, {hi}] put a window of T={T} tokens outside rows "
+                             f"of K={K} (each start must lie in [0, {K - T}])")
+    return starts.to(device=device, dtype=torch.int32).contiguous()
+
+
 def aggregate_attention(attn: torch.Tensor, tok_start: torch.Tensor | None = None,
                         num_tokens: int | None = None, out: torch.Tensor | None = None,
                         accumulate: bool = False, out_scale: float = 1.0,
                         eps: float = 1e-12) -> torch.Tensor:
     """attn [B, L, Hh, K] (bf16/fp16/fp32, last dim contiguous, other dims arbitrarily strided)
     -> float32 [B, T]:  mean over L and Hh of  a[..., st:st+T] / (sum + eps).
-    Reference: llava.py:94-132, 385-411 (L = hooked steps)."""
+    Reference: llava.py:94-132, 385-411 (L = hooked steps).
+
+    T is ``num_tokens`` (default K).  ``tok_start`` (B offsets) selects the window [st, st + T) of image b's
+    rows; without it T must not exceed K.  A list or CPU tensor of offsets is checked against [0, K - T]
+    (ValueError); a CUDA tensor is used as it is, and keeping its values in that range is the caller's
+    responsibility."""
     lib = load()
     require_cuda(attn, out)
     assert attn.dim() == 4, "attn must be [B, L, Hh, K]"
@@ -101,8 +128,7 @@ def aggregate_attention(attn: torch.Tensor, tok_start: torch.Tensor | None = Non
         raise ValueError("attention rows must be contiguous along the token axis")
     B, L, Hh, K = attn.shape
     T = K if num_tokens is None else int(num_tokens)
-    if tok_start is not None:          # list / CPU tensor / CUDA tensor of per-sample offsets
-        tok_start = torch.as_tensor(tok_start).to(device=attn.device, dtype=torch.int32).contiguous()
+    tok_start = _token_window("aggregate_attention", tok_start, B, K, T, attn.device)
     if out is None:
         out = torch.empty(B, T, dtype=torch.float32, device=attn.device)
         accumulate = False
@@ -292,17 +318,20 @@ def warp_from_attention_tokens(attn: torch.Tensor, images: torch.Tensor, grid_hw
                                return_aux: bool = False, aux: tuple | None = None,
                                stage_events=None):
     """Stages 1-5 for a uniform batch in one host call:
-    attn [B,L,Hh,K] -> token map [B,gh*gw] -> separable maps -> warped images."""
+    attn [B,L,Hh,K] -> token map [B,gh*gw] -> separable maps -> warped images.
+
+    Without ``tok_start`` K must equal gh*gw; with it, image b's tokens are [st_b, st_b + gh*gw) of its rows,
+    checked as in ``aggregate_attention`` (a CUDA ``tok_start`` is the caller's responsibility)."""
     lib = load()
     require_cuda(attn, images, out)
     assert attn.dim() == 4 and attn.stride(3) == 1
     images = images.contiguous()
     B, L, Hh, K = attn.shape
     gh, gw = grid_hw
-    if tok_start is None:
-        assert K == gh * gw, "attention row length must equal gh*gw unless tok_start is given"
-    else:
-        tok_start = torch.as_tensor(tok_start).to(device=attn.device, dtype=torch.int32).contiguous()
+    if tok_start is None and K != gh * gw:
+        raise ValueError(f"warp_from_attention_tokens: attention row length K={K} must equal gh*gw={gh * gw} "
+                         "unless tok_start is given")
+    tok_start = _token_window("warp_from_attention_tokens", tok_start, B, K, gh * gw, attn.device)
     if layout == "hwc":
         Bi, H, W, Cc = images.shape
         lay = LAYOUT_HWC
