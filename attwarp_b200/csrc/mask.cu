@@ -136,7 +136,9 @@ resize_lanczos_u8_kernel(const uint8_t* __restrict__ src, int h, int w, int Ho, 
 // horizontal pass held in registers as a sliding window (the window moves one source row every Ho / h
 // output rows); an output row is 8 x 4 IMAD with coefficients broadcast from shared memory, clip, one
 // 32-bit store.  Zero-padded coefficient rows make every output row an 8-tap row.
-constexpr int kUpTaps = 8;        // most taps per axis (coefficient rows in shared memory are padded to 8)
+// Pillow's window has 2 ceil(support) + 1 taps, always odd: an up-scaling has 7 per axis, never 8, so only the TAPS = 7
+// instances below are compiled.
+constexpr int kUpTaps = 8;        // coefficient rows in shared memory are padded to 8
 __device__ __forceinline__ void unpack4(uint32_t w, int* v) {
     v[0] = (int)(w & 0xffu); v[1] = (int)((w >> 8) & 0xffu); v[2] = (int)((w >> 16) & 0xffu); v[3] = (int)(w >> 24);
 }
@@ -729,8 +731,8 @@ int launch_lanczos_marginals(const uint8_t* src, int B, int h, int w, int H, int
     if (rc != ATTWARP_OK) return rc;
     rc = get_table(h, H, &ty);
     if (rc != ATTWARP_OK) return rc;
-    if (tx.ksize > kUpTaps || ty.ksize > kUpTaps) return fail(ATTWARP_ERR_UNSUPPORTED, "lanczos_marginals: too many taps");
-    auto kern = (tx.ksize <= 7 && ty.ksize <= 7) ? resize_lanczos_up_kernel<7, true> : resize_lanczos_up_kernel<8, true>;
+    if (tx.ksize > 7 || ty.ksize > 7) return fail(ATTWARP_ERR_UNSUPPORTED, "lanczos_marginals: too many taps");
+    auto kern = resize_lanczos_up_kernel<7, true>;
     if (ug.smem > 48 * 1024)
         AW_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ug.smem));
     kern<<<dim3(ug.n_tiles, B), ug.threads, ug.smem, st>>>(
@@ -764,10 +766,10 @@ int launch_resize_lanczos_u8(const uint8_t* src, int B, int h, int w, int Ho, in
             return check_launch("resize_lanczos_up_mma_kernel");
         }
     }
-    // up-scaling (or any resize with <= 8 taps per axis) of both axes: the register-window kernel
+    // up-scaling of both axes (7 taps each) the tensor-core kernel declined: the register-window kernel
     const UpGeometry ug = up_geometry(B, h, w, Ho, Wo);
-    if (Wo != w && Ho != h && tx.ksize <= kUpTaps && ty.ksize <= kUpTaps && ug.ok) {
-        auto kern = (tx.ksize <= 7 && ty.ksize <= 7) ? resize_lanczos_up_kernel<7, false> : resize_lanczos_up_kernel<8, false>;
+    if (Wo != w && Ho != h && tx.ksize <= 7 && ty.ksize <= 7 && ug.ok) {
+        auto kern = resize_lanczos_up_kernel<7, false>;
         if (ug.smem > 48 * 1024)
             AW_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ug.smem));
         kern<<<dim3(ug.n_tiles, B), ug.threads, ug.smem, st>>>(

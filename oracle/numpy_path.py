@@ -75,11 +75,17 @@ def inverse_transform(x, name, exp_scale=1.0, exp_divisor=1.0):
 def axis_profiles(att_map, transform="sqrt", exp_scale=1.0, exp_divisor=1.0,
                   apply_inverse=False):
     """Returns (profile_x[w], profile_y[h], total_x, total_y, used_fallback)."""
-    h, w = att_map.shape[:2]
     a = np.maximum(np.asarray(att_map).astype(np.float64), 0)           # :207-208
     biased = forward_transform(a, transform, exp_scale, exp_divisor) + BASE_ATTENTION  # :210-212
-    prof_x = biased.sum(axis=0)                                         # :215  (w,)
-    prof_y = biased.sum(axis=1)                                         # :216  (h,)
+    return finish_profiles(biased.sum(axis=0), biased.sum(axis=1),      # :215-216
+                           biased.mean(), transform, exp_scale, exp_divisor, apply_inverse)
+
+
+def finish_profiles(prof_x, prof_y, biased_mean, transform="sqrt", exp_scale=1.0, exp_divisor=1.0,
+                    apply_inverse=False):
+    """The rest of ``axis_profiles`` from the raw marginal sums of the biased map (column sums ``prof_x[w]``, row
+    sums ``prof_y[h]``) and its mean: inverse transform, totals, fallback."""
+    h, w = len(prof_y), len(prof_x)
     if apply_inverse:                                                   # :219-226
         prof_x = inverse_transform(prof_x - BASE_ATTENTION * h, transform, exp_scale,
                                    exp_divisor) + BASE_ATTENTION * h
@@ -91,7 +97,7 @@ def axis_profiles(att_map, transform="sqrt", exp_scale=1.0, exp_divisor=1.0,
     if fallback:                                                        # :233-239
         prof_x = np.ones(w, dtype=np.float64)
         prof_y = np.ones(h, dtype=np.float64)
-        m = biased.mean()
+        m = biased_mean
         tot_x = max(w * (m * h), EPSILON)
         tot_y = max(h * (m * w), EPSILON)
     return prof_x, prof_y, float(tot_x), float(tot_y), fallback
@@ -200,7 +206,12 @@ def interp_scalar_numpy_algorithm(x, xp):
 def inverse_maps(att_map, new_width, new_height, transform="sqrt", exp_scale=1.0,
                  exp_divisor=1.0, apply_inverse=False):
     """Stages 2b-4 of the NumPy path: returns float64 (map_x[new_w], map_y[new_h], xp, yp)."""
-    px, py, tx, ty, _ = axis_profiles(att_map, transform, exp_scale, exp_divisor, apply_inverse)
+    return maps_from_profiles(*axis_profiles(att_map, transform, exp_scale, exp_divisor, apply_inverse)[:4],
+                              new_width, new_height)
+
+
+def maps_from_profiles(px, py, tx, ty, new_width, new_height):
+    """Stages 3-4 from ``axis_profiles``' profiles and totals: float64 (map_x, map_y, xp, yp)."""
     xp = forward_knots(px, tx, new_width)
     yp = forward_knots(py, ty, new_height)
     map_x = interp_restated(np.arange(new_width), xp)      # new_method.py:258-260
