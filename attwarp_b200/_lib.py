@@ -79,6 +79,8 @@ SIGNATURES = {
     "attwarp_png_max_bytes": (_sz, [_i, _i, _i]),
     "attwarp_png_workspace_bytes": (_sz, [_vp, _i]),
     "attwarp_encode_png": (_i, [_vp, _i, _vp, _sz, _vp, _sz, _vp, _vp]),
+    "attwarp_overlay_workspace_bytes": (_sz, [_vp, _i, _i]),
+    "attwarp_attention_overlay": (_i, [_vp, _i, _i, _i, _i, _i, C.c_double, _vp, _sz, _vp]),
     "attwarp_warp_image_host":(_i, [_vp, _i, _i, _i, _i, _vp, _i, _i, _i, _tp, _vp,
                                      C.POINTER(_i)]),
     "attwarp_safe_softmax": (_i, [_vp, _i, _i, _f, _vp, _vp]),

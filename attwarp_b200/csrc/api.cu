@@ -43,6 +43,9 @@ size_t png_workspace_bytes_impl(const attwarp_png_image* images, int n);
 int launch_encode_png(const attwarp_png_image* images, int n, void* ws, uint8_t* out, int64_t* offsets,
                       cudaStream_t st);
 int launch_interp_linear_rows(const float* F, int B, int N, int L, float* out, cudaStream_t st);
+size_t overlay_workspace_bytes_impl(const attwarp_overlay_image* images, int n, int att_kind);
+int launch_attention_overlay(const attwarp_overlay_image* images, int n, int att_dtype, int att_kind, int gh, int gw,
+                             double alpha, void* ws, cudaStream_t st);
 
 static thread_local char g_err[512] = "";
 
@@ -482,6 +485,53 @@ int attwarp_encode_png(const attwarp_png_image* images, int n, void* workspace, 
     if (cap != cudaStreamCaptureStatusNone)
         return fail(ATTWARP_ERR_UNSUPPORTED, "encode_png: cannot be captured into a CUDA graph (host-side descriptor table)");
     return launch_encode_png(images, n, workspace, static_cast<uint8_t*>(out), offsets, st);
+}
+
+// ---------------------------------------------------------------------------------------------
+static bool overlay_shape_ok(const attwarp_overlay_image& im) {
+    return im.H > 0 && im.W > 0 && im.H <= 65535 && im.W <= 65535 && (im.C == 1 || im.C == 3);
+}
+
+size_t attwarp_overlay_workspace_bytes(const attwarp_overlay_image* images, int n, int att_kind) {
+    if (images == nullptr || n <= 0 || (att_kind != ATTWARP_OVERLAY_MAP && att_kind != ATTWARP_OVERLAY_TOKENS))
+        return 0;
+    for (int i = 0; i < n; ++i)
+        if (!overlay_shape_ok(images[i])) return 0;
+    return overlay_workspace_bytes_impl(images, n, att_kind);
+}
+
+int attwarp_attention_overlay(const attwarp_overlay_image* images, int n, int att_dtype, int att_kind, int gh, int gw,
+                              double alpha, void* workspace, size_t workspace_bytes, void* stream) {
+    AW_REQUIRE(images, "attention_overlay: NULL pointer");
+    AW_REQUIRE(n > 0, "attention_overlay: n must be positive (got %d)", n);
+    AW_REQUIRE(att_kind == ATTWARP_OVERLAY_MAP || att_kind == ATTWARP_OVERLAY_TOKENS,
+               "attention_overlay: bad attention kind %d", att_kind);
+    if (att_kind == ATTWARP_OVERLAY_MAP)
+        AW_REQUIRE(att_dtype == ATTWARP_U8 || att_dtype == ATTWARP_F32 || att_dtype == ATTWARP_F64,
+                   "attention_overlay: attention dtype must be U8, F32 or F64 (got %d)", att_dtype);
+    else
+        AW_REQUIRE(att_dtype == ATTWARP_F32, "attention_overlay: token maps must be F32 (got dtype %d)", att_dtype);
+    AW_REQUIRE(att_kind == ATTWARP_OVERLAY_MAP || (gh > 0 && gw > 0 && gh <= 65535 && gw <= 65535),
+               "attention_overlay: token grid %d x %d outside [1, 65535]", gh, gw);
+    AW_REQUIRE(isfinite(alpha), "attention_overlay: alpha must be finite");
+    for (int i = 0; i < n; ++i) {
+        const attwarp_overlay_image& im = images[i];
+        AW_REQUIRE(im.src && im.att && im.dst, "attention_overlay: image %d: NULL pointer", i);
+        AW_REQUIRE(im.src != im.dst, "attention_overlay: image %d: dst must not be src", i);
+        AW_REQUIRE(im.C == 1 || im.C == 3, "attention_overlay: image %d: C must be 1 or 3 (got %d)", i, im.C);
+        AW_REQUIRE(overlay_shape_ok(im), "attention_overlay: image %d: H, W must lie in [1, 65535] (got %d x %d)", i,
+                   im.H, im.W);
+    }
+    const size_t need = overlay_workspace_bytes_impl(images, n, att_kind);
+    if (workspace == nullptr || workspace_bytes < need)
+        return fail(ATTWARP_ERR_WORKSPACE, "attention_overlay: workspace too small (%zu < %zu)", workspace_bytes, need);
+    cudaStream_t st = as_stream(stream);
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    AW_CUDA(cudaStreamIsCapturing(st, &cap));
+    if (cap != cudaStreamCaptureStatusNone)
+        return fail(ATTWARP_ERR_UNSUPPORTED,
+                    "attention_overlay: cannot be captured into a CUDA graph (host-side descriptor table)");
+    return launch_attention_overlay(images, n, att_dtype, att_kind, gh, gw, alpha, workspace, st);
 }
 
 static int warp_image_host_impl(const void* image_host, int img_dtype, int C, int H, int W,

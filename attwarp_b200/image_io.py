@@ -31,7 +31,9 @@ batches the rest:
        cv2.imencode 4.13: 0.998x on photo-like, 1.000-1.003x on smooth gradients, 0.999x on noise (336^2, 500^2,
        1344^2); noise never exceeds the stored size plus 17 bytes per 32 KiB and 75 bytes per file.
 * ``warp_files(...)``                the driver loop of main_batched.py:243-287 for a whole list of files: decode
-  -> one ragged launch per stage -> encode (``on_device_png=True``: the device encoder above).
+  -> one ragged launch per stage -> encode (``on_device_png=True``: the device encoder above).  With
+  ``overlay_paths`` / ``original_paths`` it also writes the other two files ``save_warped_image`` writes: the JET
+  attention overlay (``ops.attention_overlay``, bit-identical to the host expression) and the decoded image.
 """
 
 from __future__ import annotations
@@ -145,7 +147,9 @@ def encode_png_batch(images: Sequence[torch.Tensor], paths: Sequence[str], worke
 
 def warp_files(image_sources: Sequence, tok: torch.Tensor, output_paths: Sequence[str], out_sizes=None,
                transform: str = "identity", exp_scale: float = 1.0, exp_divisor: float = 1.0,
-               apply_inverse: bool = False, device=None, workers: int = 8, on_device_png: bool = False) -> List[bool]:
+               apply_inverse: bool = False, device=None, workers: int = 8, on_device_png: bool = False,
+               overlay_paths: Optional[Sequence[str]] = None, original_paths: Optional[Sequence[str]] = None,
+               overlay_alpha: float = 0.5) -> List[bool]:
     """The per-image loop of the batched driver (main_batched.py:243-287: ``save_warped_image(image, mask, ...,
     width, height, "identity")`` per sample) for a list of image files and their token maps: GPU decode -> stages
     2-5 for the whole (mixed-resolution) list in one launch per stage -> PNG files.
@@ -156,11 +160,32 @@ def warp_files(image_sources: Sequence, tok: torch.Tensor, output_paths: Sequenc
     The attention the reference warps with in this flow is ``blend_mask``'s image-size uint8 mask; use
     ``ops.mota_mask`` + ``ops.maps_from_attention`` when that exact quantisation is wanted -- this entry point warps
     with the token map index-upsampled on the fly (BASELINE configs[3]).
-    on_device_png  encode the files on the GPU (``encode_png_batch(on_device=True)``): same pixels, other bytes"""
-    if len(image_sources) == 0:
+    on_device_png  encode the files on the GPU (``encode_png_batch(on_device=True)``): same pixels, other bytes
+    overlay_paths  also write, per image, the JET attention overlay save_warped_image writes as
+                   ``masked_overlay_save_path``: ``ops.attention_overlay`` of the decoded image and its token map
+                   (index-upsampled like the warp's attention), weight ``overlay_alpha`` (the drivers' 0.5)
+    original_paths also write, per image, the decoded image: save_warped_image's ``original_image_save_path``.
+                   With nvJPEG decode these are nvJPEG's pixels (module docstring), not libjpeg's
+    Every file goes through one encoder call (one ``ops.encode_png`` with ``on_device_png``, else one cv2.imwrite
+    pool).  Returns one bool per file written, grouped per kind: the n warped files, then the n overlays if
+    ``overlay_paths`` is given, then the n originals if ``original_paths`` is given -- a list of n, 2n or 3n."""
+    n = len(image_sources)
+    for name, paths in (("overlay_paths", overlay_paths), ("original_paths", original_paths)):
+        if paths is not None and len(paths) != n:
+            raise ValueError(f"warp_files: {len(paths)} {name} for {n} images")
+    if n == 0:
         return []
     imgs = decode_jpeg_batch(image_sources, device)
     dev = imgs[0].device
-    outs = ops.warp_ragged_from_tokens(tok.to(dev), imgs, out_sizes, transform=transform, exp_scale=exp_scale,
+    tok = tok.to(dev)
+    outs = ops.warp_ragged_from_tokens(tok, imgs, out_sizes, transform=transform, exp_scale=exp_scale,
                                        exp_divisor=exp_divisor, apply_inverse=apply_inverse)
-    return encode_png_batch(outs, output_paths, workers, on_device=on_device_png)
+    images, paths = list(outs), list(output_paths)
+    if overlay_paths is not None:
+        images += ops.attention_overlay(imgs, tok=tok.reshape(n, tok.shape[-2], tok.shape[-1]).float(),
+                                        alpha=overlay_alpha)
+        paths += list(overlay_paths)
+    if original_paths is not None:
+        images += list(imgs)
+        paths += list(original_paths)
+    return encode_png_batch(images, paths, workers, on_device=on_device_png)

@@ -591,3 +591,129 @@ def encode_png(images):
         check(lib.attwarp_encode_png(table_p, n, ptr(ws), ws.numel(), ptr(payload), cap, ptr(offsets),
                                      current_stream(dev)))
     return payload, offsets
+
+
+# --------------------------------------------------------------------------------------------
+# Attention overlay (save_warped_image's masked_overlay_save_path image)
+# --------------------------------------------------------------------------------------------
+# attwarp_overlay_image (include/attwarp.h)
+_OVERLAY_DTYPE = np.dtype([("src", np.uint64), ("att", np.uint64), ("dst", np.uint64), ("H", np.int32),
+                           ("W", np.int32), ("C", np.int32), ("pad", np.int32)])
+_OVERLAY_MAP, _OVERLAY_TOKENS = 0, 1
+_OVERLAY_ATT_DTYPES = (torch.uint8, torch.float32, torch.float64)
+
+
+def attention_overlay(images, att=None, tok=None, alpha: float = 0.5):
+    """The JET attention overlay ``save_warped_image`` writes (``masked_overlay_save_path``) for n images of any
+    sizes, in two launches on the current stream (nothing synchronises).  Bit-identical to that host expression:
+    ``cv2.addWeighted(applyColorMap(uint8(n * 255), JET), alpha, base, 1 - alpha, 0)`` with
+    ``n = (a - lo) / (hi - lo) if hi > lo + 1e-9 else 0`` in the precision NumPy gives the map's dtype (the
+    contract: INTEGRATION.md section B.5b, include/attwarp.h).
+
+    images  a sequence of uint8 CUDA tensors [H, W, 3] (BGR) or [H, W] / [H, W, 1] (grey, replicated to BGR as
+            cv2.cvtColor(GRAY2BGR) does), or a [B, H, W, C] tensor
+    att     per-image attention maps of each image's own size: a sequence of [H, W] tensors or a [B, H, W] tensor,
+            uint8, float32 or float64 (e.g. the uint8 mask ``mota_mask`` / ``blend_mask`` gives)
+    tok     or [n, gh, gw] float32 token maps, index-upsampled to each image as ``maps_from_tokens`` does
+            (``(y * gh) // H``, ``(x * gw) // W``); lo and hi are those of the upsampled map
+    alpha   the heat map's weight (finite); the image's is 1 - alpha
+    Returns a list of uint8 [H, W, 3] BGR CUDA tensors (views of one buffer).  Exactly one of ``att`` / ``tok``.
+    A map of another size than its image is refused: the reference resizes it with cv2.resize(INTER_LINEAR),
+    whose float result is not reproducible bit for bit."""
+    lib = load()
+    if (att is None) == (tok is None):
+        raise ValueError("attention_overlay: give exactly one of att (per-image maps) or tok (token maps)")
+    if isinstance(images, torch.Tensor):
+        if images.dim() != 4:
+            raise ValueError(f"attention_overlay: a tensor argument must be [B, H, W, C], got {tuple(images.shape)}")
+        images = list(images.unbind(0))
+    elif not isinstance(images, (list, tuple)):
+        raise ValueError(f"attention_overlay: expected a sequence of image tensors or a [B, H, W, C] tensor, "
+                         f"got {type(images)}")
+    try:
+        alpha = float(alpha)
+    except (TypeError, ValueError):
+        raise ValueError(f"attention_overlay: alpha must be a finite number, got {alpha!r}") from None
+    if not np.isfinite(alpha):
+        raise ValueError(f"attention_overlay: alpha must be finite, got {alpha}")
+    imgs, chans = [], []
+    for k, t in enumerate(images):
+        if not isinstance(t, torch.Tensor):
+            raise ValueError(f"attention_overlay: image {k} is a {type(t).__name__}, not a tensor")
+        if t.dtype != torch.uint8:
+            raise ValueError(f"attention_overlay: image {k} must be uint8, got {t.dtype}")
+        if t.dim() == 3 and t.shape[2] == 4:
+            raise ValueError(f"attention_overlay: image {k} has 4 channels; the reference's cv2.addWeighted of a "
+                             "3-channel heat map fails on them too")
+        if t.dim() not in (2, 3) or (t.dim() == 3 and t.shape[2] not in (1, 3)) or t.numel() == 0:
+            raise ValueError(f"attention_overlay: image {k} must be a non-empty [H, W], [H, W, 1] or [H, W, 3] "
+                             f"tensor, got {tuple(t.shape)}")
+        imgs.append(t.contiguous())
+        chans.append(3 if t.dim() == 3 and t.shape[2] == 3 else 1)
+    n = len(imgs)
+    if tok is not None:
+        if not isinstance(tok, torch.Tensor) or tok.dim() != 3:
+            raise ValueError("attention_overlay: tok must be a [n, gh, gw] tensor")
+        if tok.dtype != torch.float32:
+            raise ValueError(f"attention_overlay: tok must be float32, got {tok.dtype}")
+        if tok.shape[0] != n:
+            raise ValueError(f"attention_overlay: {tok.shape[0]} token maps for {n} images")
+        if tok.shape[1] == 0 or tok.shape[2] == 0:
+            raise ValueError(f"attention_overlay: empty token grid {tuple(tok.shape[1:])}")
+        atts = list(tok.contiguous().unbind(0)) if n else []
+    else:
+        if isinstance(att, torch.Tensor):
+            if att.dim() != 3:
+                raise ValueError(f"attention_overlay: an att tensor must be [B, H, W], got {tuple(att.shape)}")
+            att = list(att.unbind(0))
+        elif not isinstance(att, (list, tuple)):
+            raise ValueError(f"attention_overlay: att must be a sequence of [H, W] tensors or a [B, H, W] tensor")
+        if len(att) != n:
+            raise ValueError(f"attention_overlay: {len(att)} attention maps for {n} images")
+        atts = []
+        for k, (a, im) in enumerate(zip(att, imgs)):
+            if not isinstance(a, torch.Tensor):
+                raise ValueError(f"attention_overlay: attention map {k} is a {type(a).__name__}, not a tensor")
+            if a.dtype not in _OVERLAY_ATT_DTYPES:
+                raise ValueError(f"attention_overlay: attention map {k} has dtype {a.dtype}; uint8, float32 and "
+                                 "float64 are supported")
+            if tuple(a.shape) != tuple(im.shape[:2]):
+                raise ValueError(f"attention_overlay: attention map {k} is {tuple(a.shape)}, image {k} is "
+                                 f"{tuple(im.shape[:2])}: a map of another size would need the reference's "
+                                 "cv2.resize(INTER_LINEAR), whose float result is not reproducible bit for bit; "
+                                 "resize it to the image first")
+            atts.append(a.contiguous())
+        if len({a.dtype for a in atts}) > 1:
+            raise ValueError("attention_overlay: all attention maps must have one dtype")
+    if n == 0:
+        return []
+    dev = imgs[0].device
+    if not imgs[0].is_cuda or any(t.device != dev for t in imgs + atts):
+        raise ValueError("attention_overlay: images and attention must all be on one CUDA device")
+    for k, t in enumerate(imgs):
+        if t.shape[0] > 65535 or t.shape[1] > 65535:
+            raise ValueError(f"attention_overlay: image {k} is {tuple(t.shape[:2])}; H and W must be at most 65535")
+    if tok is not None and (tok.shape[1] > 65535 or tok.shape[2] > 65535):
+        raise ValueError(f"attention_overlay: token grid {tuple(tok.shape[1:])} above 65535")
+    # outputs: one buffer, each image at a 16-byte aligned offset
+    sizes = [int(t.shape[0]) * int(t.shape[1]) * 3 for t in imgs]
+    offs = np.zeros(n + 1, dtype=np.int64)
+    offs[1:] = np.cumsum([(s + 15) // 16 * 16 for s in sizes])
+    buf = torch.empty(int(offs[-1]), dtype=torch.uint8, device=dev)
+    outs = [buf[int(o):int(o) + s].view(int(t.shape[0]), int(t.shape[1]), 3) for o, s, t in zip(offs, sizes, imgs)]
+    table = np.zeros(n, dtype=_OVERLAY_DTYPE)
+    table["src"] = [t.data_ptr() for t in imgs]
+    table["att"] = [a.data_ptr() for a in atts]
+    table["dst"] = [o.data_ptr() for o in outs]
+    table["H"] = [t.shape[0] for t in imgs]
+    table["W"] = [t.shape[1] for t in imgs]
+    table["C"] = chans
+    table_p = table.ctypes.data_as(C.c_void_p)           # `table` stays alive until the call returns
+    kind = _OVERLAY_TOKENS if tok is not None else _OVERLAY_MAP
+    gh, gw = (int(tok.shape[1]), int(tok.shape[2])) if tok is not None else (0, 0)
+    wsb = lib.attwarp_overlay_workspace_bytes(table_p, n, kind)
+    ws = _workspace(wsb, dev)
+    with torch.cuda.device(dev):
+        check(lib.attwarp_attention_overlay(table_p, n, TORCH_DTYPE_IDS[atts[0].dtype], kind, gh, gw, alpha,
+                                            ptr(ws), ws.numel(), current_stream(dev)))
+    return outs

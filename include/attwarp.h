@@ -292,6 +292,47 @@ size_t attwarp_png_workspace_bytes(const attwarp_png_image* images_host, int n);
 int attwarp_encode_png(const attwarp_png_image* images_host, int n, void* workspace, size_t workspace_bytes,
                        void* out, size_t out_capacity, int64_t* offsets, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Attention overlay of n uint8 images of any sizes in two launches: the JET heat map blended
+ * onto the image, the file save_warped_image writes as masked_overlay_save_path
+ * (AGW/new_method.py, attwarp_b200/new_method.py:save_warped_image).  Bit-identical to that host
+ * expression for a map `a` of the image's size:
+ *   lo, hi = min(a), max(a)  (a NaN anywhere: both NaN)
+ *   n = (a - lo) / (hi - lo) if hi > lo + 1e-9 else 0, in NumPy 2's precision for the dtype:
+ *       uint8: a - lo in uint8, the rest in float64; float32: all float32; float64: all float64
+ *   out = cv2.addWeighted(JET[uint8(n * 255)], alpha, base, 1 - alpha, 0)
+ *
+ * images   : HOST array of n descriptors; DEVICE pointers src (dense [H][W][C] uint8, C = 3 BGR
+ *            or C = 1 grey, replicated to BGR), att and dst (dense [H][W][3] uint8 BGR, not src);
+ *            any byte alignment.  1 <= H, W <= 65535.  They must stay valid until the stream has
+ *            run the call.
+ * att_kind : ATTWARP_OVERLAY_MAP    att is the image's own [H][W] map of att_dtype U8, F32 or F64
+ *                                   (gh, gw ignored)
+ *            ATTWARP_OVERLAY_TOKENS att is the image's [gh][gw] F32 token map, read at
+ *                                   ((y * gh) / H, (x * gw) / W) (the index upsampling of
+ *                                   attwarp_maps_from_tokens); lo and hi are taken over the tokens
+ *                                   that rule reaches.  1 <= gh, gw <= 65535.
+ * alpha    : finite; the weights are float(alpha) and float(1 - alpha), as cv2.addWeighted takes them
+ * workspace: attwarp_overlay_workspace_bytes(images, n, att_kind) bytes of device scratch
+ * The call uploads its descriptor table from host memory: ATTWARP_ERR_UNSUPPORTED on a stream
+ * that is being captured into a CUDA graph.
+ */
+typedef enum attwarp_overlay_kind {
+    ATTWARP_OVERLAY_MAP = 0,
+    ATTWARP_OVERLAY_TOKENS = 1
+} attwarp_overlay_kind;
+
+typedef struct attwarp_overlay_image {
+    const void* src;
+    const void* att;
+    void* dst;
+    int32_t H, W, C;
+} attwarp_overlay_image;
+
+size_t attwarp_overlay_workspace_bytes(const attwarp_overlay_image* images_host, int n, int att_kind);
+int attwarp_attention_overlay(const attwarp_overlay_image* images_host, int n, int att_dtype, int att_kind, int gh,
+                              int gw, double alpha, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Stages 2-3, torch path (all float32 [B][N] row-major unless noted).
  */
