@@ -450,6 +450,141 @@ int attwarp_warp_ragged_from_tokens(const float* tok, int n, int gh, int gw,
 int attwarp_ragged_last_launches(void) { return g_ragged_last_launches; }
 
 // ---------------------------------------------------------------------------------------------
+// Ragged batch warped by per-image maps.  Workspace: the tokens call's descriptor tables and map rows, then the
+// maps' descriptors (RaggedAtt) followed by the work items, then the partials: every image's at its own offset
+// (ragged geometry), or one image's of the uniform geometry when the call goes image by image.
+struct RaggedAttSizes {
+    size_t map_floats = 0, part_doubles = 0, uniform_bytes = 0;
+    int64_t items = 0;
+};
+static bool ragged_att_sizes(const attwarp_ragged_image* images, int n, RaggedAttSizes* s) {
+    for (int i = 0; i < n; ++i) {
+        const attwarp_ragged_image& im = images[i];
+        if (im.H <= 0 || im.W <= 0 || im.Ho <= 0 || im.Wo <= 0 || im.H >= 65536 || im.W >= 65536) return false;
+        int rows, nrc, tc, nct;
+        ragged_att_geometry(im.H, im.W, &rows, &nrc, &tc, &nct);
+        s->map_floats += (size_t)im.Wo + (size_t)im.Ho;
+        s->part_doubles += (size_t)nrc * im.W + (size_t)nct * im.H;
+        s->items += (int64_t)nrc * nct;
+        const size_t u = maps_workspace_bytes_impl(1, im.H, im.W);
+        s->uniform_bytes = u > s->uniform_bytes ? u : s->uniform_bytes;
+    }
+    return true;
+}
+static size_t ragged_att_desc_bytes(int n) { return align_up(sizeof(RaggedAtt) * (size_t)n, 16); }
+static size_t ragged_att_tables_bytes(int n, int64_t items) {
+    return align_up(ragged_att_desc_bytes(n) + sizeof(int2) * (size_t)items, 256);
+}
+
+size_t attwarp_ragged_attention_workspace_bytes(const attwarp_ragged_image* images, int n) {
+    RaggedAttSizes s;
+    if (images == nullptr || n <= 0 || !ragged_att_sizes(images, n, &s)) return 0;
+    const size_t part = s.part_doubles * sizeof(double);
+    return ragged_table_bytes(n) + align_up(s.map_floats * sizeof(float), 256) + ragged_att_tables_bytes(n, s.items) +
+           (part > s.uniform_bytes ? part : s.uniform_bytes);
+}
+
+int attwarp_warp_ragged_from_attention(const attwarp_ragged_image* images, const attwarp_ragged_attention* att,
+                                       int n, int att_dtype, int C, const attwarp_transform_params* tp,
+                                       void* workspace, size_t workspace_bytes, void* stream) {
+    AW_REQUIRE(images && att && workspace, "warp_ragged_from_attention: NULL pointer");
+    AW_REQUIRE(n > 0, "warp_ragged_from_attention: n must be positive (got %d)", n);
+    AW_REQUIRE(C == 1 || C == 3 || C == 4, "warp_ragged_from_attention: C must be 1, 3 or 4 (got %d)", C);
+    AW_REQUIRE(att_dtype == ATTWARP_U8 || att_dtype == ATTWARP_F32 || att_dtype == ATTWARP_F64,
+               "warp_ragged_from_attention: attention dtype must be U8, F32 or F64 (got %d)", att_dtype);
+    int rc = check_transform(tp);
+    if (rc != ATTWARP_OK) return rc;
+    const size_t es = dtype_size(att_dtype);
+    for (int i = 0; i < n; ++i) {
+        const attwarp_ragged_image& im = images[i];
+        AW_REQUIRE(im.src && im.dst && im.src != im.dst, "warp_ragged_from_attention: image %d: bad pointers", i);
+        AW_REQUIRE(im.H > 0 && im.W > 0 && im.Ho > 0 && im.Wo > 0,
+                   "warp_ragged_from_attention: image %d: sizes must be positive", i);
+        AW_REQUIRE(im.H < 65536 && im.W < 65536, "warp_ragged_from_attention: image %d: H, W must be below 65536", i);
+        AW_REQUIRE(att[i].att != nullptr, "warp_ragged_from_attention: image %d: NULL attention map", i);
+        AW_REQUIRE((reinterpret_cast<uintptr_t>(att[i].att) & (es - 1)) == 0,
+                   "warp_ragged_from_attention: image %d: attention map not aligned to its %zu-byte elements", i, es);
+    }
+    RaggedAttSizes s;
+    ragged_att_sizes(images, n, &s);
+    const size_t need = attwarp_ragged_attention_workspace_bytes(images, n);
+    if (workspace_bytes < need)
+        return fail(ATTWARP_ERR_WORKSPACE, "warp_ragged_from_attention: workspace too small (%zu < %zu)", workspace_bytes,
+                    need);
+    cudaStream_t st = as_stream(stream);
+    {
+        // as attwarp_warp_ragged_from_tokens: a captured copy node would read the host tables at replay time
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        AW_CUDA(cudaStreamIsCapturing(st, &cap));
+        if (cap != cudaStreamCaptureStatusNone)
+            return fail(ATTWARP_ERR_UNSUPPORTED,
+                        "warp_ragged_from_attention: cannot be captured into a CUDA graph (host-side descriptor tables)");
+    }
+    char* ws = static_cast<char*>(workspace);
+    RaggedImage* dev_table = reinterpret_cast<RaggedImage*>(ws);
+    ws += ragged_table_bytes(n);
+    float* pool = reinterpret_cast<float*>(ws);
+    ws += align_up(s.map_floats * sizeof(float), 256);
+    RaggedAtt* dev_att = reinterpret_cast<RaggedAtt*>(ws);
+    int2* dev_items = reinterpret_cast<int2*>(ws + ragged_att_desc_bytes(n));
+    ws += ragged_att_tables_bytes(n, s.items);
+    double* partials = reinterpret_cast<double*>(ws);
+    const size_t part_bytes = need - (size_t)(ws - static_cast<char*>(workspace));
+
+    static thread_local std::vector<RaggedImage> host;
+    static thread_local std::vector<RaggedAtt> host_att;
+    host.assign((size_t)n + 1, RaggedImage{});
+    host_att.assign((size_t)n, RaggedAtt{});
+    int max_h = 0, max_w = 0;
+    bool degenerate = false;
+    size_t off = 0;
+    int64_t part_off = 0;
+    for (int i = 0; i < n; ++i) {
+        const attwarp_ragged_image& im = images[i];
+        RaggedImage& r = host[(size_t)i];
+        r.src = static_cast<const uint8_t*>(im.src);
+        r.dst = static_cast<uint8_t*>(im.dst);
+        r.map_x = att[i].map_x != nullptr ? att[i].map_x : pool + off; off += (size_t)im.Wo;
+        r.map_y = att[i].map_y != nullptr ? att[i].map_y : pool + off; off += (size_t)im.Ho;
+        r.H = im.H; r.W = im.W; r.Ho = im.Ho; r.Wo = im.Wo;
+        RaggedAtt& a = host_att[(size_t)i];
+        a.att = att[i].att;
+        a.H = im.H; a.W = im.W;
+        ragged_att_geometry(im.H, im.W, &a.chunk_rows, &a.n_chunks, &a.tile_cols, &a.n_tiles);
+        a.colpart = part_off; part_off += (int64_t)a.n_chunks * im.W;
+        a.rowpart = part_off; part_off += (int64_t)a.n_tiles * im.H;
+        max_h = im.H > max_h ? im.H : max_h;
+        max_w = im.W > max_w ? im.W : max_w;
+        degenerate = degenerate || im.H < 2 || im.W < 2;
+    }
+    if (degenerate) {
+        // 1-pixel axes: image by image through the uniform entry points, as attwarp_warp_ragged_from_tokens does
+        for (int i = 0; i < n; ++i) {
+            const RaggedImage& r = host[(size_t)i];
+            rc = launch_maps_from_attention(att[i].att, att_dtype, 1, r.H, r.W, r.Wo, r.Ho, *tp, partials, part_bytes,
+                                            const_cast<float*>(r.map_x), const_cast<float*>(r.map_y), nullptr, st);
+            if (rc != ATTWARP_OK) return rc;
+            rc = launch_remap(r.src, r.dst, ATTWARP_U8, ATTWARP_LAYOUT_HWC, 1, C, r.H, r.W, r.Ho, r.Wo, r.map_x, r.map_y, st);
+            if (rc != ATTWARP_OK) return rc;
+        }
+        g_ragged_last_launches = 3 * n;          // marginals + finish + resample per image
+        return ATTWARP_OK;
+    }
+    const bool quad = C == 3 && remap_quad_enabled();
+    RaggedQuadPlan plan;
+    RaggedImage* dev_sorted = dev_table + (n + 1);
+    rc = quad ? launch_remap_u8_quad_ragged_prepare(host.data(), n, dev_table, dev_sorted, &plan, st)
+              : launch_remap_u8_stream_ragged_prepare(host.data(), n, C, dev_table, st);
+    if (rc != ATTWARP_OK) return rc;
+    rc = launch_maps_from_attention_ragged(host_att.data(), n, att_dtype, dev_table, dev_att, dev_items, s.items,
+                                           partials, max_h, max_w, *tp, st);
+    if (rc != ATTWARP_OK) return rc;
+    g_ragged_last_launches = 2 + (quad ? ragged_quad_launches(plan) : 1);
+    return quad ? launch_remap_u8_quad_ragged_run(plan, dev_sorted, st)
+                : launch_remap_u8_stream_ragged_run(host.data(), n, C, dev_table, st);
+}
+
+// ---------------------------------------------------------------------------------------------
 static bool png_shape_ok(int H, int W, int C) {
     return H > 0 && W > 0 && (C == 1 || C == 3 || C == 4) && (int64_t)W * C < ((int64_t)1 << 30);
 }

@@ -48,6 +48,25 @@ struct RaggedImage {
 };
 static_assert(sizeof(RaggedImage) == 64, "descriptor layout");
 
+// ---- the attention map of one image of a ragged batch (attwarp_warp_ragged_from_attention), kept beside its
+// RaggedImage (same index) so that the stage-5 descriptor keeps its size.  Geometry: ragged_att_geometry.
+struct RaggedAtt {
+    const void* att;         // [H][W] map, dense rows, any base alignment (element-aligned for float maps)
+    int64_t colpart;         // offset (in doubles) of the image's [n_chunks][W] column partials
+    int64_t rowpart;         // offset of its [n_tiles][H] row partials
+    int H, W;
+    int chunk_rows, n_chunks;
+    int tile_cols, n_tiles;
+};
+static_assert(sizeof(RaggedAtt) == 48, "descriptor layout");
+// chunk / tile geometry of one map of a ragged batch: a function of (H, W) only
+void ragged_att_geometry(int H, int W, int* chunk_rows, int* n_chunks, int* tile_cols, int* n_tiles);
+// host_att[0..n): geometry and partial offsets filled in; uploads them with the work items to dev_att / dev_items,
+// then launches the marginals kernel over all maps and the finish kernel that writes imgs[i].map_x / map_y
+int launch_maps_from_attention_ragged(const RaggedAtt* host_att, int n, int att_dtype, const RaggedImage* dev_imgs,
+                                      RaggedAtt* dev_att, int2* dev_items, int64_t n_items, double* partials,
+                                      int max_h, int max_w, const attwarp_transform_params& tp, cudaStream_t st);
+
 // ---- internal launchers (defined in the .cu files, used by the fused drivers in api.cu) -------
 int launch_aggregate_partial(const void* attn, int dtype, int B, int L, int Hh, int T,
                              int64_t sb, int64_t sl, int64_t sh, const int32_t* tok_start,

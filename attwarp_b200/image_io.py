@@ -145,31 +145,38 @@ def encode_png_batch(images: Sequence[torch.Tensor], paths: Sequence[str], worke
         return list(ex.map(write, range(len(paths))))
 
 
-def warp_files(image_sources: Sequence, tok: torch.Tensor, output_paths: Sequence[str], out_sizes=None,
+def warp_files(image_sources: Sequence, tok: Optional[torch.Tensor], output_paths: Sequence[str], out_sizes=None,
                transform: str = "identity", exp_scale: float = 1.0, exp_divisor: float = 1.0,
                apply_inverse: bool = False, device=None, workers: int = 8, on_device_png: bool = False,
                overlay_paths: Optional[Sequence[str]] = None, original_paths: Optional[Sequence[str]] = None,
-               overlay_alpha: float = 0.5) -> List[bool]:
+               overlay_alpha: float = 0.5, att=None) -> List[bool]:
     """The per-image loop of the batched driver (main_batched.py:243-287: ``save_warped_image(image, mask, ...,
     width, height, "identity")`` per sample) for a list of image files and their token maps: GPU decode -> stages
     2-5 for the whole (mixed-resolution) list in one launch per stage -> PNG files.
 
-    tok         [n, gh, gw] float32 token maps (the aggregated attention of each sample)
+    tok         [n, gh, gw] float32 token maps (the aggregated attention of each sample), index-upsampled to each
+                image on the fly (BASELINE configs[3])
+    att         or per-image attention maps of each decoded image's size ([H_i, W_i] CUDA tensors or NumPy arrays,
+                uint8 / float32 / float64, one dtype): the reference's own input, e.g. ``blend_mask``'s uint8 mask or
+                ``ops.mota_mask`` per image; warped with ``ops.warp_ragged_from_attention``.  Exactly one of
+                ``tok`` / ``att``.
     out_sizes   per-image (height, width) of the warped files, default = the input sizes (the drivers pass the
                 sample's own size, main_batched.py:276-287)
-    The attention the reference warps with in this flow is ``blend_mask``'s image-size uint8 mask; use
-    ``ops.mota_mask`` + ``ops.maps_from_attention`` when that exact quantisation is wanted -- this entry point warps
-    with the token map index-upsampled on the fly (BASELINE configs[3]).
     on_device_png  encode the files on the GPU (``encode_png_batch(on_device=True)``): same pixels, other bytes
     overlay_paths  also write, per image, the JET attention overlay save_warped_image writes as
-                   ``masked_overlay_save_path``: ``ops.attention_overlay`` of the decoded image and its token map
-                   (index-upsampled like the warp's attention), weight ``overlay_alpha`` (the drivers' 0.5)
+                   ``masked_overlay_save_path``: ``ops.attention_overlay`` of the decoded image and its attention
+                   (``att``, or the token map index-upsampled like the warp's attention), weight ``overlay_alpha``
+                   (the drivers' 0.5)
     original_paths also write, per image, the decoded image: save_warped_image's ``original_image_save_path``.
                    With nvJPEG decode these are nvJPEG's pixels (module docstring), not libjpeg's
     Every file goes through one encoder call (one ``ops.encode_png`` with ``on_device_png``, else one cv2.imwrite
     pool).  Returns one bool per file written, grouped per kind: the n warped files, then the n overlays if
     ``overlay_paths`` is given, then the n originals if ``original_paths`` is given -- a list of n, 2n or 3n."""
     n = len(image_sources)
+    if (tok is None) == (att is None):
+        raise ValueError("warp_files: give exactly one of tok (token maps) or att (per-image attention maps)")
+    if att is not None and len(att) != n:
+        raise ValueError(f"warp_files: {len(att)} attention maps for {n} images")
     for name, paths in (("overlay_paths", overlay_paths), ("original_paths", original_paths)):
         if paths is not None and len(paths) != n:
             raise ValueError(f"warp_files: {len(paths)} {name} for {n} images")
@@ -177,13 +184,22 @@ def warp_files(image_sources: Sequence, tok: torch.Tensor, output_paths: Sequenc
         return []
     imgs = decode_jpeg_batch(image_sources, device)
     dev = imgs[0].device
-    tok = tok.to(dev)
-    outs = ops.warp_ragged_from_tokens(tok, imgs, out_sizes, transform=transform, exp_scale=exp_scale,
-                                       exp_divisor=exp_divisor, apply_inverse=apply_inverse)
+    if att is not None:
+        maps = [torch.from_numpy(np.ascontiguousarray(a)).to(dev) if isinstance(a, np.ndarray) else a.to(dev)
+                for a in att]
+        outs = ops.warp_ragged_from_attention(maps, imgs, out_sizes, transform=transform, exp_scale=exp_scale,
+                                              exp_divisor=exp_divisor, apply_inverse=apply_inverse)
+    else:
+        tok = tok.to(dev)
+        outs = ops.warp_ragged_from_tokens(tok, imgs, out_sizes, transform=transform, exp_scale=exp_scale,
+                                           exp_divisor=exp_divisor, apply_inverse=apply_inverse)
     images, paths = list(outs), list(output_paths)
     if overlay_paths is not None:
-        images += ops.attention_overlay(imgs, tok=tok.reshape(n, tok.shape[-2], tok.shape[-1]).float(),
-                                        alpha=overlay_alpha)
+        if att is not None:
+            images += ops.attention_overlay(imgs, att=maps, alpha=overlay_alpha)
+        else:
+            images += ops.attention_overlay(imgs, tok=tok.reshape(n, tok.shape[-2], tok.shape[-1]).float(),
+                                            alpha=overlay_alpha)
         paths += list(overlay_paths)
     if original_paths is not None:
         images += list(imgs)

@@ -474,6 +474,96 @@ def warp_ragged_from_tokens(tok: torch.Tensor, images, out_sizes=None, grid_hw=N
     return outs
 
 
+# attwarp_ragged_attention (include/attwarp.h)
+_RAGGED_ATT_DTYPE = np.dtype([("att", np.uint64), ("map_x", np.uint64), ("map_y", np.uint64)])
+_RAGGED_MAP_DTYPES = (torch.uint8, torch.float32, torch.float64)
+
+
+def warp_ragged_from_attention(att, images, out_sizes=None, transform="identity", exp_scale=1.0, exp_divisor=1.0,
+                               apply_inverse=False, outs=None, return_maps=False):
+    """Stages 2b-5 for n images of different shapes, each warped by its OWN attention map -- the reference's
+    ``warp_image_by_attention(image, att_map, w, h)`` (new_method.py:198-283) per image -- in one marginals launch
+    for all maps, one finish launch and the stage-5 launches of ``warp_ragged_from_tokens``.
+
+    att     sequence of n CUDA tensors [H_i, W_i] of one dtype: uint8 (e.g. ``blend_mask`` / ``mota_mask``),
+            float32 or float64.  Any strides of a 2-D view are taken (non-dense ones are copied first); rows may
+            start at any byte offset.
+    images  sequence of n uint8 HWC tensors [H_i, W_i, C], C in {1, 3, 4}, on the same device
+    out_sizes  sequence of (Ho_i, Wo_i), default = input sizes
+    Returns the list of warped images, and with ``return_maps`` also the lists of map_x [Wo_i] and map_y [Ho_i].
+    An image's maps depend on its own map only: they are bit-identical to those of a call on that image alone."""
+    lib = load()
+    n = len(images)
+    if not isinstance(att, (list, tuple)):
+        raise ValueError(f"warp_ragged_from_attention: att must be a sequence of [H, W] tensors, got {type(att).__name__}")
+    if len(att) != n:
+        raise ValueError(f"warp_ragged_from_attention: {len(att)} attention maps for {n} images")
+    if n == 0:
+        return ([], [], []) if return_maps else []
+    require_cuda(*images)
+    dev = images[0].device
+    Cc = images[0].shape[2] if images[0].dim() == 3 else 0
+    if Cc not in (1, 3, 4):
+        raise ValueError(f"warp_ragged_from_attention: images must be uint8 [H, W, C] with C in (1, 3, 4), got "
+                         f"{tuple(images[0].shape)}")
+    maps = []
+    for k, (a, im) in enumerate(zip(att, images)):
+        if not isinstance(a, torch.Tensor):
+            raise ValueError(f"warp_ragged_from_attention: attention map {k} is a {type(a).__name__}, not a tensor")
+        if a.dim() != 2:
+            raise ValueError(f"warp_ragged_from_attention: attention map {k} must be 2-D [H, W], got {tuple(a.shape)}")
+        if a.dtype not in _RAGGED_MAP_DTYPES:
+            raise ValueError(f"warp_ragged_from_attention: attention map {k} has dtype {a.dtype}; uint8, float32 and "
+                             "float64 are supported")
+        if a.device != dev:
+            raise ValueError(f"warp_ragged_from_attention: attention map {k} is on {a.device}, image 0 on {dev}: all "
+                             "tensors must be on one CUDA device")
+        if im.dim() != 3 or tuple(a.shape) != tuple(im.shape[:2]):
+            raise ValueError(f"warp_ragged_from_attention: attention map {k} is {tuple(a.shape)}, image {k} is "
+                             f"{tuple(im.shape[:2])}: the map must have its image's size")
+        maps.append(a if a.is_contiguous() else a.contiguous())
+    if len({a.dtype for a in maps}) > 1:
+        raise ValueError("warp_ragged_from_attention: all attention maps must have one dtype, got "
+                         f"{sorted({str(a.dtype) for a in maps})}")
+    imgs = [im.contiguous() for im in images]
+    if out_sizes is None:
+        out_sizes = [(im.shape[0], im.shape[1]) for im in imgs]
+    if len(out_sizes) != n:
+        raise ValueError(f"warp_ragged_from_attention: {len(out_sizes)} output sizes for {n} images")
+    if outs is None:
+        outs = [torch.empty(ho, wo, Cc, dtype=torch.uint8, device=dev) for ho, wo in out_sizes]
+    for im, o, (ho, wo) in zip(imgs, outs, out_sizes):
+        if (im.dtype != torch.uint8 or im.shape[2] != Cc or im.device != dev
+                or o.dtype != torch.uint8 or tuple(o.shape) != (ho, wo, Cc) or not o.is_contiguous()
+                or o.device != dev):
+            raise ValueError("warp_ragged_from_attention: images must be uint8 HWC tensors with the same channel "
+                             "count on one device, outputs contiguous [Ho, Wo, C]")
+    table = np.empty(n, dtype=_RAGGED_DTYPE)
+    table["src"] = [im.data_ptr() for im in imgs]
+    table["dst"] = [o.data_ptr() for o in outs]
+    table["H"] = [im.shape[0] for im in imgs]
+    table["W"] = [im.shape[1] for im in imgs]
+    table["Ho"] = [hw[0] for hw in out_sizes]
+    table["Wo"] = [hw[1] for hw in out_sizes]
+    atab = np.zeros(n, dtype=_RAGGED_ATT_DTYPE)
+    atab["att"] = [a.data_ptr() for a in maps]
+    map_xs = map_ys = None
+    if return_maps:
+        map_xs = [torch.empty(int(wo), dtype=torch.float32, device=dev) for _, wo in out_sizes]
+        map_ys = [torch.empty(int(ho), dtype=torch.float32, device=dev) for ho, _ in out_sizes]
+        atab["map_x"] = [m.data_ptr() for m in map_xs]
+        atab["map_y"] = [m.data_ptr() for m in map_ys]
+    table_p = table.ctypes.data_as(C.c_void_p)           # the tables stay alive until the call returns
+    atab_p = atab.ctypes.data_as(C.c_void_p)
+    tp = _tp(transform, exp_scale, exp_divisor, apply_inverse)
+    wsb = lib.attwarp_ragged_attention_workspace_bytes(table_p, n)
+    ws = _workspace(wsb, dev)
+    with torch.cuda.device(dev):
+        check(lib.attwarp_warp_ragged_from_attention(table_p, atab_p, n, TORCH_DTYPE_IDS[maps[0].dtype], Cc,
+                                                     C.byref(tp), ptr(ws), ws.numel(), current_stream(dev)))
+    return (outs, map_xs, map_ys) if return_maps else outs
+
+
 class RaggedBatch:
     """A mixed-resolution batch whose buffers stay put across calls (the steady state of a driver that re-uses its
     image and output buffers): the descriptor table, the output tensors and a private workspace are built ONCE,

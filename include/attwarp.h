@@ -247,9 +247,38 @@ int attwarp_warp_ragged_from_tokens(const float* tok, int n, int gh, int gw,
                                     const attwarp_transform_params* tp, void* workspace,
                                     size_t workspace_bytes, void* stream);
 
-/* Kernel launches the calling thread's last attwarp_warp_ragged_from_tokens call enqueued: one maps launch + one
- * stage-5 launch per non-empty class (images are grouped by the consumer warps their strips need and by whether
- * their destination rows are 4-byte aligned).  For accounting (bench.py's gpu_launches). */
+/* Ragged batch warped by each image's OWN attention map (warp_image_by_attention(image, att_map, w, h) per image,
+ * AGW/new_method.py:198-283, for a mixed-size list): stages 2b-5 with one marginals launch for all maps, one
+ * finish launch, and the stage-5 launches of attwarp_warp_ragged_from_tokens.
+ *
+ * images    : as for attwarp_warp_ragged_from_tokens
+ * att       : HOST array of n entries:
+ *               att    device [H][W] map of att_dtype (the image's own size), dense rows, any byte alignment
+ *                      (float32 / float64 maps: aligned to their element size)
+ *               map_x  device [Wo] floats or NULL: receives the image's map_x (else it stays in the workspace)
+ *               map_y  device [Ho] floats or NULL
+ * att_dtype : ATTWARP_U8, ATTWARP_F32 or ATTWARP_F64, one for all maps
+ * tp        : NumPy semantics (clamp at 0, transform, + 1e-9, float64 sums), as attwarp_maps_from_attention
+ * workspace : attwarp_ragged_attention_workspace_bytes(images, n) bytes of device scratch (0: invalid sizes)
+ * An image's maps depend on its own map only (its chunk / tile geometry follows from its H x W), so they are
+ * bit-identical to those of a call on that image alone.  Images with H or W below 2 make the call go image by
+ * image through the uniform entry points.  Host-side descriptor tables: ATTWARP_ERR_UNSUPPORTED under CUDA-graph
+ * capture; ATTWARP_ERR_UNSUPPORTED when the largest H + W do not fit the shared-memory knots. */
+typedef struct attwarp_ragged_attention {
+    const void* att;
+    float* map_x;
+    float* map_y;
+} attwarp_ragged_attention;
+
+size_t attwarp_ragged_attention_workspace_bytes(const attwarp_ragged_image* images, int n);
+int attwarp_warp_ragged_from_attention(const attwarp_ragged_image* images, const attwarp_ragged_attention* att,
+                                       int n, int att_dtype, int C, const attwarp_transform_params* tp,
+                                       void* workspace, size_t workspace_bytes, void* stream);
+
+/* Kernel launches the calling thread's last attwarp_warp_ragged_from_tokens / attwarp_warp_ragged_from_attention
+ * call enqueued: the maps launches (tokens: one; attention: marginals + finish) + one stage-5 launch per non-empty
+ * class (images are grouped by the consumer warps their strips need and by whether their destination rows are
+ * 4-byte aligned).  For accounting (bench.py's gpu_launches). */
 int attwarp_ragged_last_launches(void);
 
 /* attwarp_warp_image_host: the whole of warp_image_by_attention (AGW/new_method.py:198-283) for
