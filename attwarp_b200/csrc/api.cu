@@ -431,6 +431,7 @@ int attwarp_warp_ragged_from_tokens(const float* tok, int n, int gh, int gw,
             rc = launch_remap(r.src, r.dst, ATTWARP_U8, ATTWARP_LAYOUT_HWC, 1, C, r.H, r.W, r.Ho, r.Wo, r.map_x, r.map_y, st);
             if (rc != ATTWARP_OK) return rc;
         }
+        g_ragged_last_launches = 2 * n;          // maps + resample per image
         return ATTWARP_OK;
     }
     // the strip plan of stage 5 is part of the table both kernels read: plan + upload, maps, resample
