@@ -78,6 +78,8 @@ SIGNATURES = {
     "attwarp_warp_ragged_from_tokens": (_i, [_vp, _i, _i, _i, _vp, _i, _tp, _vp, _sz, _vp]),
     "attwarp_ragged_attention_workspace_bytes": (_sz, [_vp, _i]),
     "attwarp_warp_ragged_from_attention": (_i, [_vp, _vp, _i, _i, _i, _tp, _vp, _sz, _vp]),
+    "attwarp_ragged_mask_workspace_bytes": (_sz, [_vp, _i, _i, _i]),
+    "attwarp_warp_ragged_from_mask": (_i, [_vp, _vp, _i, _i, _i, _i, _tp, _vp, _sz, _vp, _vp, _vp]),
     "attwarp_png_max_bytes": (_sz, [_i, _i, _i]),
     "attwarp_png_workspace_bytes": (_sz, [_vp, _i]),
     "attwarp_encode_png": (_i, [_vp, _i, _vp, _sz, _vp, _sz, _vp, _vp]),

@@ -586,6 +586,199 @@ int attwarp_warp_ragged_from_attention(const attwarp_ragged_image* images, const
 }
 
 // ---------------------------------------------------------------------------------------------
+// Ragged batch warped by each image's LANCZOS-resized mask.  Workspace: the tokens call's descriptor tables and map
+// rows, then RaggedAtt [n], RaggedLanczos [n] and the work items (fused kernel's, then the uint8 marginals'), then the
+// image-size masks of the images the fused kernel does not take, then the partials (every image's at its own offset,
+// or one image's of the uniform entry points when the call goes image by image).
+struct RaggedMaskSizes {
+    size_t map_floats = 0, part_doubles = 0, mask_bytes = 0, uniform_bytes = 0, smem = 0;
+    int64_t fused_items = 0, att_items = 0;
+};
+static bool ragged_mask_sizes(const attwarp_ragged_image* images, int n, int gh, int gw, RaggedMaskSizes* s) {
+    for (int i = 0; i < n; ++i) {
+        const attwarp_ragged_image& im = images[i];
+        if (im.H <= 0 || im.W <= 0 || im.Ho <= 0 || im.Wo <= 0 || im.H >= 65536 || im.W >= 65536) return false;
+        s->map_floats += (size_t)im.Wo + (size_t)im.Ho;
+        int rows, nt, nx, warps;
+        size_t smem, part;
+        if (lanczos_ragged_geometry(gh, gw, im.H, im.W, &rows, &nt, &nx, &warps, &smem)) {
+            part = (size_t)nt * im.W + (size_t)nx * im.H;
+            s->fused_items += (int64_t)nt * nx;
+            s->smem = smem > s->smem ? smem : s->smem;
+        } else {
+            int nrc, tc, nct;
+            ragged_att_geometry(im.H, im.W, &rows, &nrc, &tc, &nct);
+            part = (size_t)nrc * im.W + (size_t)nct * im.H;
+            s->att_items += (int64_t)nrc * nct;
+            s->mask_bytes += align_up((size_t)im.H * im.W, 16);
+            const size_t u = maps_workspace_bytes_impl(1, im.H, im.W);
+            s->uniform_bytes = u > s->uniform_bytes ? u : s->uniform_bytes;
+        }
+        s->part_doubles += part;
+        s->uniform_bytes = part * sizeof(double) > s->uniform_bytes ? part * sizeof(double) : s->uniform_bytes;
+    }
+    return true;
+}
+static size_t ragged_mask_tables_bytes(int n, int64_t items) {
+    return align_up(align_up(sizeof(RaggedAtt) * (size_t)n, 16) + sizeof(RaggedLanczos) * (size_t)n +
+                    sizeof(int2) * (size_t)items, 256);
+}
+
+size_t attwarp_ragged_mask_workspace_bytes(const attwarp_ragged_image* images, int n, int gh, int gw) {
+    RaggedMaskSizes s;
+    if (images == nullptr || n <= 0 || gh <= 0 || gw <= 0 || !ragged_mask_sizes(images, n, gh, gw, &s)) return 0;
+    const size_t part = s.part_doubles * sizeof(double);
+    return ragged_table_bytes(n) + align_up(s.map_floats * sizeof(float), 256) +
+           ragged_mask_tables_bytes(n, s.fused_items + s.att_items) + align_up(s.mask_bytes, 256) +
+           (part > s.uniform_bytes ? part : s.uniform_bytes);
+}
+
+int attwarp_warp_ragged_from_mask(const attwarp_ragged_image* images, const void* mask_u8, int n, int gh, int gw, int C,
+                                  const attwarp_transform_params* tp, void* workspace, size_t workspace_bytes,
+                                  float* map_x_opt, float* map_y_opt, void* stream) {
+    AW_REQUIRE(images && mask_u8 && workspace, "warp_ragged_from_mask: NULL pointer");
+    AW_REQUIRE(n > 0 && gh > 0 && gw > 0, "warp_ragged_from_mask: n, gh, gw must be positive (got %d, %d, %d)", n, gh, gw);
+    AW_REQUIRE(C == 1 || C == 3 || C == 4, "warp_ragged_from_mask: C must be 1, 3 or 4 (got %d)", C);
+    int rc = check_transform(tp);
+    if (rc != ATTWARP_OK) return rc;
+    if (tp->transform != ATTWARP_T_IDENTITY)
+        return fail(ATTWARP_ERR_UNSUPPORTED, "warp_ragged_from_mask: identity transform only (got %d; resize the masks and "
+                    "use warp_ragged_from_attention)", tp->transform);
+    for (int i = 0; i < n; ++i) {
+        const attwarp_ragged_image& im = images[i];
+        AW_REQUIRE(im.src && im.dst && im.src != im.dst, "warp_ragged_from_mask: image %d: bad pointers", i);
+        AW_REQUIRE(im.H > 0 && im.W > 0 && im.Ho > 0 && im.Wo > 0, "warp_ragged_from_mask: image %d: sizes must be positive", i);
+        AW_REQUIRE(im.H < 65536 && im.W < 65536, "warp_ragged_from_mask: image %d: H, W must be below 65536", i);
+    }
+    RaggedMaskSizes s;
+    ragged_mask_sizes(images, n, gh, gw, &s);
+    const size_t need = attwarp_ragged_mask_workspace_bytes(images, n, gh, gw);
+    if (workspace_bytes < need)
+        return fail(ATTWARP_ERR_WORKSPACE, "warp_ragged_from_mask: workspace too small (%zu < %zu)", workspace_bytes, need);
+    cudaStream_t st = as_stream(stream);
+    {
+        // as attwarp_warp_ragged_from_tokens: a captured copy node would read the host tables at replay time
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        AW_CUDA(cudaStreamIsCapturing(st, &cap));
+        if (cap != cudaStreamCaptureStatusNone)
+            return fail(ATTWARP_ERR_UNSUPPORTED,
+                        "warp_ragged_from_mask: cannot be captured into a CUDA graph (host-side descriptor tables)");
+    }
+    const int64_t n_items = s.fused_items + s.att_items;
+    char* ws = static_cast<char*>(workspace);
+    RaggedImage* dev_table = reinterpret_cast<RaggedImage*>(ws);
+    ws += ragged_table_bytes(n);
+    float* pool = reinterpret_cast<float*>(ws);
+    ws += align_up(s.map_floats * sizeof(float), 256);
+    char* dev_tables = ws;
+    const size_t lz_off = align_up(sizeof(RaggedAtt) * (size_t)n, 16), items_off = lz_off + sizeof(RaggedLanczos) * (size_t)n;
+    RaggedAtt* dev_att = reinterpret_cast<RaggedAtt*>(dev_tables);
+    int2* dev_items = reinterpret_cast<int2*>(dev_tables + items_off);
+    ws += ragged_mask_tables_bytes(n, n_items);
+    uint8_t* masks = reinterpret_cast<uint8_t*>(ws);
+    ws += align_up(s.mask_bytes, 256);
+    double* partials = reinterpret_cast<double*>(ws);
+    const size_t part_bytes = need - (size_t)(ws - static_cast<char*>(workspace));
+
+    static thread_local std::vector<RaggedImage> host;
+    static thread_local std::vector<char> host_tables;
+    host.assign((size_t)n + 1, RaggedImage{});
+    host_tables.assign(items_off + sizeof(int2) * (size_t)n_items, 0);
+    RaggedAtt* host_att = reinterpret_cast<RaggedAtt*>(host_tables.data());
+    RaggedLanczos* host_lz = reinterpret_cast<RaggedLanczos*>(host_tables.data() + lz_off);
+    int2* fused_items = reinterpret_cast<int2*>(host_tables.data() + items_off);
+    int2* att_items = fused_items + s.fused_items;
+    int max_h = 0, max_w = 0, launches = 0;
+    bool degenerate = false;
+    size_t off = 0, mask_off = 0, mx_off = 0, my_off = 0;
+    int64_t part_off = 0, nf = 0, na = 0;
+    const uint8_t* mask = static_cast<const uint8_t*>(mask_u8);
+    for (int i = 0; i < n; ++i) {
+        const attwarp_ragged_image& im = images[i];
+        RaggedImage& r = host[(size_t)i];
+        r.src = static_cast<const uint8_t*>(im.src);
+        r.dst = static_cast<uint8_t*>(im.dst);
+        r.map_x = map_x_opt != nullptr ? map_x_opt + mx_off : pool + off; off += (size_t)im.Wo; mx_off += (size_t)im.Wo;
+        r.map_y = map_y_opt != nullptr ? map_y_opt + my_off : pool + off; off += (size_t)im.Ho; my_off += (size_t)im.Ho;
+        r.H = im.H; r.W = im.W; r.Ho = im.Ho; r.Wo = im.Wo;
+        RaggedAtt& a = host_att[i];
+        a.H = im.H; a.W = im.W;
+        int rows, nt, nx, warps;
+        size_t smem;
+        if (lanczos_ragged_geometry(gh, gw, im.H, im.W, &rows, &nt, &nx, &warps, &smem)) {
+            // the fused kernel: row tiles as chunks, column CTAs as tiles of the finish kernel's partial layout
+            a.att = mask + (size_t)i * gh * gw;
+            a.chunk_rows = rows; a.n_chunks = nt;
+            a.tile_cols = warps * 64; a.n_tiles = nx;
+            rc = lanczos_ragged_tables(gh, gw, im.H, im.W, rows, &host_lz[i]);
+            if (rc != ATTWARP_OK) return rc;
+            host_lz[i].warps = warps;
+            for (int t = 0; t < nt; ++t)
+                for (int x = 0; x < nx; ++x) fused_items[nf++] = make_int2(i, t << 8 | x);
+        } else {
+            // resized to image size first, then summed by the ragged uint8 marginals kernel
+            a.att = masks + mask_off;
+            mask_off += align_up((size_t)im.H * im.W, 16);
+            ragged_att_geometry(im.H, im.W, &a.chunk_rows, &a.n_chunks, &a.tile_cols, &a.n_tiles);
+            for (int c = 0; c < a.n_chunks; ++c)
+                for (int t = 0; t < a.n_tiles; ++t) att_items[na++] = make_int2(i, c << 8 | t);
+            rc = launch_resize_lanczos_u8(mask + (size_t)i * gh * gw, 1, gh, gw, im.H, im.W,
+                                          static_cast<uint8_t*>(const_cast<void*>(a.att)), st);
+            if (rc != ATTWARP_OK) return rc;
+            ++launches;
+        }
+        a.colpart = part_off; part_off += (int64_t)a.n_chunks * im.W;
+        a.rowpart = part_off; part_off += (int64_t)a.n_tiles * im.H;
+        max_h = im.H > max_h ? im.H : max_h;
+        max_w = im.W > max_w ? im.W : max_w;
+        degenerate = degenerate || im.H < 2 || im.W < 2;
+    }
+    if (degenerate) {
+        // 1-pixel axes: image by image through the uniform entry points, as attwarp_warp_ragged_from_attention does
+        for (int i = 0; i < n; ++i) {
+            const RaggedImage& r = host[(size_t)i];
+            float* mx = const_cast<float*>(r.map_x);
+            float* my = const_cast<float*>(r.map_y);
+            if (host_lz[i].planes != nullptr)           // taken by the fused kernel
+                rc = launch_maps_from_mask(mask + (size_t)i * gh * gw, 1, gh, gw, r.H, r.W, r.Wo, r.Ho, *tp, partials,
+                                           part_bytes, mx, my, st);
+            else
+                rc = launch_maps_from_attention(host_att[i].att, ATTWARP_U8, 1, r.H, r.W, r.Wo, r.Ho, *tp, partials,
+                                                part_bytes, mx, my, nullptr, st);
+            if (rc != ATTWARP_OK) return rc;
+            rc = launch_remap(r.src, r.dst, ATTWARP_U8, ATTWARP_LAYOUT_HWC, 1, C, r.H, r.W, r.Ho, r.Wo, r.map_x, r.map_y, st);
+            if (rc != ATTWARP_OK) return rc;
+        }
+        g_ragged_last_launches = launches + 3 * n;    // resizes + marginals, finish and resample per image
+        return ATTWARP_OK;
+    }
+    const bool quad = C == 3 && remap_quad_enabled();
+    RaggedQuadPlan plan;
+    RaggedImage* dev_sorted = dev_table + (n + 1);
+    rc = quad ? launch_remap_u8_quad_ragged_prepare(host.data(), n, dev_table, dev_sorted, &plan, st)
+              : launch_remap_u8_stream_ragged_prepare(host.data(), n, C, dev_table, st);
+    if (rc != ATTWARP_OK) return rc;
+    AW_CUDA(cudaMemcpyAsync(dev_tables, host_tables.data(), host_tables.size(), cudaMemcpyHostToDevice, st));
+    if (s.fused_items > 0) {
+        rc = launch_lanczos_marginals_ragged(dev_items, s.fused_items, dev_att,
+                                             reinterpret_cast<const RaggedLanczos*>(dev_tables + lz_off), gw, s.smem,
+                                             partials, st);
+        if (rc != ATTWARP_OK) return rc;
+        ++launches;
+    }
+    if (s.att_items > 0) {
+        rc = launch_marginals_ragged_u8_identity(dev_items + s.fused_items, s.att_items, dev_att, partials, st);
+        if (rc != ATTWARP_OK) return rc;
+        ++launches;
+    }
+    rc = launch_maps_from_partials_ragged(n, dev_table, dev_att, partials, max_h, max_w, *tp, st);
+    if (rc != ATTWARP_OK) return rc;
+    g_ragged_last_launches = launches + 1 + (quad ? ragged_quad_launches(plan) : 1);
+    return quad ? launch_remap_u8_quad_ragged_run(plan, dev_sorted, st)
+                : launch_remap_u8_stream_ragged_run(host.data(), n, C, dev_table, st);
+}
+
+// ---------------------------------------------------------------------------------------------
 static bool png_shape_ok(int H, int W, int C) {
     return H > 0 && W > 0 && (C == 1 || C == 3 || C == 4) && (int64_t)W * C < ((int64_t)1 << 30);
 }

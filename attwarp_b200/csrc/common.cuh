@@ -66,6 +66,32 @@ void ragged_att_geometry(int H, int W, int* chunk_rows, int* n_chunks, int* tile
 int launch_maps_from_attention_ragged(const RaggedAtt* host_att, int n, int att_dtype, const RaggedImage* dev_imgs,
                                       RaggedAtt* dev_att, int2* dev_items, int64_t n_items, double* partials,
                                       int max_h, int max_w, const attwarp_transform_params& tp, cudaStream_t st);
+// the two launches of that call apart, for attwarp_warp_ragged_from_mask: the uint8 identity marginals over the items
+// dev_items[0..n_items) (descriptors already on the device), and the finish over all n images
+int launch_marginals_ragged_u8_identity(const int2* dev_items, int64_t n_items, const RaggedAtt* dev_att,
+                                        double* partials, cudaStream_t st);
+int launch_maps_from_partials_ragged(int n, const RaggedImage* dev_imgs, const RaggedAtt* dev_att, const double* partials,
+                                     int max_h, int max_w, const attwarp_transform_params& tp, cudaStream_t st);
+
+// ---- the LANCZOS coefficients of one mask of a ragged list (attwarp_warp_ragged_from_mask), beside its RaggedAtt
+// (whose chunk_rows / n_chunks / tile_cols / n_tiles hold the fused kernel's rows per tile, row tiles, columns per CTA
+// and column CTAs).  Device pointers into the coefficient tables mask.cu keeps per size.
+struct RaggedLanczos {
+    const int2* bx;          // horizontal pass: first tap per output column
+    const int* kx;           //                  [W][ksx] 22-bit weights
+    const int2* by;          // vertical pass: window per output row
+    const uint8_t* planes;   //                [row tile][3][rows][16] coefficient byte planes
+    int ksx, warps;          // taps per column; 64-column strips per CTA
+};
+static_assert(sizeof(RaggedLanczos) == 40, "descriptor layout");
+// Geometry of the tensor-core marginals kernel for an h x w mask resized to H x W, as a call on that image alone takes
+// it (false: that call would not run this kernel); pure host arithmetic
+bool lanczos_ragged_geometry(int h, int w, int H, int W, int* rows, int* n_tiles, int* x_ctas, int* warps, size_t* smem);
+// the coefficient tables of (h, w) -> (H, W) at `rows` rows per tile (built and uploaded once per size and device)
+int lanczos_ragged_tables(int h, int w, int H, int W, int rows, RaggedLanczos* l);
+// one launch over the items (image, row tile << 8 | column CTA); the descriptors are on the device
+int launch_lanczos_marginals_ragged(const int2* dev_items, int64_t n_items, const RaggedAtt* dev_att,
+                                    const RaggedLanczos* dev_lz, int w, size_t smem, double* partials, cudaStream_t st);
 
 // ---- internal launchers (defined in the .cu files, used by the fused drivers in api.cu) -------
 int launch_aggregate_partial(const void* attn, int dtype, int B, int L, int Hh, int T,

@@ -309,33 +309,32 @@ __device__ __forceinline__ void mma_s8u8(int (&d)[4], const uint32_t (&a)[2], ui
     asm volatile("mma.sync.aligned.m16n8k16.row.col.s32.s8.u8.s32 {%0,%1,%2,%3}, {%4,%5}, {%6}, {%0,%1,%2,%3};"
                  : "+r"(d[0]), "+r"(d[1]), "+r"(d[2]), "+r"(d[3]) : "r"(a[0]), "r"(a[1]), "r"(b));
 }
-template <bool MARG>
-__device__ __forceinline__ void mma_write_row_sums(const int* rsum, int rows, int b, int y0, int Ho, int Wo, int x_base,
-                                                   int cols_cta, double* __restrict__ rowpart);
 // MARG (the fusion of llava.py:243-255 with new_method.py:215-216, as resize_lanczos_up_kernel<., true>): the mask is
 // not written; column sums go to colpart [b][row tile][Wo], row sums to rowpart [b][x CTA][Ho] (exact integers).
+// One CTA's tile: output rows [y0, y0 + rows_per_tile) x columns [x_base, x_base + 64 n_warps) of one image.  img: the
+// image's [h][w] mask; planes: the tile's byte planes; out_img: the image's [Ho][Wo] mask (!MARG); cp: the column
+// partials of the tile's chunk (indexed by column), rp: the row partials of the CTA's columns (indexed by y - y0).
+// Warps from n_warps on (a ragged CTA is sized for the widest image) only take part in the horizontal pass.
 template <bool MARG>
-__global__ void __launch_bounds__(kMmaMaxWarps * 32)
-resize_lanczos_up_mma_kernel(const uint8_t* __restrict__ src, int h, int w, int Ho, int Wo,
-                             const int2* __restrict__ bx, const int* __restrict__ kx, int ksx,
-                             const int2* __restrict__ by, const int* __restrict__ ky, int ksy,
-                             const uint8_t* __restrict__ planes, int rows_per_tile, uint8_t* __restrict__ dst,
-                             double* __restrict__ colpart, double* __restrict__ rowpart) {
+__device__ __forceinline__ void lanczos_up_mma_tile(const uint8_t* __restrict__ img, int w, int Ho, int Wo,
+                                                    const int2* __restrict__ bx, const int* __restrict__ kx, int ksx,
+                                                    const int2* __restrict__ by, const uint8_t* __restrict__ planes,
+                                                    int rows_per_tile, int n_warps, int x_base, int y0,
+                                                    uint8_t* __restrict__ out_img, double* __restrict__ cp,
+                                                    double* __restrict__ rp) {
     extern __shared__ __align__(16) uint8_t sm_b[];
-    const int n_warps = blockDim.x >> 5, cols_cta = n_warps * kMmaStrip;
-    const int b = blockIdx.z;
-    const int x_base = blockIdx.x * cols_cta;
-    const int y0 = blockIdx.y * rows_per_tile, y1 = min(y0 + rows_per_tile, Ho);
+    const int cols_cta = n_warps * kMmaStrip;
+    const int y1 = min(y0 + rows_per_tile, Ho);
     const int r0 = by[y0].x;
     const int nr = by[y1 - 1].x + by[y1 - 1].y - r0;     // source rows the tile taps: [r0, r0 + nr), nr <= 16
     uint8_t* tmpT = sm_b;                                              // [cols_cta][16]
     uint8_t* apl = tmpT + (size_t)cols_cta * kMmaK;                    // [3][rows_per_tile][16]
     int* rsum = reinterpret_cast<int*>(apl + (size_t)3 * rows_per_tile * kMmaK);   // [rows_per_tile] (MARG)
     uint8_t* in = reinterpret_cast<uint8_t*>(rsum + rows_per_tile);    // [nr][w]
-    const uint8_t* img = src + ((int64_t)b * h + r0) * w;
-    for (int i = threadIdx.x; i < nr * w; i += blockDim.x) in[i] = img[i];
+    const uint8_t* src = img + (int64_t)r0 * w;
+    for (int i = threadIdx.x; i < nr * w; i += blockDim.x) in[i] = src[i];
     {   // the coefficient band of this tile, byte planes (get_planes built them once)
-        const uint4* pl = reinterpret_cast<const uint4*>(planes) + (size_t)blockIdx.y * 3 * rows_per_tile;
+        const uint4* pl = reinterpret_cast<const uint4*>(planes);
         for (int i = threadIdx.x; i < 3 * rows_per_tile; i += blockDim.x) reinterpret_cast<uint4*>(apl)[i] = __ldg(pl + i);
     }
     if (MARG)
@@ -364,8 +363,9 @@ resize_lanczos_up_mma_kernel(const uint8_t* __restrict__ src, int h, int w, int 
     __syncthreads();
     const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, tig = lane & 3;
     const int xs = x_base + wid * kMmaStrip;             // the warp's strip of 64 columns
-    if (!MARG && xs >= Wo) return;
-    if (xs < Wo) {
+    const bool strip = wid < n_warps && xs < Wo;
+    if (!MARG && !strip) return;
+    if (strip) {
     uint32_t bf[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
@@ -373,7 +373,7 @@ resize_lanczos_up_mma_kernel(const uint8_t* __restrict__ src, int h, int w, int 
         bf[j] = *reinterpret_cast<const uint32_t*>(tmpT + (size_t)xl * kMmaK + 4 * tig);
     }
     const bool store_ok = xs + 16 * tig < Wo;            // Wo is a multiple of 16: whole 16-byte groups
-    uint8_t* out = MARG ? nullptr : dst + ((int64_t)b * Ho + y0) * Wo + xs + 16 * tig;
+    uint8_t* out = MARG ? nullptr : out_img + (int64_t)y0 * Wo + xs + 16 * tig;
     // MARG: column sums of the thread's 16 columns over its rows, two columns per register (16-bit lanes:
     // <= 2 rows x 32 blocks x 255); csum[2 m] = columns 4 m, 4 m + 2, csum[2 m + 1] = columns 4 m + 1, 4 m + 3
     uint32_t csum[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
@@ -447,7 +447,6 @@ resize_lanczos_up_mma_kernel(const uint8_t* __restrict__ src, int h, int w, int 
                 hi16 += __shfl_xor_sync(0xffffffffu, hi16, d);
             }
             if (g == 0) {
-                double* cp = colpart + ((int64_t)b * gridDim.y + blockIdx.y) * Wo;
                 const double base = (double)(y1 - y0) * kBaseAttention;
                 const int c = xs + 16 * tig + 4 * (m >> 1) + (m & 1);       // and c + 2
                 if (c < Wo) cp[c] = (double)lo16 + base;
@@ -455,21 +454,45 @@ resize_lanczos_up_mma_kernel(const uint8_t* __restrict__ src, int h, int w, int 
             }
         }
     }
-    }   // xs < Wo
+    }   // strip
     if (MARG) {
+        // the row sums of the CTA's columns: one partial per column range
         __syncthreads();
-        mma_write_row_sums<MARG>(rsum, y1 - y0, b, y0, Ho, Wo, x_base, cols_cta, rowpart);
+        const int cols = min(cols_cta, Wo - x_base);
+        const double row_base = (double)cols * kBaseAttention;
+        for (int i = threadIdx.x; i < y1 - y0; i += blockDim.x) rp[i] = (double)rsum[i] + row_base;
     }
 }
-// MARG: the row sums of the CTA's columns, one partial per CTA column (rowpart [b][x CTA][Ho])
+
 template <bool MARG>
-__device__ __forceinline__ void mma_write_row_sums(const int* rsum, int rows, int b, int y0, int Ho, int Wo, int x_base,
-                                                   int cols_cta, double* __restrict__ rowpart) {
-    if (!MARG) return;
-    const int cols = min(cols_cta, Wo - x_base);
-    const double row_base = (double)cols * kBaseAttention;
-    double* rp = rowpart + ((int64_t)b * gridDim.x + blockIdx.x) * Ho + y0;
-    for (int i = threadIdx.x; i < rows; i += blockDim.x) rp[i] = (double)rsum[i] + row_base;
+__global__ void __launch_bounds__(kMmaMaxWarps * 32)
+resize_lanczos_up_mma_kernel(const uint8_t* __restrict__ src, int h, int w, int Ho, int Wo,
+                             const int2* __restrict__ bx, const int* __restrict__ kx, int ksx,
+                             const int2* __restrict__ by, const uint8_t* __restrict__ planes, int rows_per_tile,
+                             uint8_t* __restrict__ dst, double* __restrict__ colpart, double* __restrict__ rowpart) {
+    const int b = blockIdx.z, y0 = blockIdx.y * rows_per_tile, n_warps = blockDim.x >> 5;
+    lanczos_up_mma_tile<MARG>(src + (int64_t)b * h * w, w, Ho, Wo, bx, kx, ksx, by,
+                              planes + (size_t)blockIdx.y * 3 * rows_per_tile * kMmaK, rows_per_tile, n_warps,
+                              blockIdx.x * n_warps * kMmaStrip, y0, MARG ? nullptr : dst + (int64_t)b * Ho * Wo,
+                              MARG ? colpart + ((int64_t)b * gridDim.y + blockIdx.y) * Wo : nullptr,
+                              MARG ? rowpart + ((int64_t)b * gridDim.x + blockIdx.x) * Ho + y0 : nullptr);
+}
+
+// The marginals variant over a ragged list of masks (attwarp_warp_ragged_from_mask) in one launch: CTA = item
+// (image, row tile << 8 | column CTA) of a host-built table.  Every image keeps the tiles, column CTAs and coefficient
+// planes a call on it alone uses (lanczos_ragged_geometry) and writes its partials where its RaggedAtt says, in the
+// layout the ragged finish kernel reads: [row tiles][W] column and [column CTAs][H] row partials.  So its partials, and
+// its maps, are those of attwarp_maps_from_mask on that image alone, whatever the rest of the list.
+__global__ void __launch_bounds__(kMmaMaxWarps * 32)
+resize_lanczos_up_mma_ragged_kernel(const int2* __restrict__ items, const RaggedAtt* __restrict__ atts,
+                                    const RaggedLanczos* __restrict__ lz, int w, double* __restrict__ part) {
+    const int2 it = items[blockIdx.x];
+    const RaggedAtt& a = atts[it.x];
+    const RaggedLanczos& l = lz[it.x];
+    const int tile = it.y >> 8, xc = it.y & 255, rows = a.chunk_rows, y0 = tile * rows;
+    lanczos_up_mma_tile<true>(static_cast<const uint8_t*>(a.att), w, a.H, a.W, l.bx, l.kx, l.ksx, l.by,
+                              l.planes + (size_t)tile * 3 * rows * kMmaK, rows, l.warps, xc * a.tile_cols, y0, nullptr,
+                              part + a.colpart + (int64_t)tile * a.W, part + a.rowpart + (int64_t)xc * a.H + y0);
 }
 
 // ---- coefficient tables (Resample.c precompute_coeffs + normalize_coeffs_8bpc, Lanczos, support 3) ----
@@ -717,7 +740,7 @@ int launch_lanczos_marginals(const uint8_t* src, int B, int h, int w, int H, int
             const int prc = get_planes(h, H, mg.rows, &planes);
             if (prc != ATTWARP_OK) return prc;
             resize_lanczos_up_mma_kernel<true><<<dim3(mg.x_ctas, mg.n_tiles, B), mg.warps * 32, mg.smem, st>>>(
-                src, h, w, H, W, tx.bounds, tx.weights, tx.ksize, ty.bounds, ty.weights, ty.ksize, planes, mg.rows, nullptr, colpart, rowpart);
+                src, h, w, H, W, tx.bounds, tx.weights, tx.ksize, ty.bounds, planes, mg.rows, nullptr, colpart, rowpart);
             *n_chunks = mg.n_tiles;
             *n_col_tiles = mg.x_ctas;
             return check_launch("resize_lanczos_up_mma_kernel<marginals>");
@@ -742,6 +765,46 @@ int launch_lanczos_marginals(const uint8_t* src, int B, int h, int w, int H, int
     return check_launch("resize_lanczos_up_kernel<marginals>");
 }
 
+// The route launch_lanczos_marginals takes for B = 1, restated without the device: the tensor-core kernel when it is
+// enabled and its geometry fits (an up-scaling has 7 taps per axis, within kUpTaps).
+bool lanczos_ragged_geometry(int h, int w, int H, int W, int* rows, int* n_tiles, int* x_ctas, int* warps, size_t* smem) {
+    if (H <= h || W <= w || h > 0xffff || w > 0xffff || !lanczos_mma_enabled()) return false;
+    const MmaGeometry mg = mma_geometry(1, h, w, H, W, nullptr, true);
+    if (!mg.ok || mg.x_ctas > 255) return false;
+    *rows = mg.rows;
+    *n_tiles = mg.n_tiles;
+    *x_ctas = mg.x_ctas;
+    *warps = mg.warps;
+    *smem = mg.smem;
+    return true;
+}
+
+int lanczos_ragged_tables(int h, int w, int H, int W, int rows, RaggedLanczos* l) {
+    CoeffTable tx, ty;
+    int rc = get_table(w, W, &tx);
+    if (rc != ATTWARP_OK) return rc;
+    rc = get_table(h, H, &ty);
+    if (rc != ATTWARP_OK) return rc;
+    if (tx.ksize > kUpTaps || ty.ksize > kUpTaps)
+        return fail(ATTWARP_ERR_UNSUPPORTED, "lanczos_marginals: %dx%d -> %dx%d has more than %d taps", h, w, H, W, kUpTaps);
+    l->bx = tx.bounds;
+    l->kx = tx.weights;
+    l->ksx = tx.ksize;
+    l->by = ty.bounds;
+    return get_planes(h, H, rows, &l->planes);
+}
+
+int launch_lanczos_marginals_ragged(const int2* dev_items, int64_t n_items, const RaggedAtt* dev_att,
+                                    const RaggedLanczos* dev_lz, int w, size_t smem, double* partials, cudaStream_t st) {
+    if (n_items <= 0 || n_items > 0x7fffffff)
+        return fail(ATTWARP_ERR_UNSUPPORTED, "lanczos_marginals_ragged: %lld work items", (long long)n_items);
+    if (smem > 48 * 1024)
+        AW_CUDA(cudaFuncSetAttribute(resize_lanczos_up_mma_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    resize_lanczos_up_mma_ragged_kernel<<<(unsigned)n_items, kMmaMaxWarps * 32, smem, st>>>(dev_items, dev_att, dev_lz, w,
+                                                                                           partials);
+    return check_launch("resize_lanczos_up_mma_ragged_kernel");
+}
+
 int launch_resize_lanczos_u8(const uint8_t* src, int B, int h, int w, int Ho, int Wo, uint8_t* dst, cudaStream_t st) {
     CoeffTable tx, ty;
     if (Wo != w) {
@@ -762,7 +825,7 @@ int launch_resize_lanczos_u8(const uint8_t* src, int B, int h, int w, int Ho, in
             const int prc = get_planes(h, Ho, mg.rows, &planes);
             if (prc != ATTWARP_OK) return prc;
             resize_lanczos_up_mma_kernel<false><<<dim3(mg.x_ctas, mg.n_tiles, B), mg.warps * 32, mg.smem, st>>>(
-                src, h, w, Ho, Wo, tx.bounds, tx.weights, tx.ksize, ty.bounds, ty.weights, ty.ksize, planes, mg.rows, dst, nullptr, nullptr);
+                src, h, w, Ho, Wo, tx.bounds, tx.weights, tx.ksize, ty.bounds, planes, mg.rows, dst, nullptr, nullptr);
             return check_launch("resize_lanczos_up_mma_kernel");
         }
     }

@@ -145,11 +145,25 @@ def encode_png_batch(images: Sequence[torch.Tensor], paths: Sequence[str], worke
         return list(ex.map(write, range(len(paths))))
 
 
+def _mota_masks(tok: torch.Tensor, imgs: Sequence[torch.Tensor]) -> List[torch.Tensor]:
+    """blend_mask's uint8 mask of each image's size (``ops.mota_mask`` per image): one revise_mask launch, then one
+    LANCZOS resize per distinct image size."""
+    _, u8 = ops.revise_mask(tok, return_u8=True)
+    groups = {}
+    for k, im in enumerate(imgs):
+        groups.setdefault((int(im.shape[0]), int(im.shape[1])), []).append(k)
+    masks: List[Optional[torch.Tensor]] = [None] * len(imgs)
+    for hw, idx in groups.items():
+        for k, m in zip(idx, ops.resize_lanczos_u8(u8[idx], hw).unbind(0)):
+            masks[k] = m
+    return masks  # type: ignore[return-value]
+
+
 def warp_files(image_sources: Sequence, tok: Optional[torch.Tensor], output_paths: Sequence[str], out_sizes=None,
                transform: str = "identity", exp_scale: float = 1.0, exp_divisor: float = 1.0,
                apply_inverse: bool = False, device=None, workers: int = 8, on_device_png: bool = False,
                overlay_paths: Optional[Sequence[str]] = None, original_paths: Optional[Sequence[str]] = None,
-               overlay_alpha: float = 0.5, att=None) -> List[bool]:
+               overlay_alpha: float = 0.5, att=None, mask: str = "index") -> List[bool]:
     """The per-image loop of the batched driver (main_batched.py:243-287: ``save_warped_image(image, mask, ...,
     width, height, "identity")`` per sample) for a list of image files and their token maps: GPU decode -> stages
     2-5 for the whole (mixed-resolution) list in one launch per stage -> PNG files.
@@ -160,6 +174,10 @@ def warp_files(image_sources: Sequence, tok: Optional[torch.Tensor], output_path
                 uint8 / float32 / float64, one dtype): the reference's own input, e.g. ``blend_mask``'s uint8 mask or
                 ``ops.mota_mask`` per image; warped with ``ops.warp_ragged_from_attention``.  Exactly one of
                 ``tok`` / ``att``.
+    mask        how ``tok`` becomes each image's attention: ``"index"`` upsamples the token map (nearest index, as
+                above); ``"mota"`` is the drivers' own ``blend_mask`` mask -- revise_mask, then Pillow's LANCZOS
+                resize to each image's size -- warped with ``ops.warp_ragged_from_mota_tokens`` (identity transform
+                only), and the overlays are drawn from that mask as ``save_warped_image`` draws them
     out_sizes   per-image (height, width) of the warped files, default = the input sizes (the drivers pass the
                 sample's own size, main_batched.py:276-287)
     on_device_png  encode the files on the GPU (``encode_png_batch(on_device=True)``): same pixels, other bytes
@@ -180,6 +198,10 @@ def warp_files(image_sources: Sequence, tok: Optional[torch.Tensor], output_path
     for name, paths in (("overlay_paths", overlay_paths), ("original_paths", original_paths)):
         if paths is not None and len(paths) != n:
             raise ValueError(f"warp_files: {len(paths)} {name} for {n} images")
+    if mask not in ("index", "mota"):
+        raise ValueError(f"warp_files: mask must be 'index' or 'mota', got {mask!r}")
+    if mask == "mota" and (tok is None or transform != "identity"):
+        raise ValueError("warp_files: mask='mota' takes token maps and the identity transform (blend_mask's flow)")
     if n == 0:
         return []
     imgs = decode_jpeg_batch(image_sources, device)
@@ -189,6 +211,9 @@ def warp_files(image_sources: Sequence, tok: Optional[torch.Tensor], output_path
                 for a in att]
         outs = ops.warp_ragged_from_attention(maps, imgs, out_sizes, transform=transform, exp_scale=exp_scale,
                                               exp_divisor=exp_divisor, apply_inverse=apply_inverse)
+    elif mask == "mota":
+        tok = tok.to(dev).reshape(n, tok.shape[-2], tok.shape[-1]).float()
+        outs = ops.warp_ragged_from_mota_tokens(tok, imgs, out_sizes, apply_inverse=apply_inverse)
     else:
         tok = tok.to(dev)
         outs = ops.warp_ragged_from_tokens(tok, imgs, out_sizes, transform=transform, exp_scale=exp_scale,
@@ -197,6 +222,8 @@ def warp_files(image_sources: Sequence, tok: Optional[torch.Tensor], output_path
     if overlay_paths is not None:
         if att is not None:
             images += ops.attention_overlay(imgs, att=maps, alpha=overlay_alpha)
+        elif mask == "mota":
+            images += ops.attention_overlay(imgs, att=_mota_masks(tok, imgs), alpha=overlay_alpha)
         else:
             images += ops.attention_overlay(imgs, tok=tok.reshape(n, tok.shape[-2], tok.shape[-1]).float(),
                                             alpha=overlay_alpha)

@@ -564,6 +564,68 @@ def warp_ragged_from_attention(att, images, out_sizes=None, transform="identity"
     return (outs, map_xs, map_ys) if return_maps else outs
 
 
+def warp_ragged_from_mota_tokens(tok: torch.Tensor, images, out_sizes=None, kernel_size: int = 3,
+                                 enhance_coe: float = 10.0, apply_inverse: bool = False, return_maps: bool = False):
+    """The drivers' flow for a mixed-size list: per image ``blend_mask`` (revise_mask -> uint8 -> Pillow LANCZOS resize
+    to that image's own size, llava.py:240-256) then ``save_warped_image(..., "identity")`` -- one ``revise_mask``
+    launch for all token maps, then ``attwarp_warp_ragged_from_mask``: one fused LANCZOS + marginals launch, one finish
+    launch and the stage-5 launches of ``warp_ragged_from_tokens``.
+
+    tok     [n, gh, gw] float32 token maps on the device
+    images  sequence of n uint8 HWC tensors [H_i, W_i, C], C in {1, 3, 4}, on the same device
+    out_sizes  sequence of (Ho_i, Wo_i), default = input sizes
+    Returns the list of warped images, and with ``return_maps`` also the lists of map_x [Wo_i] and map_y [Ho_i].
+    An image's maps are bit-identical to ``maps_from_mota_tokens`` on that image alone (images the fused kernel does not
+    take -- down-scaling, smaller than the token grid -- are resized first, as that call does)."""
+    lib = load()
+    n = len(images)
+    if not isinstance(tok, torch.Tensor) or tok.dim() != 3:
+        raise ValueError("warp_ragged_from_mota_tokens: tok must be a [n, gh, gw] tensor")
+    if tok.shape[0] != n:
+        raise ValueError(f"warp_ragged_from_mota_tokens: {tok.shape[0]} token maps for {n} images")
+    if n == 0:
+        return ([], [], []) if return_maps else []
+    require_cuda(tok, *images)
+    dev = tok.device
+    Cc = images[0].shape[2] if images[0].dim() == 3 else 0
+    if Cc not in (1, 3, 4):
+        raise ValueError(f"warp_ragged_from_mota_tokens: images must be uint8 [H, W, C] with C in (1, 3, 4), got "
+                         f"{tuple(images[0].shape)}")
+    imgs = [im.contiguous() for im in images]
+    if out_sizes is None:
+        out_sizes = [(im.shape[0], im.shape[1]) for im in imgs]
+    if len(out_sizes) != n:
+        raise ValueError(f"warp_ragged_from_mota_tokens: {len(out_sizes)} output sizes for {n} images")
+    outs = [torch.empty(int(ho), int(wo), Cc, dtype=torch.uint8, device=dev) for ho, wo in out_sizes]
+    for im in imgs:
+        if im.dtype != torch.uint8 or im.dim() != 3 or im.shape[2] != Cc or im.device != dev:
+            raise ValueError("warp_ragged_from_mota_tokens: images must be uint8 HWC tensors with the same channel "
+                             "count on the token maps' device")
+    _, u8 = revise_mask(tok, kernel_size, enhance_coe, return_u8=True)
+    gh, gw = int(u8.shape[1]), int(u8.shape[2])
+    table = np.empty(n, dtype=_RAGGED_DTYPE)
+    table["src"] = [im.data_ptr() for im in imgs]
+    table["dst"] = [o.data_ptr() for o in outs]
+    table["H"] = [im.shape[0] for im in imgs]
+    table["W"] = [im.shape[1] for im in imgs]
+    table["Ho"] = [hw[0] for hw in out_sizes]
+    table["Wo"] = [hw[1] for hw in out_sizes]
+    map_x = map_y = None
+    if return_maps:
+        map_x = torch.empty(int(table["Wo"].sum()), dtype=torch.float32, device=dev)
+        map_y = torch.empty(int(table["Ho"].sum()), dtype=torch.float32, device=dev)
+    table_p = table.ctypes.data_as(C.c_void_p)           # `table` stays alive until the call returns
+    tp = _tp("identity", 1.0, 1.0, apply_inverse)
+    wsb = lib.attwarp_ragged_mask_workspace_bytes(table_p, n, gh, gw)
+    ws = _workspace(wsb, dev)
+    with torch.cuda.device(dev):
+        check(lib.attwarp_warp_ragged_from_mask(table_p, ptr(u8), n, gh, gw, Cc, C.byref(tp), ptr(ws), ws.numel(),
+                                                ptr(map_x), ptr(map_y), current_stream(dev)))
+    if not return_maps:
+        return outs
+    return (outs, list(map_x.split([int(w) for w in table["Wo"]])), list(map_y.split([int(h) for h in table["Ho"]])))
+
+
 class RaggedBatch:
     """A mixed-resolution batch whose buffers stay put across calls (the steady state of a driver that re-uses its
     image and output buffers): the descriptor table, the output tensors and a private workspace are built ONCE,

@@ -275,10 +275,37 @@ int attwarp_warp_ragged_from_attention(const attwarp_ragged_image* images, const
                                        int n, int att_dtype, int C, const attwarp_transform_params* tp,
                                        void* workspace, size_t workspace_bytes, void* stream);
 
-/* Kernel launches the calling thread's last attwarp_warp_ragged_from_tokens / attwarp_warp_ragged_from_attention
- * call enqueued: the maps launches (tokens: one; attention: marginals + finish) + one stage-5 launch per non-empty
- * class (images are grouped by the consumer warps their strips need and by whether their destination rows are
- * 4-byte aligned).  For accounting (bench.py's gpu_launches). */
+/* Ragged batch warped by the drivers' own attention, built from token maps: per image blend_mask's uint8 mask
+ * (revise_mask, then Pillow's LANCZOS resize to the image's own size; llava.py:240-256) followed by
+ * save_warped_image(..., "identity") (new_method.py:207-283), for a mixed-size list -- attwarp_maps_from_mask for
+ * every image, with one launch per stage for the whole list and no image-size mask written for the images the fused
+ * kernel takes.
+ *
+ * images    : as for attwarp_warp_ragged_from_tokens
+ * mask_u8   : device [n][gh][gw] uint8, attwarp_revise_mask's uint8 output for the n token maps
+ * tp        : identity transform only (apply_inverse 0 or 1); ATTWARP_ERR_UNSUPPORTED otherwise
+ * workspace : attwarp_ragged_mask_workspace_bytes(images, n, gh, gw) bytes of device scratch (0: invalid sizes)
+ * map_x_opt : NULL, or device floats [sum of Wo]: receives the images' map_x rows back to back, in list order
+ * map_y_opt : NULL, or device floats [sum of Ho]: the same for map_y
+ * An image whose resize attwarp_maps_from_mask takes on the tensor cores (an up-scaling of both axes that fits its
+ * tiles) keeps the tiles, coefficients and partial sums of a call on that image alone, so its maps are bit-identical
+ * to attwarp_maps_from_mask on that image; the others (down-scaling, image smaller than the token grid, ...) are
+ * resized with attwarp_resize_lanczos_u8 into the workspace and summed with the marginals kernel of
+ * attwarp_warp_ragged_from_attention.  Then one finish launch for all images and the stage-5 launches of
+ * attwarp_warp_ragged_from_tokens.  Images with H or W below 2 make the call go image by image.  The coefficient
+ * tables are built on the host and uploaded once per size and device, like attwarp_maps_from_mask's.  Host-side
+ * descriptor tables: ATTWARP_ERR_UNSUPPORTED under CUDA-graph capture. */
+size_t attwarp_ragged_mask_workspace_bytes(const attwarp_ragged_image* images, int n, int gh, int gw);
+int attwarp_warp_ragged_from_mask(const attwarp_ragged_image* images, const void* mask_u8, int n, int gh, int gw, int C,
+                                  const attwarp_transform_params* tp, void* workspace, size_t workspace_bytes,
+                                  float* map_x_opt, float* map_y_opt, void* stream);
+
+/* Kernel launches the calling thread's last attwarp_warp_ragged_from_tokens / attwarp_warp_ragged_from_attention /
+ * attwarp_warp_ragged_from_mask call enqueued: the maps launches (tokens: one; attention: marginals + finish; mask:
+ * one resize per image the fused kernel does not take, the fused marginals, the uint8 marginals when some image
+ * needs them, finish) + one stage-5 launch per non-empty class (images are grouped by the consumer warps their
+ * strips need and by whether their destination rows are 4-byte aligned).  For accounting (bench.py's
+ * gpu_launches). */
 int attwarp_ragged_last_launches(void);
 
 /* attwarp_warp_image_host: the whole of warp_image_by_attention (AGW/new_method.py:198-283) for
