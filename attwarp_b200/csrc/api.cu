@@ -9,6 +9,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "jpeg_decode.h"
 
 namespace aw {
 
@@ -42,6 +43,9 @@ size_t png_max_bytes_impl(int H, int W, int C);
 size_t png_workspace_bytes_impl(const attwarp_png_image* images, int n);
 int launch_encode_png(const attwarp_png_image* images, int n, void* ws, uint8_t* out, int64_t* offsets,
                       cudaStream_t st);
+size_t jpeg_workspace_bytes_impl(const jpeg::Header* headers, int n);
+int launch_decode_jpeg(const attwarp_jpeg_image* images, const jpeg::Header* headers, int n, void* ws,
+                       int32_t* status, cudaStream_t st);
 int launch_interp_linear_rows(const float* F, int B, int N, int L, float* out, cudaStream_t st);
 size_t overlay_workspace_bytes_impl(const attwarp_overlay_image* images, int n, int att_kind);
 int launch_attention_overlay(const attwarp_overlay_image* images, int n, int att_dtype, int att_kind, int gh, int gw,
@@ -814,6 +818,59 @@ int attwarp_encode_png(const attwarp_png_image* images, int n, void* workspace, 
     if (cap != cudaStreamCaptureStatusNone)
         return fail(ATTWARP_ERR_UNSUPPORTED, "encode_png: cannot be captured into a CUDA graph (host-side descriptor table)");
     return launch_encode_png(images, n, workspace, static_cast<uint8_t*>(out), offsets, st);
+}
+
+// ---------------------------------------------------------------------------------------------
+int attwarp_jpeg_probe(const void* bytes, size_t nbytes, attwarp_jpeg_info* info) {
+    AW_REQUIRE(bytes && info, "jpeg_probe: NULL pointer");
+    aw::jpeg::Header h;
+    aw::jpeg::parse_header(static_cast<const uint8_t*>(bytes), nbytes, &h);
+    info->H = h.H;
+    info->W = h.W;
+    info->components = h.ncomp;
+    info->support = h.support;
+    return ATTWARP_OK;
+}
+
+// the headers of `images`, parsed into a per-thread vector; ATTWARP_OK when every image is device-decodable
+static int jpeg_headers(const attwarp_jpeg_image* images, int n, std::vector<aw::jpeg::Header>& hs) {
+    hs.resize((size_t)n);
+    for (int i = 0; i < n; ++i) {
+        const attwarp_jpeg_image& im = images[i];
+        AW_REQUIRE(im.host && im.dev && im.dst, "decode_jpeg: image %d: NULL pointer", i);
+        const int s = aw::jpeg::parse_header(static_cast<const uint8_t*>(im.host), im.nbytes, &hs[(size_t)i]);
+        if (s != aw::jpeg::kOk)
+            return fail(ATTWARP_ERR_UNSUPPORTED, "decode_jpeg: image %d is not device-decodable (support code %d)", i, s);
+        AW_REQUIRE(im.H == hs[(size_t)i].H && im.W == hs[(size_t)i].W,
+                   "decode_jpeg: image %d: dst is %d x %d, the file is %d x %d", i, im.H, im.W, hs[(size_t)i].H,
+                   hs[(size_t)i].W);
+    }
+    return ATTWARP_OK;
+}
+
+size_t attwarp_jpeg_workspace_bytes(const attwarp_jpeg_image* images, int n) {
+    if (images == nullptr || n <= 0) return 0;
+    static thread_local std::vector<aw::jpeg::Header> hs;
+    if (jpeg_headers(images, n, hs) != ATTWARP_OK) return 0;
+    return jpeg_workspace_bytes_impl(hs.data(), n);
+}
+
+int attwarp_decode_jpeg(const attwarp_jpeg_image* images, int n, void* workspace, size_t workspace_bytes,
+                        int32_t* status_out, void* stream) {
+    AW_REQUIRE(images && status_out, "decode_jpeg: NULL pointer");
+    AW_REQUIRE(n > 0, "decode_jpeg: n must be positive (got %d)", n);
+    static thread_local std::vector<aw::jpeg::Header> hs;
+    const int rc = jpeg_headers(images, n, hs);
+    if (rc != ATTWARP_OK) return rc;
+    const size_t need = jpeg_workspace_bytes_impl(hs.data(), n);
+    if (workspace == nullptr || workspace_bytes < need)
+        return fail(ATTWARP_ERR_WORKSPACE, "decode_jpeg: workspace too small (%zu < %zu)", workspace_bytes, need);
+    cudaStream_t st = as_stream(stream);
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    AW_CUDA(cudaStreamIsCapturing(st, &cap));
+    if (cap != cudaStreamCaptureStatusNone)
+        return fail(ATTWARP_ERR_UNSUPPORTED, "decode_jpeg: cannot be captured into a CUDA graph (host-side descriptor table)");
+    return launch_decode_jpeg(images, hs.data(), n, workspace, status_out, st);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -13,6 +13,16 @@ batches the rest:
   (nvJPEG replicates chroma samples where libjpeg's "fancy" up-sampling interpolates them).  ``exact=True`` decodes
   on the host with Pillow instead -- bit-identical to ``Image.open(path).convert('RGB')`` -- for runs that must
   reproduce the reference's pixels.  Anything that is not a JPEG (PNG, ...) is decoded on the host, exactly.
+  ``exact_device=True`` gives the same pixels as ``exact=True`` with the JPEG decode on the GPU (``ops.decode_jpeg``,
+  csrc/jpeg.cu: seven launches for the whole mixed-size list, only the compressed bytes cross PCIe): libjpeg-turbo's
+  Huffman decode, ISLOW IDCT with its range-limit table, fancy h2v1 / h2v2 / h1v2 up-sampling (replication for
+  4:1:1 and for chroma 2 samples wide or less) and ycc_rgb_convert, restated.  It takes baseline / extended
+  sequential Huffman files with 8-bit samples, one interleaved scan (or one grey component), YCbCr (JFIF, or
+  component IDs 1/2/3) or grey, luma sampling 4:4:4, 4:2:2, 4:2:0, 4:4:0 or 4:1:1, any restart interval, any
+  tables, APPn / COM / EXIF skipped (no rotation, like Pillow's open).  Other JPEGs (progressive, arithmetic,
+  12-bit, CMYK / YCCK / RGB, multi-scan, ...) go to Pillow and other formats to cv2, both exact; ``ops.jpeg_probe``
+  tells which path a file takes.  A file whose entropy-coded data is malformed raises ValueError naming it (Pillow
+  would recover from some such files with a warning; the device decoder never guesses pixels).
 * ``encode_png_batch(images, paths)`` device tensors -> PNG files: device -> pinned host copy, then
   ``cv2.imwrite`` in a thread pool -- the reference's own encoder, so the files decode to the same bytes.
   ``on_device=True`` encodes on the GPU instead (``encode_png_device``, ``ops.encode_png``: two launches for the
@@ -59,22 +69,41 @@ def _is_jpeg(buf: bytes) -> bool:
     return len(buf) > 3 and buf[0] == 0xFF and buf[1] == 0xD8
 
 
-def decode_jpeg_batch(sources: Sequence, device=None, exact: bool = False) -> List[torch.Tensor]:
+def _pillow_bgr(b: bytes, dev) -> torch.Tensor:
+    import io
+
+    from PIL import Image
+    rgb = np.array(Image.open(io.BytesIO(b)).convert("RGB"))
+    return torch.from_numpy(np.ascontiguousarray(rgb[..., ::-1])).to(dev, non_blocking=True)
+
+
+def decode_jpeg_batch(sources: Sequence, device=None, exact: bool = False,
+                      exact_device: bool = False) -> List[torch.Tensor]:
     """Paths or encoded bytes -> list of uint8 [H, W, 3] BGR tensors on ``device`` (cv2.imread's channel order, the
     one ``save_warped_image`` warps in).  JPEG files are decoded on the GPU in one batched nvJPEG call; grey JPEGs
     come out as three equal channels (like ``Image.convert('RGB')``).  ``exact=True``: host decode with Pillow,
-    bit-identical to the reference's reader, then one copy to the device."""
+    bit-identical to the reference's reader, then one copy to the device.  ``exact_device=True``: bit-identical too,
+    with the JPEGs ``ops.jpeg_probe`` accepts decoded on the GPU in one ``ops.decode_jpeg`` call; other JPEGs
+    (progressive, CMYK, ...) are decoded by Pillow and other formats by cv2, as without the keyword."""
+    if exact and exact_device:
+        raise ValueError("decode_jpeg_batch: exact and exact_device are exclusive")
     dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
     bufs = [_read_bytes(s) for s in sources]
     out: List[Optional[torch.Tensor]] = [None] * len(bufs)
     if exact:
-        import io
-
-        from PIL import Image
         for i, b in enumerate(bufs):
-            rgb = np.array(Image.open(io.BytesIO(b)).convert("RGB"))
-            out[i] = torch.from_numpy(np.ascontiguousarray(rgb[..., ::-1])).to(dev, non_blocking=True)
+            out[i] = _pillow_bgr(b, dev)
         return out  # type: ignore[return-value]
+    if exact_device:
+        jpegs = [i for i, b in enumerate(bufs) if _is_jpeg(b)]
+        dev_idx = [i for i in jpegs if ops.jpeg_probe(bufs[i])[3] == 0]
+        if dev_idx:
+            for i, t in zip(dev_idx, ops.decode_jpeg([bufs[i] for i in dev_idx], dev)):
+                out[i] = t
+        for i in jpegs:
+            if out[i] is None:
+                out[i] = _pillow_bgr(bufs[i], dev)
+        return _decode_others(bufs, out, dev)
     from torchvision.io import ImageReadMode, decode_jpeg
     jpeg_idx = [i for i, b in enumerate(bufs) if _is_jpeg(b)]
     if jpeg_idx:
@@ -82,6 +111,11 @@ def decode_jpeg_batch(sources: Sequence, device=None, exact: bool = False) -> Li
         decoded = decode_jpeg(datas, mode=ImageReadMode.RGB, device=dev)          # list of [3, H, W] RGB
         for i, t in zip(jpeg_idx, decoded):
             out[i] = t.flip(0).permute(1, 2, 0).contiguous()                      # -> [H, W, 3] BGR
+    return _decode_others(bufs, out, dev)
+
+
+def _decode_others(bufs, out, dev) -> List[torch.Tensor]:
+    """cv2.imdecode (exact) of the sources not decoded yet."""
     for i, b in enumerate(bufs):
         if out[i] is None:
             import cv2
@@ -163,7 +197,7 @@ def warp_files(image_sources: Sequence, tok: Optional[torch.Tensor], output_path
                transform: str = "identity", exp_scale: float = 1.0, exp_divisor: float = 1.0,
                apply_inverse: bool = False, device=None, workers: int = 8, on_device_png: bool = False,
                overlay_paths: Optional[Sequence[str]] = None, original_paths: Optional[Sequence[str]] = None,
-               overlay_alpha: float = 0.5, att=None, mask: str = "index") -> List[bool]:
+               overlay_alpha: float = 0.5, att=None, mask: str = "index", exact_decode: bool = False) -> List[bool]:
     """The per-image loop of the batched driver (main_batched.py:243-287: ``save_warped_image(image, mask, ...,
     width, height, "identity")`` per sample) for a list of image files and their token maps: GPU decode -> stages
     2-5 for the whole (mixed-resolution) list in one launch per stage -> PNG files.
@@ -187,6 +221,8 @@ def warp_files(image_sources: Sequence, tok: Optional[torch.Tensor], output_path
                    (the drivers' 0.5)
     original_paths also write, per image, the decoded image: save_warped_image's ``original_image_save_path``.
                    With nvJPEG decode these are nvJPEG's pixels (module docstring), not libjpeg's
+    exact_decode   decode with ``decode_jpeg_batch(exact_device=True)``: the images are Pillow's pixels, bit for bit,
+                   so the warped, overlay and original files are those of the reference's reader
     Every file goes through one encoder call (one ``ops.encode_png`` with ``on_device_png``, else one cv2.imwrite
     pool).  Returns one bool per file written, grouped per kind: the n warped files, then the n overlays if
     ``overlay_paths`` is given, then the n originals if ``original_paths`` is given -- a list of n, 2n or 3n."""
@@ -204,7 +240,7 @@ def warp_files(image_sources: Sequence, tok: Optional[torch.Tensor], output_path
         raise ValueError("warp_files: mask='mota' takes token maps and the identity transform (blend_mask's flow)")
     if n == 0:
         return []
-    imgs = decode_jpeg_batch(image_sources, device)
+    imgs = decode_jpeg_batch(image_sources, device, exact_device=exact_decode)
     dev = imgs[0].device
     if att is not None:
         maps = [torch.from_numpy(np.ascontiguousarray(a)).to(dev) if isinstance(a, np.ndarray) else a.to(dev)

@@ -746,6 +746,81 @@ def encode_png(images):
 
 
 # --------------------------------------------------------------------------------------------
+# Baseline JPEG decode, bit-identical to Pillow (the reference drivers' reader)
+# --------------------------------------------------------------------------------------------
+# attwarp_jpeg_info / attwarp_jpeg_image (include/attwarp.h)
+_JPEG_INFO_DTYPE = np.dtype([("H", np.int32), ("W", np.int32), ("components", np.int32), ("support", np.int32)])
+_JPEG_DTYPE = np.dtype([("host", np.uint64), ("dev", np.uint64), ("nbytes", np.uint64), ("dst", np.uint64),
+                        ("H", np.int32), ("W", np.int32)])
+JPEG_SUPPORT_REASONS = {1: "not a JPEG file", 2: "truncated markers", 3: "progressive", 4: "arithmetic-coded",
+                        5: "lossless or hierarchical", 6: "12-bit samples or 16-bit quantisation tables",
+                        7: "colour space other than grey / YCbCr", 8: "sampling factors",
+                        9: "multi-scan, DNL or data after EOI", 10: "missing or invalid table", 11: "size"}
+JPEG_STATUS_REASONS = {1: "entropy-coded data ends before the last block", 2: "invalid Huffman code",
+                       3: "coefficient index past 63", 4: "restart marker missing or out of order",
+                       5: "unexpected marker inside the entropy-coded data"}
+
+
+def jpeg_probe(buf) -> tuple:
+    """(H, W, components, support) of a file's bytes from its markers, on the host (no GPU).  support 0: the file
+    is one ``decode_jpeg`` takes; otherwise a key of ``JPEG_SUPPORT_REASONS``."""
+    data = np.frombuffer(bytes(buf), dtype=np.uint8)
+    info = np.zeros(1, dtype=_JPEG_INFO_DTYPE)
+    check(load().attwarp_jpeg_probe(data.ctypes.data_as(C.c_void_p), data.size, info.ctypes.data_as(C.c_void_p)))
+    return tuple(int(info[0][k]) for k in ("H", "W", "components", "support"))
+
+
+def decode_jpeg(buffers, device=None):
+    """Baseline JPEG files (a sequence of bytes-like objects) -> list of uint8 [H, W, 3] **BGR** CUDA tensors,
+    bit-identical to ``np.array(Image.open(f).convert('RGB'))[..., ::-1]`` (Pillow's libjpeg-turbo: ISLOW IDCT,
+    fancy up-sampling); grey files come out as three equal channels.  The whole list is decoded on the GPU in seven
+    launches: only the compressed bytes are copied to the device (one copy from pinned memory).
+
+    Raises ValueError naming the first file ``jpeg_probe`` does not accept (see include/attwarp.h for the subset),
+    and, after one synchronisation that reads the per-file status, the first file whose entropy-coded data is
+    malformed (no pixels of such a file are returned)."""
+    lib = load()
+    dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    bufs = [bytes(b) for b in buffers]
+    n = len(bufs)
+    if n == 0:
+        return []
+    infos = [jpeg_probe(b) for b in bufs]
+    for i, (_, _, _, sup) in enumerate(infos):
+        if sup != 0:
+            raise ValueError(f"decode_jpeg: file {i} is not device-decodable: "
+                             f"{JPEG_SUPPORT_REASONS.get(sup, sup)} (support code {sup})")
+    sizes = [len(b) for b in bufs]
+    offs = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
+    host = torch.empty(int(offs[-1]), dtype=torch.uint8, pin_memory=True)
+    hv = host.numpy()
+    for b, o in zip(bufs, offs[:-1]):
+        hv[o:o + len(b)] = np.frombuffer(b, dtype=np.uint8)
+    with torch.cuda.device(dev):
+        data = host.to(dev, non_blocking=True)
+        outs = [torch.empty((h, w, 3), dtype=torch.uint8, device=dev) for h, w, _, _ in infos]
+        status = torch.empty(n, dtype=torch.int32, device=dev)
+        table = np.zeros(n, dtype=_JPEG_DTYPE)
+        table["host"] = host.data_ptr() + offs[:-1]
+        table["dev"] = data.data_ptr() + offs[:-1]
+        table["nbytes"] = sizes
+        table["dst"] = [t.data_ptr() for t in outs]
+        table["H"] = [h for h, _, _, _ in infos]
+        table["W"] = [w for _, w, _, _ in infos]
+        table_p = table.ctypes.data_as(C.c_void_p)
+        wsb = lib.attwarp_jpeg_workspace_bytes(table_p, n)
+        ws = _workspace(wsb, dev)
+        check(lib.attwarp_decode_jpeg(table_p, n, ptr(ws), ws.numel(), ptr(status), current_stream(dev)))
+        st = status.cpu().numpy()                      # synchronises: the decode (and the upload) have run
+    bad = np.nonzero(st)[0]
+    if bad.size:
+        i = int(bad[0])
+        raise ValueError(f"decode_jpeg: file {i} has malformed entropy-coded data: "
+                         f"{JPEG_STATUS_REASONS.get(int(st[i]), int(st[i]))} (status {int(st[i])})")
+    return outs
+
+
+# --------------------------------------------------------------------------------------------
 # Attention overlay (save_warped_image's masked_overlay_save_path image)
 # --------------------------------------------------------------------------------------------
 # attwarp_overlay_image (include/attwarp.h)

@@ -389,6 +389,75 @@ size_t attwarp_overlay_workspace_bytes(const attwarp_overlay_image* images_host,
 int attwarp_attention_overlay(const attwarp_overlay_image* images_host, int n, int att_dtype, int att_kind, int gh,
                               int gw, double alpha, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Baseline JPEG decode of n files of any sizes in a fixed number of launches, bit-identical to
+ * Image.open(path).convert('RGB') with Pillow's libjpeg-turbo (ISLOW IDCT, fancy up-sampling) --
+ * how the reference drivers read their images (AGW/main.py:152) -- in cv2.imread's BGR order.
+ *
+ * Device-decodable files (attwarp_jpeg_probe's support code ATTWARP_JPEG_OK): baseline or extended
+ * sequential Huffman, 8-bit samples, 8-bit quantisation tables; one scan holding every component;
+ * 1 component (grey, written as three equal channels) or 3 (YCbCr: a JFIF marker, or no colour
+ * marker and component IDs 1, 2, 3); luma sampling 1x1, 2x1, 2x2, 1x2 or 4x1 with chroma 1x1 (grey:
+ * any); any restart interval; the entropy-coded data running to an EOI that ends the file.  APPn
+ * and COM markers are skipped (no EXIF rotation, as Pillow's open does not rotate).
+ *
+ * attwarp_jpeg_probe: host only, no GPU.  Parses the markers of bytes[0 .. nbytes) and fills
+ *   *info (H, W, components, support).  Returns ATTWARP_ERR_INVALID_ARG for NULL pointers, else
+ *   ATTWARP_OK whatever the support code.
+ * attwarp_jpeg_workspace_bytes: device scratch one call over `images` needs; 0 when an image is
+ *   not device-decodable or a pointer is NULL.
+ * attwarp_decode_jpeg:
+ *   images     HOST array of n descriptors: host and dev both hold the file's nbytes bytes (the
+ *              host copy is parsed during the call, the device copy is read by the kernels); dst is
+ *              a DEVICE [H][W][3] uint8 buffer at any byte alignment, H and W the file's.  dev and
+ *              dst must stay valid until the stream has run the call.
+ *   status_out DEVICE int32 [n]: per image ATTWARP_JPEG_ST_OK or the reason its entropy-coded data
+ *              is malformed.  The dst of a failed image is left untouched; no pixel of it is guessed.
+ *   Argument errors (NULL, n <= 0, a size mismatch, a file that is not device-decodable: message
+ *   names the image) return before any CUDA call.  The call uploads its descriptor table from host
+ *   memory: ATTWARP_ERR_UNSUPPORTED on a stream that is being captured into a CUDA graph.
+ */
+typedef enum attwarp_jpeg_support {
+    ATTWARP_JPEG_OK = 0,
+    ATTWARP_JPEG_NOT_JPEG = 1,       /* no SOI marker                                          */
+    ATTWARP_JPEG_TRUNCATED = 2,      /* the markers end before the scan                         */
+    ATTWARP_JPEG_PROGRESSIVE = 3,
+    ATTWARP_JPEG_ARITHMETIC = 4,
+    ATTWARP_JPEG_OTHER_PROCESS = 5,  /* lossless, hierarchical                                  */
+    ATTWARP_JPEG_PRECISION = 6,      /* 12-bit samples or 16-bit quantisation tables            */
+    ATTWARP_JPEG_COLOUR = 7,         /* CMYK, YCCK, RGB, Adobe marker, 2 or 4 components        */
+    ATTWARP_JPEG_SAMPLING = 8,
+    ATTWARP_JPEG_STRUCTURE = 9,      /* multi-scan, DNL, data after EOI, misplaced markers      */
+    ATTWARP_JPEG_BAD_TABLE = 10,     /* missing or invalid Huffman / quantisation table         */
+    ATTWARP_JPEG_SIZE = 11           /* zero lines (DNL) or a file of 512 MiB or more           */
+} attwarp_jpeg_support;
+
+typedef enum attwarp_jpeg_status {
+    ATTWARP_JPEG_ST_OK = 0,
+    ATTWARP_JPEG_ST_SHORT_DATA = 1,     /* the data ends before the last block of an interval  */
+    ATTWARP_JPEG_ST_BAD_CODE = 2,       /* a bit pattern that is no code of its Huffman table  */
+    ATTWARP_JPEG_ST_COEF_OVERFLOW = 3,  /* a coefficient index past 63                         */
+    ATTWARP_JPEG_ST_RESTART = 4,        /* an RSTn missing, out of order or extra               */
+    ATTWARP_JPEG_ST_MARKER = 5          /* another marker inside the entropy-coded data        */
+} attwarp_jpeg_status;
+
+typedef struct attwarp_jpeg_info {
+    int32_t H, W, components, support;
+} attwarp_jpeg_info;
+
+typedef struct attwarp_jpeg_image {
+    const void* host;
+    const void* dev;
+    size_t nbytes;
+    void* dst;
+    int32_t H, W;
+} attwarp_jpeg_image;
+
+int attwarp_jpeg_probe(const void* bytes, size_t nbytes, attwarp_jpeg_info* info);
+size_t attwarp_jpeg_workspace_bytes(const attwarp_jpeg_image* images_host, int n);
+int attwarp_decode_jpeg(const attwarp_jpeg_image* images_host, int n, void* workspace, size_t workspace_bytes,
+                        int32_t* status_out, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Stages 2-3, torch path (all float32 [B][N] row-major unless noted).
  */
