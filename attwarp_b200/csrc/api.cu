@@ -100,6 +100,16 @@ static int check_transform(const attwarp_transform_params* tp) {
     return ATTWARP_OK;
 }
 
+// The calls that upload descriptor tables from this thread's host buffers refuse a stream that is being captured into
+// a CUDA graph: a captured copy node would read those buffers at replay time, after later calls have rewritten them.
+static int refuse_graph_capture(cudaStream_t st, const char* what) {
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    AW_CUDA(cudaStreamIsCapturing(st, &cap));
+    if (cap != cudaStreamCaptureStatusNone)
+        return fail(ATTWARP_ERR_UNSUPPORTED, "%s: cannot be captured into a CUDA graph (host-side descriptor tables)", what);
+    return ATTWARP_OK;
+}
+
 // ---- per-thread device scratch for the host-buffer entry point --------------------------------
 struct HostArena {
     cudaStream_t stream = nullptr;
@@ -366,19 +376,100 @@ int attwarp_warp_from_pdfs(const float* px, const float* py, int B, int Nx, int 
     return launch_remap(src, dst, dtype, layout, B, C, H, W, Ho, Wo, map_x, map_y, st);
 }
 
+}  // extern "C" (the ragged helpers below include templates, which cannot have C linkage)
+
 // ---------------------------------------------------------------------------------------------
-// Ragged batch: descriptor table (n + 1 entries) followed by the map rows of every image.
-// (n + 1 entries in batch order, then n + kRaggedClasses entries grouped by width class for the stage-5 launches)
+// Ragged batches.  Every call's workspace starts with the descriptor tables (n + 1 entries in list order, then
+// n + kRaggedClasses entries grouped by width class for the stage-5 launches) and the map rows of every image.
 static size_t ragged_table_bytes(int n) { return align_up(sizeof(RaggedImage) * (size_t)(2 * n + 1 + kRaggedClasses), 256); }
 
-// kernel launches of this thread's last attwarp_warp_ragged_from_tokens call (maps + one resample launch per class)
+// bytes of that shared prefix, 0 when an image has invalid sizes
+static size_t ragged_prefix_bytes(const attwarp_ragged_image* images, int n) {
+    size_t floats = 0;
+    for (int i = 0; i < n; ++i) {
+        const attwarp_ragged_image& im = images[i];
+        if (im.H <= 0 || im.W <= 0 || im.Ho <= 0 || im.Wo <= 0 || im.H >= 65536 || im.W >= 65536) return 0;
+        floats += (size_t)im.Wo + (size_t)im.Ho;
+    }
+    return ragged_table_bytes(n) + align_up(floats * sizeof(float), 256);
+}
+
+// kernel launches of this thread's last ragged call (maps + one resample launch per class)
 static thread_local int g_ragged_last_launches = 0;
+
+// A ragged call's list: the host descriptor table (n + 1 entries, the last one for the stage-5 plan), the device table
+// at the start of the workspace, and what the maps kernels need to know of the whole list.
+struct RaggedList {
+    RaggedImage* host = nullptr;
+    RaggedImage* dev = nullptr;
+    int max_h = 0, max_w = 0;
+    bool degenerate = false;     // an image with a 1-pixel axis: the call goes image by image
+};
+
+// Checks every image and fills the host table in one pass.  Each image's map rows are taken from the workspace pool
+// in list order (the attention and mask calls may point them at the caller's buffers afterwards; the pool keeps its
+// layout either way).
+static int ragged_list(const char* what, const attwarp_ragged_image* images, int n, void* workspace, RaggedList* l) {
+    static thread_local std::vector<RaggedImage> host;
+    host.assign((size_t)n + 1, RaggedImage{});
+    l->host = host.data();
+    l->dev = static_cast<RaggedImage*>(workspace);
+    float* pool = reinterpret_cast<float*>(static_cast<char*>(workspace) + ragged_table_bytes(n));
+    size_t off = 0;
+    for (int i = 0; i < n; ++i) {
+        const attwarp_ragged_image& im = images[i];
+        AW_REQUIRE(im.src && im.dst && im.src != im.dst, "%s: image %d: bad pointers", what, i);
+        AW_REQUIRE(im.H > 0 && im.W > 0 && im.Ho > 0 && im.Wo > 0, "%s: image %d: sizes must be positive", what, i);
+        AW_REQUIRE(im.H < 65536 && im.W < 65536, "%s: image %d: H, W must be below 65536", what, i);
+        RaggedImage& r = host[(size_t)i];
+        r.src = static_cast<const uint8_t*>(im.src);
+        r.dst = static_cast<uint8_t*>(im.dst);
+        r.map_x = pool + off; off += (size_t)im.Wo;
+        r.map_y = pool + off; off += (size_t)im.Ho;
+        r.H = im.H; r.W = im.W; r.Ho = im.Ho; r.Wo = im.Wo;
+        l->max_h = im.H > l->max_h ? im.H : l->max_h;
+        l->max_w = im.W > l->max_w ? im.W : l->max_w;
+        l->degenerate = l->degenerate || im.H < 2 || im.W < 2;
+    }
+    return ATTWARP_OK;
+}
+
+// A list with a 1-pixel axis goes image by image through the uniform entry points (the streaming kernel needs two
+// source rows and columns); such lists are not a throughput case.  maps(i, r) writes image i's maps.
+template <class Maps>
+static int ragged_per_image(const RaggedList& l, int n, int C, cudaStream_t st, int launches, Maps&& maps) {
+    for (int i = 0; i < n; ++i) {
+        const RaggedImage& r = l.host[i];
+        int rc = maps(i, r);
+        if (rc != ATTWARP_OK) return rc;
+        rc = launch_remap(r.src, r.dst, ATTWARP_U8, ATTWARP_LAYOUT_HWC, 1, C, r.H, r.W, r.Ho, r.Wo, r.map_x, r.map_y, st);
+        if (rc != ATTWARP_OK) return rc;
+    }
+    g_ragged_last_launches = launches;
+    return ATTWARP_OK;
+}
+
+// The strip plan of stage 5 is part of the table both the maps and the resample kernels read: plan + upload, then
+// maps() enqueues the `maps_launches` maps launches, then the resample.
+template <class Maps>
+static int ragged_stage5(const RaggedList& l, int n, int C, cudaStream_t st, int maps_launches, Maps&& maps) {
+    const bool quad = C == 3 && remap_quad_enabled();
+    RaggedQuadPlan plan;
+    RaggedImage* dev_sorted = l.dev + (n + 1);
+    int rc = quad ? launch_remap_u8_quad_ragged_prepare(l.host, n, l.dev, dev_sorted, &plan, st)
+                  : launch_remap_u8_stream_ragged_prepare(l.host, n, C, l.dev, st);
+    if (rc != ATTWARP_OK) return rc;
+    if ((rc = maps()) != ATTWARP_OK) return rc;
+    g_ragged_last_launches = maps_launches + (quad ? ragged_quad_launches(plan) : 1);
+    return quad ? launch_remap_u8_quad_ragged_run(plan, dev_sorted, st)
+                : launch_remap_u8_stream_ragged_run(l.host, n, C, l.dev, st);
+}
+
+extern "C" {
 
 size_t attwarp_ragged_workspace_bytes(const attwarp_ragged_image* images, int n) {
     if (images == nullptr || n <= 0) return 0;
-    size_t floats = 0;
-    for (int i = 0; i < n; ++i) floats += (size_t)(images[i].Wo > 0 ? images[i].Wo : 0) + (size_t)(images[i].Ho > 0 ? images[i].Ho : 0);
-    return ragged_table_bytes(n) + align_up(floats * sizeof(float), 256);
+    return ragged_prefix_bytes(images, n);
 }
 
 int attwarp_warp_ragged_from_tokens(const float* tok, int n, int gh, int gw,
@@ -390,331 +481,217 @@ int attwarp_warp_ragged_from_tokens(const float* tok, int n, int gh, int gw,
     AW_REQUIRE(C == 1 || C == 3 || C == 4, "warp_ragged: C must be 1, 3 or 4 (got %d)", C);
     int rc = check_transform(tp);
     if (rc != ATTWARP_OK) return rc;
-    const size_t need = attwarp_ragged_workspace_bytes(images, n);
+    RaggedList l;
+    if ((rc = ragged_list("warp_ragged", images, n, workspace, &l)) != ATTWARP_OK) return rc;
+    const size_t need = ragged_prefix_bytes(images, n);
     if (workspace_bytes < need)
         return fail(ATTWARP_ERR_WORKSPACE, "warp_ragged: workspace too small (%zu < %zu)", workspace_bytes, need);
     cudaStream_t st = as_stream(stream);
-    {
-        // the descriptor tables are uploaded from this thread's host buffers: a captured copy node would read them at
-        // replay time, after later calls have rewritten them
-        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        AW_CUDA(cudaStreamIsCapturing(st, &cap));
-        if (cap != cudaStreamCaptureStatusNone)
-            return fail(ATTWARP_ERR_UNSUPPORTED, "warp_ragged: cannot be captured into a CUDA graph (host-side descriptor tables)");
-    }
-    RaggedImage* dev_table = static_cast<RaggedImage*>(workspace);
-    float* pool = reinterpret_cast<float*>(static_cast<char*>(workspace) + ragged_table_bytes(n));
-    static thread_local std::vector<RaggedImage> host;
-    host.assign((size_t)n + 1, RaggedImage{});
-    int max_h = 0, max_w = 0;
-    bool degenerate = false;
-    size_t off = 0;
-    for (int i = 0; i < n; ++i) {
-        const attwarp_ragged_image& im = images[i];
-        AW_REQUIRE(im.src && im.dst && im.src != im.dst, "warp_ragged: image %d: bad pointers", i);
-        AW_REQUIRE(im.H > 0 && im.W > 0 && im.Ho > 0 && im.Wo > 0, "warp_ragged: image %d: sizes must be positive", i);
-        AW_REQUIRE(im.H < 65536 && im.W < 65536, "warp_ragged: image %d: H, W must be below 65536", i);
-        RaggedImage& r = host[(size_t)i];
-        r.src = static_cast<const uint8_t*>(im.src);
-        r.dst = static_cast<uint8_t*>(im.dst);
-        r.map_x = pool + off; off += (size_t)im.Wo;
-        r.map_y = pool + off; off += (size_t)im.Ho;
-        r.H = im.H; r.W = im.W; r.Ho = im.Ho; r.Wo = im.Wo;
-        max_h = im.H > max_h ? im.H : max_h;
-        max_w = im.W > max_w ? im.W : max_w;
-        degenerate = degenerate || im.H < 2 || im.W < 2;
-    }
-    if (degenerate) {
-        // 1-pixel axes go through the per-image entry points (the streaming kernel needs two source rows
-        // and columns); such batches are not a throughput case
-        for (int i = 0; i < n; ++i) {
-            const RaggedImage& r = host[(size_t)i];
-            rc = launch_maps_from_tokens(tok + (size_t)i * gh * gw, 1, 1.0f, nullptr, 1, gh, gw, r.H, r.W, r.Wo, r.Ho,
-                                         *tp, const_cast<float*>(r.map_x), const_cast<float*>(r.map_y), nullptr, st);
-            if (rc != ATTWARP_OK) return rc;
-            rc = launch_remap(r.src, r.dst, ATTWARP_U8, ATTWARP_LAYOUT_HWC, 1, C, r.H, r.W, r.Ho, r.Wo, r.map_x, r.map_y, st);
-            if (rc != ATTWARP_OK) return rc;
-        }
-        g_ragged_last_launches = 2 * n;          // maps + resample per image
-        return ATTWARP_OK;
-    }
-    // the strip plan of stage 5 is part of the table both kernels read: plan + upload, maps, resample
-    const bool quad = C == 3 && remap_quad_enabled();
-    RaggedQuadPlan plan;
-    RaggedImage* dev_sorted = dev_table + (n + 1);
-    rc = quad ? launch_remap_u8_quad_ragged_prepare(host.data(), n, dev_table, dev_sorted, &plan, st)
-              : launch_remap_u8_stream_ragged_prepare(host.data(), n, C, dev_table, st);
-    if (rc != ATTWARP_OK) return rc;
-    rc = launch_maps_from_tokens_ragged(tok, n, gh, gw, dev_table, max_h, max_w, *tp, nullptr, st);
-    if (rc != ATTWARP_OK) return rc;
-    g_ragged_last_launches = 1 + (quad ? ragged_quad_launches(plan) : 1);
-    return quad ? launch_remap_u8_quad_ragged_run(plan, dev_sorted, st)
-                : launch_remap_u8_stream_ragged_run(host.data(), n, C, dev_table, st);
+    if ((rc = refuse_graph_capture(st, "warp_ragged")) != ATTWARP_OK) return rc;
+    if (l.degenerate)          // maps + resample per image
+        return ragged_per_image(l, n, C, st, 2 * n, [&](int i, const RaggedImage& r) {
+            return launch_maps_from_tokens(tok + (size_t)i * gh * gw, 1, 1.0f, nullptr, 1, gh, gw, r.H, r.W, r.Wo, r.Ho,
+                                           *tp, const_cast<float*>(r.map_x), const_cast<float*>(r.map_y), nullptr, st);
+        });
+    return ragged_stage5(l, n, C, st, 1, [&] {
+        return launch_maps_from_tokens_ragged(tok, n, gh, gw, l.dev, l.max_h, l.max_w, *tp, nullptr, st);
+    });
 }
 
 int attwarp_ragged_last_launches(void) { return g_ragged_last_launches; }
 
 // ---------------------------------------------------------------------------------------------
-// Ragged batch warped by per-image maps.  Workspace: the tokens call's descriptor tables and map rows, then the
-// maps' descriptors (RaggedAtt) followed by the work items, then the partials: every image's at its own offset
-// (ragged geometry), or one image's of the uniform geometry when the call goes image by image.
-struct RaggedAttSizes {
-    size_t map_floats = 0, part_doubles = 0, uniform_bytes = 0;
+// Ragged batch warped by per-image maps.  Workspace: the shared prefix, then the maps' descriptors (RaggedAtt) followed
+// by the work items, then the partials: every image's at its own offset (ragged geometry), or one image's of the
+// uniform geometry when the call goes image by image.
+struct RaggedAttLayout {
     int64_t items = 0;
+    size_t att = 0, item_at = 0, partials = 0, part_bytes = 0, total = 0;     // byte offsets and sizes
 };
-static bool ragged_att_sizes(const attwarp_ragged_image* images, int n, RaggedAttSizes* s) {
+static bool ragged_att_layout(const attwarp_ragged_image* images, int n, RaggedAttLayout* w) {
+    const size_t prefix = ragged_prefix_bytes(images, n);
+    if (prefix == 0) return false;
+    size_t part_doubles = 0, uniform_bytes = 0;
     for (int i = 0; i < n; ++i) {
         const attwarp_ragged_image& im = images[i];
-        if (im.H <= 0 || im.W <= 0 || im.Ho <= 0 || im.Wo <= 0 || im.H >= 65536 || im.W >= 65536) return false;
         int rows, nrc, tc, nct;
         ragged_att_geometry(im.H, im.W, &rows, &nrc, &tc, &nct);
-        s->map_floats += (size_t)im.Wo + (size_t)im.Ho;
-        s->part_doubles += (size_t)nrc * im.W + (size_t)nct * im.H;
-        s->items += (int64_t)nrc * nct;
+        part_doubles += (size_t)nrc * im.W + (size_t)nct * im.H;
+        w->items += (int64_t)nrc * nct;
         const size_t u = maps_workspace_bytes_impl(1, im.H, im.W);
-        s->uniform_bytes = u > s->uniform_bytes ? u : s->uniform_bytes;
+        uniform_bytes = u > uniform_bytes ? u : uniform_bytes;
     }
+    const size_t desc = align_up(sizeof(RaggedAtt) * (size_t)n, 16), part = part_doubles * sizeof(double);
+    w->att = prefix;
+    w->item_at = prefix + desc;
+    w->partials = prefix + align_up(desc + sizeof(int2) * (size_t)w->items, 256);
+    w->part_bytes = part > uniform_bytes ? part : uniform_bytes;
+    w->total = w->partials + w->part_bytes;
     return true;
-}
-static size_t ragged_att_desc_bytes(int n) { return align_up(sizeof(RaggedAtt) * (size_t)n, 16); }
-static size_t ragged_att_tables_bytes(int n, int64_t items) {
-    return align_up(ragged_att_desc_bytes(n) + sizeof(int2) * (size_t)items, 256);
 }
 
 size_t attwarp_ragged_attention_workspace_bytes(const attwarp_ragged_image* images, int n) {
-    RaggedAttSizes s;
-    if (images == nullptr || n <= 0 || !ragged_att_sizes(images, n, &s)) return 0;
-    const size_t part = s.part_doubles * sizeof(double);
-    return ragged_table_bytes(n) + align_up(s.map_floats * sizeof(float), 256) + ragged_att_tables_bytes(n, s.items) +
-           (part > s.uniform_bytes ? part : s.uniform_bytes);
+    RaggedAttLayout w;
+    if (images == nullptr || n <= 0 || !ragged_att_layout(images, n, &w)) return 0;
+    return w.total;
 }
 
 int attwarp_warp_ragged_from_attention(const attwarp_ragged_image* images, const attwarp_ragged_attention* att,
                                        int n, int att_dtype, int C, const attwarp_transform_params* tp,
                                        void* workspace, size_t workspace_bytes, void* stream) {
-    AW_REQUIRE(images && att && workspace, "warp_ragged_from_attention: NULL pointer");
-    AW_REQUIRE(n > 0, "warp_ragged_from_attention: n must be positive (got %d)", n);
-    AW_REQUIRE(C == 1 || C == 3 || C == 4, "warp_ragged_from_attention: C must be 1, 3 or 4 (got %d)", C);
+    const char* const what = "warp_ragged_from_attention";
+    AW_REQUIRE(images && att && workspace, "%s: NULL pointer", what);
+    AW_REQUIRE(n > 0, "%s: n must be positive (got %d)", what, n);
+    AW_REQUIRE(C == 1 || C == 3 || C == 4, "%s: C must be 1, 3 or 4 (got %d)", what, C);
     AW_REQUIRE(att_dtype == ATTWARP_U8 || att_dtype == ATTWARP_F32 || att_dtype == ATTWARP_F64,
-               "warp_ragged_from_attention: attention dtype must be U8, F32 or F64 (got %d)", att_dtype);
+               "%s: attention dtype must be U8, F32 or F64 (got %d)", what, att_dtype);
     int rc = check_transform(tp);
     if (rc != ATTWARP_OK) return rc;
+    RaggedList l;
+    if ((rc = ragged_list(what, images, n, workspace, &l)) != ATTWARP_OK) return rc;
     const size_t es = dtype_size(att_dtype);
-    for (int i = 0; i < n; ++i) {
-        const attwarp_ragged_image& im = images[i];
-        AW_REQUIRE(im.src && im.dst && im.src != im.dst, "warp_ragged_from_attention: image %d: bad pointers", i);
-        AW_REQUIRE(im.H > 0 && im.W > 0 && im.Ho > 0 && im.Wo > 0,
-                   "warp_ragged_from_attention: image %d: sizes must be positive", i);
-        AW_REQUIRE(im.H < 65536 && im.W < 65536, "warp_ragged_from_attention: image %d: H, W must be below 65536", i);
-        AW_REQUIRE(att[i].att != nullptr, "warp_ragged_from_attention: image %d: NULL attention map", i);
-        AW_REQUIRE((reinterpret_cast<uintptr_t>(att[i].att) & (es - 1)) == 0,
-                   "warp_ragged_from_attention: image %d: attention map not aligned to its %zu-byte elements", i, es);
-    }
-    RaggedAttSizes s;
-    ragged_att_sizes(images, n, &s);
-    const size_t need = attwarp_ragged_attention_workspace_bytes(images, n);
-    if (workspace_bytes < need)
-        return fail(ATTWARP_ERR_WORKSPACE, "warp_ragged_from_attention: workspace too small (%zu < %zu)", workspace_bytes,
-                    need);
-    cudaStream_t st = as_stream(stream);
-    {
-        // as attwarp_warp_ragged_from_tokens: a captured copy node would read the host tables at replay time
-        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        AW_CUDA(cudaStreamIsCapturing(st, &cap));
-        if (cap != cudaStreamCaptureStatusNone)
-            return fail(ATTWARP_ERR_UNSUPPORTED,
-                        "warp_ragged_from_attention: cannot be captured into a CUDA graph (host-side descriptor tables)");
-    }
-    char* ws = static_cast<char*>(workspace);
-    RaggedImage* dev_table = reinterpret_cast<RaggedImage*>(ws);
-    ws += ragged_table_bytes(n);
-    float* pool = reinterpret_cast<float*>(ws);
-    ws += align_up(s.map_floats * sizeof(float), 256);
-    RaggedAtt* dev_att = reinterpret_cast<RaggedAtt*>(ws);
-    int2* dev_items = reinterpret_cast<int2*>(ws + ragged_att_desc_bytes(n));
-    ws += ragged_att_tables_bytes(n, s.items);
-    double* partials = reinterpret_cast<double*>(ws);
-    const size_t part_bytes = need - (size_t)(ws - static_cast<char*>(workspace));
-
-    static thread_local std::vector<RaggedImage> host;
     static thread_local std::vector<RaggedAtt> host_att;
-    host.assign((size_t)n + 1, RaggedImage{});
     host_att.assign((size_t)n, RaggedAtt{});
-    int max_h = 0, max_w = 0;
-    bool degenerate = false;
-    size_t off = 0;
     int64_t part_off = 0;
     for (int i = 0; i < n; ++i) {
-        const attwarp_ragged_image& im = images[i];
-        RaggedImage& r = host[(size_t)i];
-        r.src = static_cast<const uint8_t*>(im.src);
-        r.dst = static_cast<uint8_t*>(im.dst);
-        r.map_x = att[i].map_x != nullptr ? att[i].map_x : pool + off; off += (size_t)im.Wo;
-        r.map_y = att[i].map_y != nullptr ? att[i].map_y : pool + off; off += (size_t)im.Ho;
-        r.H = im.H; r.W = im.W; r.Ho = im.Ho; r.Wo = im.Wo;
+        AW_REQUIRE(att[i].att != nullptr, "%s: image %d: NULL attention map", what, i);
+        AW_REQUIRE((reinterpret_cast<uintptr_t>(att[i].att) & (es - 1)) == 0,
+                   "%s: image %d: attention map not aligned to its %zu-byte elements", what, i, es);
+        RaggedImage& r = l.host[i];
+        if (att[i].map_x != nullptr) r.map_x = att[i].map_x;
+        if (att[i].map_y != nullptr) r.map_y = att[i].map_y;
         RaggedAtt& a = host_att[(size_t)i];
         a.att = att[i].att;
-        a.H = im.H; a.W = im.W;
-        ragged_att_geometry(im.H, im.W, &a.chunk_rows, &a.n_chunks, &a.tile_cols, &a.n_tiles);
-        a.colpart = part_off; part_off += (int64_t)a.n_chunks * im.W;
-        a.rowpart = part_off; part_off += (int64_t)a.n_tiles * im.H;
-        max_h = im.H > max_h ? im.H : max_h;
-        max_w = im.W > max_w ? im.W : max_w;
-        degenerate = degenerate || im.H < 2 || im.W < 2;
+        a.H = r.H; a.W = r.W;
+        ragged_att_geometry(r.H, r.W, &a.chunk_rows, &a.n_chunks, &a.tile_cols, &a.n_tiles);
+        a.colpart = part_off; part_off += (int64_t)a.n_chunks * r.W;
+        a.rowpart = part_off; part_off += (int64_t)a.n_tiles * r.H;
     }
-    if (degenerate) {
-        // 1-pixel axes: image by image through the uniform entry points, as attwarp_warp_ragged_from_tokens does
-        for (int i = 0; i < n; ++i) {
-            const RaggedImage& r = host[(size_t)i];
-            rc = launch_maps_from_attention(att[i].att, att_dtype, 1, r.H, r.W, r.Wo, r.Ho, *tp, partials, part_bytes,
-                                            const_cast<float*>(r.map_x), const_cast<float*>(r.map_y), nullptr, st);
-            if (rc != ATTWARP_OK) return rc;
-            rc = launch_remap(r.src, r.dst, ATTWARP_U8, ATTWARP_LAYOUT_HWC, 1, C, r.H, r.W, r.Ho, r.Wo, r.map_x, r.map_y, st);
-            if (rc != ATTWARP_OK) return rc;
-        }
-        g_ragged_last_launches = 3 * n;          // marginals + finish + resample per image
-        return ATTWARP_OK;
-    }
-    const bool quad = C == 3 && remap_quad_enabled();
-    RaggedQuadPlan plan;
-    RaggedImage* dev_sorted = dev_table + (n + 1);
-    rc = quad ? launch_remap_u8_quad_ragged_prepare(host.data(), n, dev_table, dev_sorted, &plan, st)
-              : launch_remap_u8_stream_ragged_prepare(host.data(), n, C, dev_table, st);
-    if (rc != ATTWARP_OK) return rc;
-    rc = launch_maps_from_attention_ragged(host_att.data(), n, att_dtype, dev_table, dev_att, dev_items, s.items,
-                                           partials, max_h, max_w, *tp, st);
-    if (rc != ATTWARP_OK) return rc;
-    g_ragged_last_launches = 2 + (quad ? ragged_quad_launches(plan) : 1);
-    return quad ? launch_remap_u8_quad_ragged_run(plan, dev_sorted, st)
-                : launch_remap_u8_stream_ragged_run(host.data(), n, C, dev_table, st);
+    RaggedAttLayout w;
+    ragged_att_layout(images, n, &w);
+    if (workspace_bytes < w.total)
+        return fail(ATTWARP_ERR_WORKSPACE, "%s: workspace too small (%zu < %zu)", what, workspace_bytes, w.total);
+    cudaStream_t st = as_stream(stream);
+    if ((rc = refuse_graph_capture(st, what)) != ATTWARP_OK) return rc;
+    char* ws = static_cast<char*>(workspace);
+    double* partials = reinterpret_cast<double*>(ws + w.partials);
+    if (l.degenerate)          // marginals + finish + resample per image
+        return ragged_per_image(l, n, C, st, 3 * n, [&](int i, const RaggedImage& r) {
+            return launch_maps_from_attention(att[i].att, att_dtype, 1, r.H, r.W, r.Wo, r.Ho, *tp, partials,
+                                              w.part_bytes, const_cast<float*>(r.map_x), const_cast<float*>(r.map_y),
+                                              nullptr, st);
+        });
+    return ragged_stage5(l, n, C, st, 2, [&] {
+        return launch_maps_from_attention_ragged(host_att.data(), n, att_dtype, l.dev,
+                                                 reinterpret_cast<RaggedAtt*>(ws + w.att),
+                                                 reinterpret_cast<int2*>(ws + w.item_at), w.items, partials, l.max_h,
+                                                 l.max_w, *tp, st);
+    });
 }
 
 // ---------------------------------------------------------------------------------------------
-// Ragged batch warped by each image's LANCZOS-resized mask.  Workspace: the tokens call's descriptor tables and map
-// rows, then RaggedAtt [n], RaggedLanczos [n] and the work items (fused kernel's, then the uint8 marginals'), then the
-// image-size masks of the images the fused kernel does not take, then the partials (every image's at its own offset,
-// or one image's of the uniform entry points when the call goes image by image).
-struct RaggedMaskSizes {
-    size_t map_floats = 0, part_doubles = 0, mask_bytes = 0, uniform_bytes = 0, smem = 0;
+// Ragged batch warped by each image's LANCZOS-resized mask.  Workspace: the shared prefix, then RaggedAtt [n],
+// RaggedLanczos [n] and the work items (fused kernel's, then the uint8 marginals'), then the image-size masks of the
+// images the fused kernel does not take, then the partials (every image's at its own offset, or one image's of the
+// uniform entry points when the call goes image by image).
+struct RaggedMaskLayout {
     int64_t fused_items = 0, att_items = 0;
+    size_t smem = 0;                                       // the fused kernel's shared memory
+    size_t tables = 0, lz = 0, item_at = 0, table_bytes = 0;   // the uploaded tables; lz, item_at: offsets into them
+    size_t masks = 0, partials = 0, part_bytes = 0, total = 0;
 };
-static bool ragged_mask_sizes(const attwarp_ragged_image* images, int n, int gh, int gw, RaggedMaskSizes* s) {
+static bool ragged_mask_layout(const attwarp_ragged_image* images, int n, int gh, int gw, RaggedMaskLayout* w) {
+    const size_t prefix = ragged_prefix_bytes(images, n);
+    if (prefix == 0) return false;
+    size_t part_doubles = 0, mask_bytes = 0, uniform_bytes = 0;
     for (int i = 0; i < n; ++i) {
         const attwarp_ragged_image& im = images[i];
-        if (im.H <= 0 || im.W <= 0 || im.Ho <= 0 || im.Wo <= 0 || im.H >= 65536 || im.W >= 65536) return false;
-        s->map_floats += (size_t)im.Wo + (size_t)im.Ho;
         int rows, nt, nx, warps;
         size_t smem, part;
         if (lanczos_ragged_geometry(gh, gw, im.H, im.W, &rows, &nt, &nx, &warps, &smem)) {
             part = (size_t)nt * im.W + (size_t)nx * im.H;
-            s->fused_items += (int64_t)nt * nx;
-            s->smem = smem > s->smem ? smem : s->smem;
+            w->fused_items += (int64_t)nt * nx;
+            w->smem = smem > w->smem ? smem : w->smem;
         } else {
             int nrc, tc, nct;
             ragged_att_geometry(im.H, im.W, &rows, &nrc, &tc, &nct);
             part = (size_t)nrc * im.W + (size_t)nct * im.H;
-            s->att_items += (int64_t)nrc * nct;
-            s->mask_bytes += align_up((size_t)im.H * im.W, 16);
+            w->att_items += (int64_t)nrc * nct;
+            mask_bytes += align_up((size_t)im.H * im.W, 16);
             const size_t u = maps_workspace_bytes_impl(1, im.H, im.W);
-            s->uniform_bytes = u > s->uniform_bytes ? u : s->uniform_bytes;
+            uniform_bytes = u > uniform_bytes ? u : uniform_bytes;
         }
-        s->part_doubles += part;
-        s->uniform_bytes = part * sizeof(double) > s->uniform_bytes ? part * sizeof(double) : s->uniform_bytes;
+        part_doubles += part;
+        uniform_bytes = part * sizeof(double) > uniform_bytes ? part * sizeof(double) : uniform_bytes;
     }
+    w->tables = prefix;
+    w->lz = align_up(sizeof(RaggedAtt) * (size_t)n, 16);
+    w->item_at = w->lz + sizeof(RaggedLanczos) * (size_t)n;
+    w->table_bytes = w->item_at + sizeof(int2) * (size_t)(w->fused_items + w->att_items);
+    w->masks = w->tables + align_up(w->table_bytes, 256);
+    w->partials = w->masks + align_up(mask_bytes, 256);
+    const size_t part = part_doubles * sizeof(double);
+    w->part_bytes = part > uniform_bytes ? part : uniform_bytes;
+    w->total = w->partials + w->part_bytes;
     return true;
-}
-static size_t ragged_mask_tables_bytes(int n, int64_t items) {
-    return align_up(align_up(sizeof(RaggedAtt) * (size_t)n, 16) + sizeof(RaggedLanczos) * (size_t)n +
-                    sizeof(int2) * (size_t)items, 256);
 }
 
 size_t attwarp_ragged_mask_workspace_bytes(const attwarp_ragged_image* images, int n, int gh, int gw) {
-    RaggedMaskSizes s;
-    if (images == nullptr || n <= 0 || gh <= 0 || gw <= 0 || !ragged_mask_sizes(images, n, gh, gw, &s)) return 0;
-    const size_t part = s.part_doubles * sizeof(double);
-    return ragged_table_bytes(n) + align_up(s.map_floats * sizeof(float), 256) +
-           ragged_mask_tables_bytes(n, s.fused_items + s.att_items) + align_up(s.mask_bytes, 256) +
-           (part > s.uniform_bytes ? part : s.uniform_bytes);
+    RaggedMaskLayout w;
+    if (images == nullptr || n <= 0 || gh <= 0 || gw <= 0 || !ragged_mask_layout(images, n, gh, gw, &w)) return 0;
+    return w.total;
 }
 
 int attwarp_warp_ragged_from_mask(const attwarp_ragged_image* images, const void* mask_u8, int n, int gh, int gw, int C,
                                   const attwarp_transform_params* tp, void* workspace, size_t workspace_bytes,
                                   float* map_x_opt, float* map_y_opt, void* stream) {
-    AW_REQUIRE(images && mask_u8 && workspace, "warp_ragged_from_mask: NULL pointer");
-    AW_REQUIRE(n > 0 && gh > 0 && gw > 0, "warp_ragged_from_mask: n, gh, gw must be positive (got %d, %d, %d)", n, gh, gw);
-    AW_REQUIRE(C == 1 || C == 3 || C == 4, "warp_ragged_from_mask: C must be 1, 3 or 4 (got %d)", C);
+    const char* const what = "warp_ragged_from_mask";
+    AW_REQUIRE(images && mask_u8 && workspace, "%s: NULL pointer", what);
+    AW_REQUIRE(n > 0 && gh > 0 && gw > 0, "%s: n, gh, gw must be positive (got %d, %d, %d)", what, n, gh, gw);
+    AW_REQUIRE(C == 1 || C == 3 || C == 4, "%s: C must be 1, 3 or 4 (got %d)", what, C);
     int rc = check_transform(tp);
     if (rc != ATTWARP_OK) return rc;
     if (tp->transform != ATTWARP_T_IDENTITY)
-        return fail(ATTWARP_ERR_UNSUPPORTED, "warp_ragged_from_mask: identity transform only (got %d; resize the masks and "
-                    "use warp_ragged_from_attention)", tp->transform);
-    for (int i = 0; i < n; ++i) {
-        const attwarp_ragged_image& im = images[i];
-        AW_REQUIRE(im.src && im.dst && im.src != im.dst, "warp_ragged_from_mask: image %d: bad pointers", i);
-        AW_REQUIRE(im.H > 0 && im.W > 0 && im.Ho > 0 && im.Wo > 0, "warp_ragged_from_mask: image %d: sizes must be positive", i);
-        AW_REQUIRE(im.H < 65536 && im.W < 65536, "warp_ragged_from_mask: image %d: H, W must be below 65536", i);
-    }
-    RaggedMaskSizes s;
-    ragged_mask_sizes(images, n, gh, gw, &s);
-    const size_t need = attwarp_ragged_mask_workspace_bytes(images, n, gh, gw);
-    if (workspace_bytes < need)
-        return fail(ATTWARP_ERR_WORKSPACE, "warp_ragged_from_mask: workspace too small (%zu < %zu)", workspace_bytes, need);
+        return fail(ATTWARP_ERR_UNSUPPORTED, "%s: identity transform only (got %d; resize the masks and "
+                    "use warp_ragged_from_attention)", what, tp->transform);
+    RaggedList l;
+    if ((rc = ragged_list(what, images, n, workspace, &l)) != ATTWARP_OK) return rc;
+    RaggedMaskLayout w;
+    ragged_mask_layout(images, n, gh, gw, &w);
+    if (workspace_bytes < w.total)
+        return fail(ATTWARP_ERR_WORKSPACE, "%s: workspace too small (%zu < %zu)", what, workspace_bytes, w.total);
     cudaStream_t st = as_stream(stream);
-    {
-        // as attwarp_warp_ragged_from_tokens: a captured copy node would read the host tables at replay time
-        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        AW_CUDA(cudaStreamIsCapturing(st, &cap));
-        if (cap != cudaStreamCaptureStatusNone)
-            return fail(ATTWARP_ERR_UNSUPPORTED,
-                        "warp_ragged_from_mask: cannot be captured into a CUDA graph (host-side descriptor tables)");
-    }
-    const int64_t n_items = s.fused_items + s.att_items;
+    if ((rc = refuse_graph_capture(st, what)) != ATTWARP_OK) return rc;
     char* ws = static_cast<char*>(workspace);
-    RaggedImage* dev_table = reinterpret_cast<RaggedImage*>(ws);
-    ws += ragged_table_bytes(n);
-    float* pool = reinterpret_cast<float*>(ws);
-    ws += align_up(s.map_floats * sizeof(float), 256);
-    char* dev_tables = ws;
-    const size_t lz_off = align_up(sizeof(RaggedAtt) * (size_t)n, 16), items_off = lz_off + sizeof(RaggedLanczos) * (size_t)n;
-    RaggedAtt* dev_att = reinterpret_cast<RaggedAtt*>(dev_tables);
-    int2* dev_items = reinterpret_cast<int2*>(dev_tables + items_off);
-    ws += ragged_mask_tables_bytes(n, n_items);
-    uint8_t* masks = reinterpret_cast<uint8_t*>(ws);
-    ws += align_up(s.mask_bytes, 256);
-    double* partials = reinterpret_cast<double*>(ws);
-    const size_t part_bytes = need - (size_t)(ws - static_cast<char*>(workspace));
+    uint8_t* masks = reinterpret_cast<uint8_t*>(ws + w.masks);
+    double* partials = reinterpret_cast<double*>(ws + w.partials);
 
-    static thread_local std::vector<RaggedImage> host;
     static thread_local std::vector<char> host_tables;
-    host.assign((size_t)n + 1, RaggedImage{});
-    host_tables.assign(items_off + sizeof(int2) * (size_t)n_items, 0);
+    host_tables.assign(w.table_bytes, 0);
     RaggedAtt* host_att = reinterpret_cast<RaggedAtt*>(host_tables.data());
-    RaggedLanczos* host_lz = reinterpret_cast<RaggedLanczos*>(host_tables.data() + lz_off);
-    int2* fused_items = reinterpret_cast<int2*>(host_tables.data() + items_off);
-    int2* att_items = fused_items + s.fused_items;
-    int max_h = 0, max_w = 0, launches = 0;
-    bool degenerate = false;
-    size_t off = 0, mask_off = 0, mx_off = 0, my_off = 0;
+    RaggedLanczos* host_lz = reinterpret_cast<RaggedLanczos*>(host_tables.data() + w.lz);
+    int2* fused_items = reinterpret_cast<int2*>(host_tables.data() + w.item_at);
+    int2* att_items = fused_items + w.fused_items;
+    int launches = 0;
+    size_t mask_off = 0, mx_off = 0, my_off = 0;
     int64_t part_off = 0, nf = 0, na = 0;
     const uint8_t* mask = static_cast<const uint8_t*>(mask_u8);
     for (int i = 0; i < n; ++i) {
-        const attwarp_ragged_image& im = images[i];
-        RaggedImage& r = host[(size_t)i];
-        r.src = static_cast<const uint8_t*>(im.src);
-        r.dst = static_cast<uint8_t*>(im.dst);
-        r.map_x = map_x_opt != nullptr ? map_x_opt + mx_off : pool + off; off += (size_t)im.Wo; mx_off += (size_t)im.Wo;
-        r.map_y = map_y_opt != nullptr ? map_y_opt + my_off : pool + off; off += (size_t)im.Ho; my_off += (size_t)im.Ho;
-        r.H = im.H; r.W = im.W; r.Ho = im.Ho; r.Wo = im.Wo;
+        RaggedImage& r = l.host[i];
+        if (map_x_opt != nullptr) r.map_x = map_x_opt + mx_off;
+        if (map_y_opt != nullptr) r.map_y = map_y_opt + my_off;
+        mx_off += (size_t)r.Wo;
+        my_off += (size_t)r.Ho;
         RaggedAtt& a = host_att[i];
-        a.H = im.H; a.W = im.W;
+        a.H = r.H; a.W = r.W;
         int rows, nt, nx, warps;
         size_t smem;
-        if (lanczos_ragged_geometry(gh, gw, im.H, im.W, &rows, &nt, &nx, &warps, &smem)) {
+        if (lanczos_ragged_geometry(gh, gw, r.H, r.W, &rows, &nt, &nx, &warps, &smem)) {
             // the fused kernel: row tiles as chunks, column CTAs as tiles of the finish kernel's partial layout
             a.att = mask + (size_t)i * gh * gw;
             a.chunk_rows = rows; a.n_chunks = nt;
             a.tile_cols = warps * 64; a.n_tiles = nx;
-            rc = lanczos_ragged_tables(gh, gw, im.H, im.W, rows, &host_lz[i]);
+            rc = lanczos_ragged_tables(gh, gw, r.H, r.W, rows, &host_lz[i]);
             if (rc != ATTWARP_OK) return rc;
             host_lz[i].warps = warps;
             for (int t = 0; t < nt; ++t)
@@ -722,64 +699,46 @@ int attwarp_warp_ragged_from_mask(const attwarp_ragged_image* images, const void
         } else {
             // resized to image size first, then summed by the ragged uint8 marginals kernel
             a.att = masks + mask_off;
-            mask_off += align_up((size_t)im.H * im.W, 16);
-            ragged_att_geometry(im.H, im.W, &a.chunk_rows, &a.n_chunks, &a.tile_cols, &a.n_tiles);
+            mask_off += align_up((size_t)r.H * r.W, 16);
+            ragged_att_geometry(r.H, r.W, &a.chunk_rows, &a.n_chunks, &a.tile_cols, &a.n_tiles);
             for (int c = 0; c < a.n_chunks; ++c)
                 for (int t = 0; t < a.n_tiles; ++t) att_items[na++] = make_int2(i, c << 8 | t);
-            rc = launch_resize_lanczos_u8(mask + (size_t)i * gh * gw, 1, gh, gw, im.H, im.W,
+            rc = launch_resize_lanczos_u8(mask + (size_t)i * gh * gw, 1, gh, gw, r.H, r.W,
                                           static_cast<uint8_t*>(const_cast<void*>(a.att)), st);
             if (rc != ATTWARP_OK) return rc;
             ++launches;
         }
-        a.colpart = part_off; part_off += (int64_t)a.n_chunks * im.W;
-        a.rowpart = part_off; part_off += (int64_t)a.n_tiles * im.H;
-        max_h = im.H > max_h ? im.H : max_h;
-        max_w = im.W > max_w ? im.W : max_w;
-        degenerate = degenerate || im.H < 2 || im.W < 2;
+        a.colpart = part_off; part_off += (int64_t)a.n_chunks * r.W;
+        a.rowpart = part_off; part_off += (int64_t)a.n_tiles * r.H;
     }
-    if (degenerate) {
-        // 1-pixel axes: image by image through the uniform entry points, as attwarp_warp_ragged_from_attention does
-        for (int i = 0; i < n; ++i) {
-            const RaggedImage& r = host[(size_t)i];
+    if (l.degenerate)          // resizes + marginals, finish and resample per image
+        return ragged_per_image(l, n, C, st, launches + 3 * n, [&](int i, const RaggedImage& r) {
             float* mx = const_cast<float*>(r.map_x);
             float* my = const_cast<float*>(r.map_y);
             if (host_lz[i].planes != nullptr)           // taken by the fused kernel
-                rc = launch_maps_from_mask(mask + (size_t)i * gh * gw, 1, gh, gw, r.H, r.W, r.Wo, r.Ho, *tp, partials,
-                                           part_bytes, mx, my, st);
-            else
-                rc = launch_maps_from_attention(host_att[i].att, ATTWARP_U8, 1, r.H, r.W, r.Wo, r.Ho, *tp, partials,
-                                                part_bytes, mx, my, nullptr, st);
-            if (rc != ATTWARP_OK) return rc;
-            rc = launch_remap(r.src, r.dst, ATTWARP_U8, ATTWARP_LAYOUT_HWC, 1, C, r.H, r.W, r.Ho, r.Wo, r.map_x, r.map_y, st);
+                return launch_maps_from_mask(mask + (size_t)i * gh * gw, 1, gh, gw, r.H, r.W, r.Wo, r.Ho, *tp, partials,
+                                             w.part_bytes, mx, my, st);
+            return launch_maps_from_attention(host_att[i].att, ATTWARP_U8, 1, r.H, r.W, r.Wo, r.Ho, *tp, partials,
+                                              w.part_bytes, mx, my, nullptr, st);
+        });
+    char* dev_tables = ws + w.tables;
+    const RaggedAtt* dev_att = reinterpret_cast<const RaggedAtt*>(dev_tables);
+    const int2* dev_items = reinterpret_cast<const int2*>(dev_tables + w.item_at);
+    const int maps_launches = launches + (w.fused_items > 0) + (w.att_items > 0) + 1;
+    return ragged_stage5(l, n, C, st, maps_launches, [&]() -> int {
+        AW_CUDA(cudaMemcpyAsync(dev_tables, host_tables.data(), host_tables.size(), cudaMemcpyHostToDevice, st));
+        if (w.fused_items > 0) {
+            rc = launch_lanczos_marginals_ragged(dev_items, w.fused_items, dev_att,
+                                                 reinterpret_cast<const RaggedLanczos*>(dev_tables + w.lz), gw, w.smem,
+                                                 partials, st);
             if (rc != ATTWARP_OK) return rc;
         }
-        g_ragged_last_launches = launches + 3 * n;    // resizes + marginals, finish and resample per image
-        return ATTWARP_OK;
-    }
-    const bool quad = C == 3 && remap_quad_enabled();
-    RaggedQuadPlan plan;
-    RaggedImage* dev_sorted = dev_table + (n + 1);
-    rc = quad ? launch_remap_u8_quad_ragged_prepare(host.data(), n, dev_table, dev_sorted, &plan, st)
-              : launch_remap_u8_stream_ragged_prepare(host.data(), n, C, dev_table, st);
-    if (rc != ATTWARP_OK) return rc;
-    AW_CUDA(cudaMemcpyAsync(dev_tables, host_tables.data(), host_tables.size(), cudaMemcpyHostToDevice, st));
-    if (s.fused_items > 0) {
-        rc = launch_lanczos_marginals_ragged(dev_items, s.fused_items, dev_att,
-                                             reinterpret_cast<const RaggedLanczos*>(dev_tables + lz_off), gw, s.smem,
-                                             partials, st);
-        if (rc != ATTWARP_OK) return rc;
-        ++launches;
-    }
-    if (s.att_items > 0) {
-        rc = launch_marginals_ragged_u8_identity(dev_items + s.fused_items, s.att_items, dev_att, partials, st);
-        if (rc != ATTWARP_OK) return rc;
-        ++launches;
-    }
-    rc = launch_maps_from_partials_ragged(n, dev_table, dev_att, partials, max_h, max_w, *tp, st);
-    if (rc != ATTWARP_OK) return rc;
-    g_ragged_last_launches = launches + 1 + (quad ? ragged_quad_launches(plan) : 1);
-    return quad ? launch_remap_u8_quad_ragged_run(plan, dev_sorted, st)
-                : launch_remap_u8_stream_ragged_run(host.data(), n, C, dev_table, st);
+        if (w.att_items > 0) {
+            rc = launch_marginals_ragged_u8_identity(dev_items + w.fused_items, w.att_items, dev_att, partials, st);
+            if (rc != ATTWARP_OK) return rc;
+        }
+        return launch_maps_from_partials_ragged(n, l.dev, dev_att, partials, l.max_h, l.max_w, *tp, st);
+    });
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -813,10 +772,8 @@ int attwarp_encode_png(const attwarp_png_image* images, int n, void* workspace, 
     if (workspace == nullptr || workspace_bytes < need)
         return fail(ATTWARP_ERR_WORKSPACE, "encode_png: workspace too small (%zu < %zu)", workspace_bytes, need);
     cudaStream_t st = as_stream(stream);
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    AW_CUDA(cudaStreamIsCapturing(st, &cap));
-    if (cap != cudaStreamCaptureStatusNone)
-        return fail(ATTWARP_ERR_UNSUPPORTED, "encode_png: cannot be captured into a CUDA graph (host-side descriptor table)");
+    const int rc = refuse_graph_capture(st, "encode_png");
+    if (rc != ATTWARP_OK) return rc;
     return launch_encode_png(images, n, workspace, static_cast<uint8_t*>(out), offsets, st);
 }
 
@@ -860,16 +817,13 @@ int attwarp_decode_jpeg(const attwarp_jpeg_image* images, int n, void* workspace
     AW_REQUIRE(images && status_out, "decode_jpeg: NULL pointer");
     AW_REQUIRE(n > 0, "decode_jpeg: n must be positive (got %d)", n);
     static thread_local std::vector<aw::jpeg::Header> hs;
-    const int rc = jpeg_headers(images, n, hs);
+    int rc = jpeg_headers(images, n, hs);
     if (rc != ATTWARP_OK) return rc;
     const size_t need = jpeg_workspace_bytes_impl(hs.data(), n);
     if (workspace == nullptr || workspace_bytes < need)
         return fail(ATTWARP_ERR_WORKSPACE, "decode_jpeg: workspace too small (%zu < %zu)", workspace_bytes, need);
     cudaStream_t st = as_stream(stream);
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    AW_CUDA(cudaStreamIsCapturing(st, &cap));
-    if (cap != cudaStreamCaptureStatusNone)
-        return fail(ATTWARP_ERR_UNSUPPORTED, "decode_jpeg: cannot be captured into a CUDA graph (host-side descriptor table)");
+    if ((rc = refuse_graph_capture(st, "decode_jpeg")) != ATTWARP_OK) return rc;
     return launch_decode_jpeg(images, hs.data(), n, workspace, status_out, st);
 }
 
@@ -912,11 +866,8 @@ int attwarp_attention_overlay(const attwarp_overlay_image* images, int n, int at
     if (workspace == nullptr || workspace_bytes < need)
         return fail(ATTWARP_ERR_WORKSPACE, "attention_overlay: workspace too small (%zu < %zu)", workspace_bytes, need);
     cudaStream_t st = as_stream(stream);
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    AW_CUDA(cudaStreamIsCapturing(st, &cap));
-    if (cap != cudaStreamCaptureStatusNone)
-        return fail(ATTWARP_ERR_UNSUPPORTED,
-                    "attention_overlay: cannot be captured into a CUDA graph (host-side descriptor table)");
+    const int rc = refuse_graph_capture(st, "attention_overlay");
+    if (rc != ATTWARP_OK) return rc;
     return launch_attention_overlay(images, n, att_dtype, att_kind, gh, gw, alpha, workspace, st);
 }
 

@@ -422,6 +422,48 @@ def warp_from_pdfs(img: torch.Tensor, px: torch.Tensor, py: torch.Tensor, alpha:
 # --------------------------------------------------------------------------------------------
 # ragged batches (mixed resolutions, BASELINE configs[3])
 # --------------------------------------------------------------------------------------------
+def _ragged_list(name, images, out_sizes, outs, anchor):
+    """The list of a ragged call: the images made contiguous, the outputs (allocated when ``outs`` is None), the output
+    sizes as ints -- default the input sizes -- and the descriptor table (attwarp_ragged_image [n]) of them all.  Every
+    image must be a uint8 [H, W, C] tensor with one C on ``anchor``'s device, every output a contiguous uint8
+    [Ho, Wo, C] tensor there.  The library writes each image through its table row at that row's size, and NumPy
+    broadcasts a one-element list into every row, so lists of the wrong length are refused before anything else."""
+    n = len(images)
+    if out_sizes is not None and len(out_sizes) != n:
+        raise ValueError(f"{name}: {len(out_sizes)} output sizes for {n} images")
+    if outs is not None and len(outs) != n:
+        raise ValueError(f"{name}: {len(outs)} outputs for {n} images")
+    require_cuda(anchor, *images)
+    dev, index = anchor.device, anchor.get_device()      # get_device(): no torch.device built per tensor
+    imgs = [im.contiguous() for im in images]
+    Cc = imgs[0].shape[2] if imgs[0].dim() == 3 else 0
+    for im in imgs:
+        if im.dtype != torch.uint8 or im.dim() != 3 or im.shape[2] != Cc or im.get_device() != index:
+            raise ValueError(f"{name}: images must be uint8 HWC tensors with the same channel count on one device, got "
+                             f"{im.dtype} {tuple(im.shape)} on {im.device} (expected C={Cc} on {dev})")
+    if out_sizes is None:
+        out_sizes = [(im.shape[0], im.shape[1]) for im in imgs]
+    else:
+        out_sizes = [(int(ho), int(wo)) for ho, wo in out_sizes]
+    if outs is None:
+        outs = [torch.empty(ho, wo, Cc, dtype=torch.uint8, device=dev) for ho, wo in out_sizes]
+    else:
+        outs = list(outs)
+        for k, (o, (ho, wo)) in enumerate(zip(outs, out_sizes)):
+            if o.dtype != torch.uint8 or o.shape != (ho, wo, Cc) or not o.is_contiguous() or o.get_device() != index:
+                raise ValueError(f"{name}: outputs must be contiguous [Ho, Wo, C] uint8 tensors on {dev}: output {k} "
+                                 f"is {o.dtype} {tuple(o.shape)} on {o.device}, expected {(ho, wo, Cc)}")
+    # one structured array (a ctypes struct per image costs ~3 us each)
+    table = np.empty(n, dtype=_RAGGED_DTYPE)
+    table["src"] = [im.data_ptr() for im in imgs]
+    table["dst"] = [o.data_ptr() for o in outs]
+    table["H"] = [im.shape[0] for im in imgs]
+    table["W"] = [im.shape[1] for im in imgs]
+    table["Ho"] = [hw[0] for hw in out_sizes]
+    table["Wo"] = [hw[1] for hw in out_sizes]
+    return imgs, outs, out_sizes, table
+
+
 def warp_ragged_from_tokens(tok: torch.Tensor, images, out_sizes=None, grid_hw=None,
                             transform="identity", exp_scale=1.0, exp_divisor=1.0,
                             apply_inverse=False, outs=None):
@@ -438,38 +480,19 @@ def warp_ragged_from_tokens(tok: torch.Tensor, images, out_sizes=None, grid_hw=N
         raise ValueError(f"warp_ragged_from_tokens: {tok.shape[0]} token maps for {n} images")
     if n == 0:                      # the reference's per-image loop over an empty list does nothing
         return []
+    imgs, outs, _, table = _ragged_list("warp_ragged_from_tokens", images, out_sizes, outs, tok)
+    dev = tok.device
     if tok.dim() == 3:
         gh, gw = tok.shape[1], tok.shape[2]
     else:
         gh, gw = grid_hw
     tok = tok.reshape(n, gh * gw).to(torch.float32).contiguous()
-    require_cuda(tok, *images)
-    dev = tok.device
-    Cc = images[0].shape[2]
-    imgs = [im.contiguous() for im in images]
-    if out_sizes is None:
-        out_sizes = [(im.shape[0], im.shape[1]) for im in imgs]
-    if outs is None:
-        outs = [torch.empty(ho, wo, Cc, dtype=torch.uint8, device=dev) for ho, wo in out_sizes]
-    # descriptor table as one structured array (a ctypes struct per image costs ~3 us each)
-    table = np.empty(n, dtype=_RAGGED_DTYPE)
-    table["src"] = [im.data_ptr() for im in imgs]
-    table["dst"] = [o.data_ptr() for o in outs]
-    table["H"] = [im.shape[0] for im in imgs]
-    table["W"] = [im.shape[1] for im in imgs]
-    table["Ho"] = [hw[0] for hw in out_sizes]
-    table["Wo"] = [hw[1] for hw in out_sizes]
-    for im, o, (ho, wo) in zip(imgs, outs, out_sizes):
-        if (im.dtype != torch.uint8 or im.dim() != 3 or im.shape[2] != Cc or im.device != dev
-                or o.dtype != torch.uint8 or tuple(o.shape) != (ho, wo, Cc) or not o.is_contiguous()):
-            raise ValueError("warp_ragged_from_tokens: images must be uint8 HWC tensors with the same channel "
-                             "count on one device, outputs contiguous [Ho, Wo, C]")
     table_p = table.ctypes.data_as(C.c_void_p)           # `table` stays alive until the call returns
     tp = _tp(transform, exp_scale, exp_divisor, apply_inverse)
     wsb = lib.attwarp_ragged_workspace_bytes(table_p, n)
     ws = _workspace(wsb, dev)
     with torch.cuda.device(dev):
-        check(lib.attwarp_warp_ragged_from_tokens(ptr(tok), n, gh, gw, table_p, Cc, C.byref(tp),
+        check(lib.attwarp_warp_ragged_from_tokens(ptr(tok), n, gh, gw, table_p, imgs[0].shape[2], C.byref(tp),
                                                   ptr(ws), ws.numel(), current_stream(dev)))
     return outs
 
@@ -500,14 +523,14 @@ def warp_ragged_from_attention(att, images, out_sizes=None, transform="identity"
         raise ValueError(f"warp_ragged_from_attention: {len(att)} attention maps for {n} images")
     if n == 0:
         return ([], [], []) if return_maps else []
-    require_cuda(*images)
-    dev = images[0].device
-    Cc = images[0].shape[2] if images[0].dim() == 3 else 0
+    imgs, outs, out_sizes, table = _ragged_list("warp_ragged_from_attention", images, out_sizes, outs, images[0])
+    dev = imgs[0].device
+    Cc = imgs[0].shape[2]
     if Cc not in (1, 3, 4):
         raise ValueError(f"warp_ragged_from_attention: images must be uint8 [H, W, C] with C in (1, 3, 4), got "
-                         f"{tuple(images[0].shape)}")
+                         f"{tuple(imgs[0].shape)}")
     maps = []
-    for k, (a, im) in enumerate(zip(att, images)):
+    for k, (a, im) in enumerate(zip(att, imgs)):
         if not isinstance(a, torch.Tensor):
             raise ValueError(f"warp_ragged_from_attention: attention map {k} is a {type(a).__name__}, not a tensor")
         if a.dim() != 2:
@@ -518,39 +541,19 @@ def warp_ragged_from_attention(att, images, out_sizes=None, transform="identity"
         if a.device != dev:
             raise ValueError(f"warp_ragged_from_attention: attention map {k} is on {a.device}, image 0 on {dev}: all "
                              "tensors must be on one CUDA device")
-        if im.dim() != 3 or tuple(a.shape) != tuple(im.shape[:2]):
+        if tuple(a.shape) != tuple(im.shape[:2]):
             raise ValueError(f"warp_ragged_from_attention: attention map {k} is {tuple(a.shape)}, image {k} is "
                              f"{tuple(im.shape[:2])}: the map must have its image's size")
         maps.append(a if a.is_contiguous() else a.contiguous())
     if len({a.dtype for a in maps}) > 1:
         raise ValueError("warp_ragged_from_attention: all attention maps must have one dtype, got "
                          f"{sorted({str(a.dtype) for a in maps})}")
-    imgs = [im.contiguous() for im in images]
-    if out_sizes is None:
-        out_sizes = [(im.shape[0], im.shape[1]) for im in imgs]
-    if len(out_sizes) != n:
-        raise ValueError(f"warp_ragged_from_attention: {len(out_sizes)} output sizes for {n} images")
-    if outs is None:
-        outs = [torch.empty(ho, wo, Cc, dtype=torch.uint8, device=dev) for ho, wo in out_sizes]
-    for im, o, (ho, wo) in zip(imgs, outs, out_sizes):
-        if (im.dtype != torch.uint8 or im.shape[2] != Cc or im.device != dev
-                or o.dtype != torch.uint8 or tuple(o.shape) != (ho, wo, Cc) or not o.is_contiguous()
-                or o.device != dev):
-            raise ValueError("warp_ragged_from_attention: images must be uint8 HWC tensors with the same channel "
-                             "count on one device, outputs contiguous [Ho, Wo, C]")
-    table = np.empty(n, dtype=_RAGGED_DTYPE)
-    table["src"] = [im.data_ptr() for im in imgs]
-    table["dst"] = [o.data_ptr() for o in outs]
-    table["H"] = [im.shape[0] for im in imgs]
-    table["W"] = [im.shape[1] for im in imgs]
-    table["Ho"] = [hw[0] for hw in out_sizes]
-    table["Wo"] = [hw[1] for hw in out_sizes]
     atab = np.zeros(n, dtype=_RAGGED_ATT_DTYPE)
     atab["att"] = [a.data_ptr() for a in maps]
     map_xs = map_ys = None
     if return_maps:
-        map_xs = [torch.empty(int(wo), dtype=torch.float32, device=dev) for _, wo in out_sizes]
-        map_ys = [torch.empty(int(ho), dtype=torch.float32, device=dev) for ho, _ in out_sizes]
+        map_xs = [torch.empty(wo, dtype=torch.float32, device=dev) for _, wo in out_sizes]
+        map_ys = [torch.empty(ho, dtype=torch.float32, device=dev) for ho, _ in out_sizes]
         atab["map_x"] = [m.data_ptr() for m in map_xs]
         atab["map_y"] = [m.data_ptr() for m in map_ys]
     table_p = table.ctypes.data_as(C.c_void_p)           # the tables stay alive until the call returns
@@ -585,31 +588,14 @@ def warp_ragged_from_mota_tokens(tok: torch.Tensor, images, out_sizes=None, kern
         raise ValueError(f"warp_ragged_from_mota_tokens: {tok.shape[0]} token maps for {n} images")
     if n == 0:
         return ([], [], []) if return_maps else []
-    require_cuda(tok, *images)
+    imgs, outs, out_sizes, table = _ragged_list("warp_ragged_from_mota_tokens", images, out_sizes, None, tok)
     dev = tok.device
-    Cc = images[0].shape[2] if images[0].dim() == 3 else 0
+    Cc = imgs[0].shape[2]
     if Cc not in (1, 3, 4):
         raise ValueError(f"warp_ragged_from_mota_tokens: images must be uint8 [H, W, C] with C in (1, 3, 4), got "
-                         f"{tuple(images[0].shape)}")
-    imgs = [im.contiguous() for im in images]
-    if out_sizes is None:
-        out_sizes = [(im.shape[0], im.shape[1]) for im in imgs]
-    if len(out_sizes) != n:
-        raise ValueError(f"warp_ragged_from_mota_tokens: {len(out_sizes)} output sizes for {n} images")
-    outs = [torch.empty(int(ho), int(wo), Cc, dtype=torch.uint8, device=dev) for ho, wo in out_sizes]
-    for im in imgs:
-        if im.dtype != torch.uint8 or im.dim() != 3 or im.shape[2] != Cc or im.device != dev:
-            raise ValueError("warp_ragged_from_mota_tokens: images must be uint8 HWC tensors with the same channel "
-                             "count on the token maps' device")
+                         f"{tuple(imgs[0].shape)}")
     _, u8 = revise_mask(tok, kernel_size, enhance_coe, return_u8=True)
     gh, gw = int(u8.shape[1]), int(u8.shape[2])
-    table = np.empty(n, dtype=_RAGGED_DTYPE)
-    table["src"] = [im.data_ptr() for im in imgs]
-    table["dst"] = [o.data_ptr() for o in outs]
-    table["H"] = [im.shape[0] for im in imgs]
-    table["W"] = [im.shape[1] for im in imgs]
-    table["Ho"] = [hw[0] for hw in out_sizes]
-    table["Wo"] = [hw[1] for hw in out_sizes]
     map_x = map_y = None
     if return_maps:
         map_x = torch.empty(int(table["Wo"].sum()), dtype=torch.float32, device=dev)
@@ -623,7 +609,7 @@ def warp_ragged_from_mota_tokens(tok: torch.Tensor, images, out_sizes=None, kern
                                                 ptr(map_x), ptr(map_y), current_stream(dev)))
     if not return_maps:
         return outs
-    return (outs, list(map_x.split([int(w) for w in table["Wo"]])), list(map_y.split([int(h) for h in table["Ho"]])))
+    return (outs, list(map_x.split([wo for _, wo in out_sizes])), list(map_y.split([ho for ho, _ in out_sizes])))
 
 
 class RaggedBatch:
@@ -640,29 +626,9 @@ class RaggedBatch:
         lib = load()
         n = len(images)
         assert n > 0
-        require_cuda(*images)
-        self.device = images[0].device
-        self.C = int(images[0].shape[2])
-        self.images = [im.contiguous() for im in images]
-        if out_sizes is None:
-            out_sizes = [(im.shape[0], im.shape[1]) for im in self.images]
-        self.out_sizes = [(int(h), int(w)) for h, w in out_sizes]
-        if outs is None:
-            outs = [torch.empty(ho, wo, self.C, dtype=torch.uint8, device=self.device) for ho, wo in self.out_sizes]
-        self.outs = list(outs)
-        for im, o, (ho, wo) in zip(self.images, self.outs, self.out_sizes):
-            if (im.dtype != torch.uint8 or im.dim() != 3 or im.shape[2] != self.C or im.device != self.device
-                    or o.dtype != torch.uint8 or tuple(o.shape) != (ho, wo, self.C) or not o.is_contiguous()
-                    or o.device != self.device):
-                raise ValueError("RaggedBatch: images must be uint8 HWC tensors with the same channel count on one "
-                                 "device, outputs contiguous [Ho, Wo, C]")
-        table = np.empty(n, dtype=_RAGGED_DTYPE)
-        table["src"] = [im.data_ptr() for im in self.images]
-        table["dst"] = [o.data_ptr() for o in self.outs]
-        table["H"] = [im.shape[0] for im in self.images]
-        table["W"] = [im.shape[1] for im in self.images]
-        table["Ho"] = [hw[0] for hw in self.out_sizes]
-        table["Wo"] = [hw[1] for hw in self.out_sizes]
+        self.images, self.outs, self.out_sizes, table = _ragged_list("RaggedBatch", images, out_sizes, outs, images[0])
+        self.device = self.images[0].device
+        self.C = int(self.images[0].shape[2])
         self._table = table
         self._table_p = table.ctypes.data_as(C.c_void_p)
         self.n = n

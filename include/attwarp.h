@@ -231,7 +231,7 @@ int attwarp_warp_from_pdfs(const float* px, const float* py, int B, int Nx, int 
  * tok       : device [n][gh*gw] float32 token maps (stage-1 output), index-upsampled to each
  *             image's H x W exactly like attwarp_maps_from_tokens
  * workspace : attwarp_ragged_workspace_bytes(images, n) bytes of device scratch (descriptor table
- *             + the per-image map rows)
+ *             + the per-image map rows; 0: invalid sizes)
  * The call uploads its descriptor tables from host memory and fans the stage-5 launches out over internal streams;
  * it returns ATTWARP_ERR_UNSUPPORTED on a stream that is being captured into a CUDA graph.
  */
