@@ -86,6 +86,9 @@ SIGNATURES = {
     "attwarp_jpeg_probe": (_i, [_vp, _sz, _vp]),
     "attwarp_jpeg_workspace_bytes": (_sz, [_vp, _i]),
     "attwarp_decode_jpeg": (_i, [_vp, _i, _vp, _sz, _vp, _vp]),
+    "attwarp_png_probe": (_i, [_vp, _sz, _vp]),
+    "attwarp_png_decode_workspace_bytes": (_sz, [_vp, _i]),
+    "attwarp_decode_png": (_i, [_vp, _i, _vp, _sz, _vp, _vp]),
     "attwarp_overlay_workspace_bytes": (_sz, [_vp, _i, _i]),
     "attwarp_attention_overlay": (_i, [_vp, _i, _i, _i, _i, _i, C.c_double, _vp, _sz, _vp]),
     "attwarp_warp_image_host":(_i, [_vp, _i, _i, _i, _i, _vp, _i, _i, _i, _tp, _vp,

@@ -10,6 +10,7 @@
 
 #include "common.cuh"
 #include "jpeg_decode.h"
+#include "png_inflate.h"
 
 namespace aw {
 
@@ -46,6 +47,9 @@ int launch_encode_png(const attwarp_png_image* images, int n, void* ws, uint8_t*
 size_t jpeg_workspace_bytes_impl(const jpeg::Header* headers, int n);
 int launch_decode_jpeg(const attwarp_jpeg_image* images, const jpeg::Header* headers, int n, void* ws,
                        int32_t* status, cudaStream_t st);
+size_t png_decode_workspace_bytes_impl(const png::Header* hs, int n);
+int launch_decode_png(const attwarp_png_file* files, const png::Header* hs, int n, void* ws, int32_t* status,
+                      cudaStream_t st);
 int launch_interp_linear_rows(const float* F, int B, int N, int L, float* out, cudaStream_t st);
 size_t overlay_workspace_bytes_impl(const attwarp_overlay_image* images, int n, int att_kind);
 int launch_attention_overlay(const attwarp_overlay_image* images, int n, int att_dtype, int att_kind, int gh, int gw,
@@ -825,6 +829,57 @@ int attwarp_decode_jpeg(const attwarp_jpeg_image* images, int n, void* workspace
     cudaStream_t st = as_stream(stream);
     if ((rc = refuse_graph_capture(st, "decode_jpeg")) != ATTWARP_OK) return rc;
     return launch_decode_jpeg(images, hs.data(), n, workspace, status_out, st);
+}
+
+// ---------------------------------------------------------------------------------------------
+int attwarp_png_probe(const void* bytes, size_t nbytes, attwarp_png_info* info) {
+    AW_REQUIRE(bytes && info, "png_probe: NULL pointer");
+    aw::png::Header h;
+    aw::png::parse_png(static_cast<const uint8_t*>(bytes), nbytes, &h, [](uint32_t, uint32_t) {});
+    info->H = h.H;
+    info->W = h.W;
+    info->colour_type = h.colour;
+    info->bit_depth = h.depth;
+    info->support = h.support;
+    return ATTWARP_OK;
+}
+
+// the headers of `files`, parsed into a per-thread vector; ATTWARP_OK when every file is device-decodable
+static int png_headers(const attwarp_png_file* files, int n, std::vector<aw::png::Header>& hs) {
+    hs.resize((size_t)n);
+    for (int i = 0; i < n; ++i) {
+        const attwarp_png_file& f = files[i];
+        AW_REQUIRE(f.host && f.dev && f.dst, "decode_png: file %d: NULL pointer", i);
+        aw::png::Header& h = hs[(size_t)i];
+        const int s = aw::png::parse_png(static_cast<const uint8_t*>(f.host), f.nbytes, &h, [](uint32_t, uint32_t) {});
+        if (s != aw::png::kPngOk)
+            return fail(ATTWARP_ERR_UNSUPPORTED, "decode_png: file %d is not device-decodable (support code %d)", i, s);
+        AW_REQUIRE(f.H == h.H && f.W == h.W, "decode_png: file %d: dst is %d x %d, the file is %d x %d", i, f.H, f.W,
+                   h.H, h.W);
+    }
+    return ATTWARP_OK;
+}
+
+size_t attwarp_png_decode_workspace_bytes(const attwarp_png_file* files, int n) {
+    if (files == nullptr || n <= 0) return 0;
+    static thread_local std::vector<aw::png::Header> hs;
+    if (png_headers(files, n, hs) != ATTWARP_OK) return 0;
+    return png_decode_workspace_bytes_impl(hs.data(), n);
+}
+
+int attwarp_decode_png(const attwarp_png_file* files, int n, void* workspace, size_t workspace_bytes,
+                       int32_t* status_out, void* stream) {
+    AW_REQUIRE(files && status_out, "decode_png: NULL pointer");
+    AW_REQUIRE(n > 0, "decode_png: n must be positive (got %d)", n);
+    static thread_local std::vector<aw::png::Header> hs;
+    int rc = png_headers(files, n, hs);
+    if (rc != ATTWARP_OK) return rc;
+    const size_t need = png_decode_workspace_bytes_impl(hs.data(), n);
+    if (workspace == nullptr || workspace_bytes < need)
+        return fail(ATTWARP_ERR_WORKSPACE, "decode_png: workspace too small (%zu < %zu)", workspace_bytes, need);
+    cudaStream_t st = as_stream(stream);
+    if ((rc = refuse_graph_capture(st, "decode_png")) != ATTWARP_OK) return rc;
+    return launch_decode_png(files, hs.data(), n, workspace, status_out, st);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -27,7 +27,7 @@ constexpr int kSegThreads = 256;
 constexpr int kAsmThreads = 256;
 constexpr int kFileOverhead = 8 + 25 + 14 + 16 + 12;   // signature, IHDR, zlib header chunk, Adler chunk, IEND
 constexpr int kChunkOverhead = 12;             // length, type, CRC
-constexpr uint32_t kAdlerMod = 65521;
+using png::kAdlerMod;
 
 // one image of the batch (device table; entry n is a sentinel whose seg_begin is the total segment count)
 struct PngImage {
@@ -385,8 +385,7 @@ png_assemble_kernel(const PngImage* __restrict__ imgs, int n, const PngSegment* 
             uint32_t aa = s_adler_a, bb = s_adler_b;
             for (int k = base; k < min(base + nt, se); ++k) {
                 const PngSegment& r = res[k];
-                bb = (uint32_t)(((uint64_t)bb + (uint64_t)aa * r.len + r.adler_b) % kAdlerMod);
-                aa = (aa + r.adler_a) % kAdlerMod;
+                png::adler_combine(aa, bb, r.adler_a, r.adler_b, r.len);
             }
             s_adler_a = aa;
             s_adler_b = bb;

@@ -267,6 +267,16 @@ AW_PNG_HD void rle_tokens(const uint8_t* buf, int n, int a, int b, int prev_brea
     }
 }
 
+// ---- Adler-32 ---------------------------------------------------------------------------------------------------
+constexpr uint32_t kAdlerMod = 65521;
+
+// Folds a piece of `len` bytes into the running Adler-32 sums (a, b) (a starts at 1, b at 0): seg_a = sum of its
+// bytes b_k, seg_b = sum of (len - k) b_k, both mod 65521.
+AW_PNG_HD void adler_combine(uint32_t& a, uint32_t& b, uint32_t seg_a, uint32_t seg_b, uint32_t len) {
+    b = (uint32_t)(((uint64_t)b + (uint64_t)a * len + seg_b) % kAdlerMod);
+    a = (a + seg_a) % kAdlerMod;
+}
+
 // ---- CRC-32 (ISO-HDLC, reflected polynomial 0xEDB88320) -------------------------------------------------------------
 constexpr uint32_t kCrcPoly = 0xEDB88320u;
 

@@ -23,6 +23,14 @@ batches the rest:
   12-bit, CMYK / YCCK / RGB, multi-scan, ...) go to Pillow and other formats to cv2, both exact; ``ops.jpeg_probe``
   tells which path a file takes.  A file whose entropy-coded data is malformed raises ValueError naming it (Pillow
   would recover from some such files with a warning; the device decoder never guesses pixels).
+  PNGs go the same way under ``exact_device=True``: the ones ``ops.png_probe`` accepts (not interlaced; 8-bit
+  grey / RGB / palette / grey + alpha / RGBA, 1/2/4-bit grey and palette) are decoded on the GPU in one
+  ``ops.decode_png`` call (csrc/png_decode.cu: one launch for the whole mixed-size list, the inflate of each file
+  split across a CTA), giving the pixels cv2.imdecode and Pillow give them; they accept and reject the malformed
+  files libpng does (bad IDAT CRC, Adler-32, truncated stream, too few rows, a filter type above 4 rejected; a bad
+  ancillary CRC, extra rows, bytes after the stream accepted).  Other PNGs stay with cv2.  Known gap: for 16-bit
+  grey files cv2 (which decodes them on that path) shifts samples right by 8 where Pillow's ``convert('RGB')``
+  clips them to 255, so under ``exact_device=True`` those files are not Pillow's pixels (DESIGN.md section 6 item 9).
 * ``encode_png_batch(images, paths)`` device tensors -> PNG files: device -> pinned host copy, then
   ``cv2.imwrite`` in a thread pool -- the reference's own encoder, so the files decode to the same bytes.
   ``on_device=True`` encodes on the GPU instead (``encode_png_device``, ``ops.encode_png``: two launches for the
@@ -69,6 +77,10 @@ def _is_jpeg(buf: bytes) -> bool:
     return len(buf) > 3 and buf[0] == 0xFF and buf[1] == 0xD8
 
 
+def _is_png(buf: bytes) -> bool:
+    return buf[:8] == b"\x89PNG\r\n\x1a\n"
+
+
 def _pillow_bgr(b: bytes, dev) -> torch.Tensor:
     import io
 
@@ -83,8 +95,9 @@ def decode_jpeg_batch(sources: Sequence, device=None, exact: bool = False,
     one ``save_warped_image`` warps in).  JPEG files are decoded on the GPU in one batched nvJPEG call; grey JPEGs
     come out as three equal channels (like ``Image.convert('RGB')``).  ``exact=True``: host decode with Pillow,
     bit-identical to the reference's reader, then one copy to the device.  ``exact_device=True``: bit-identical too,
-    with the JPEGs ``ops.jpeg_probe`` accepts decoded on the GPU in one ``ops.decode_jpeg`` call; other JPEGs
-    (progressive, CMYK, ...) are decoded by Pillow and other formats by cv2, as without the keyword."""
+    with the JPEGs ``ops.jpeg_probe`` accepts decoded on the GPU in one ``ops.decode_jpeg`` call and the PNGs
+    ``ops.png_probe`` accepts in one ``ops.decode_png`` call; other JPEGs (progressive, CMYK, ...) are decoded by
+    Pillow and other files (16-bit or interlaced PNGs, ...) by cv2, as without the keyword."""
     if exact and exact_device:
         raise ValueError("decode_jpeg_batch: exact and exact_device are exclusive")
     dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
@@ -103,6 +116,14 @@ def decode_jpeg_batch(sources: Sequence, device=None, exact: bool = False,
         for i in jpegs:
             if out[i] is None:
                 out[i] = _pillow_bgr(bufs[i], dev)
+        png_idx = [i for i, b in enumerate(bufs) if _is_png(b) and ops.png_probe(b)[4] == 0]
+        if png_idx:
+            try:
+                decoded = ops.decode_png([bufs[i] for i in png_idx], dev)
+            except ops.PngDecodeError as exc:
+                raise ValueError(f"decode_jpeg_batch: source {png_idx[exc.file]} {exc.reason}") from exc
+            for i, t in zip(png_idx, decoded):
+                out[i] = t
         return _decode_others(bufs, out, dev)
     from torchvision.io import ImageReadMode, decode_jpeg
     jpeg_idx = [i for i, b in enumerate(bufs) if _is_jpeg(b)]

@@ -787,6 +787,87 @@ def decode_jpeg(buffers, device=None):
 
 
 # --------------------------------------------------------------------------------------------
+# PNG decode, pixel for pixel as Pillow's convert('RGB')
+# --------------------------------------------------------------------------------------------
+# attwarp_png_info / attwarp_png_file (include/attwarp.h)
+_PNG_INFO_DTYPE = np.dtype([("H", np.int32), ("W", np.int32), ("colour_type", np.int32), ("bit_depth", np.int32),
+                            ("support", np.int32)])
+_PNG_FILE_DTYPE = _JPEG_DTYPE
+PNG_SUPPORT_REASONS = {1: "not a PNG file", 2: "truncated", 3: "16-bit samples", 4: "interlaced",
+                       5: "bad CRC on a critical chunk", 6: "chunk structure, IHDR or zlib header", 7: "size"}
+PNG_STATUS_REASONS = {1: "invalid deflate block type", 2: "invalid Huffman code", 3: "distance too far back",
+                      4: "stored block length mismatch", 5: "zlib stream ends early", 6: "Adler-32 mismatch",
+                      7: "IDAT CRC mismatch", 8: "invalid filter type", 9: "too little image data"}
+
+
+class PngDecodeError(ValueError):
+    """A file ``decode_png`` refuses: ``file`` is its index in the call's list, ``reason`` what is wrong with it."""
+
+    def __init__(self, file: int, reason: str):
+        super().__init__(f"decode_png: file {file} {reason}")
+        self.file, self.reason = file, reason
+
+
+def png_probe(buf) -> tuple:
+    """(H, W, colour_type, bit_depth, support) of a file's bytes from its chunks, on the host (no GPU).  support 0:
+    the file is one ``decode_png`` takes; otherwise a key of ``PNG_SUPPORT_REASONS``."""
+    data = np.frombuffer(bytes(buf), dtype=np.uint8)
+    info = np.zeros(1, dtype=_PNG_INFO_DTYPE)
+    check(load().attwarp_png_probe(data.ctypes.data_as(C.c_void_p), data.size, info.ctypes.data_as(C.c_void_p)))
+    return tuple(int(info[0][k]) for k in ("H", "W", "colour_type", "bit_depth", "support"))
+
+
+def decode_png(buffers, device=None):
+    """PNG files (a sequence of bytes-like objects) -> list of uint8 [H, W, 3] **BGR** CUDA tensors, equal to
+    ``np.array(Image.open(f).convert('RGB'))[..., ::-1]``.  The whole list is decoded on the GPU in one launch:
+    only the file bytes are copied to the device (one copy from pinned memory).
+
+    Raises ``PngDecodeError`` (a ValueError) naming the first file ``png_probe`` does not accept (see
+    include/attwarp.h for the subset), and, after one synchronisation that reads the per-file status, the first
+    malformed file (no pixels of such a file are returned)."""
+    lib = load()
+    dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    bufs = [bytes(b) for b in buffers]
+    n = len(bufs)
+    if n == 0:
+        return []
+    infos = [png_probe(b) for b in bufs]
+    for i, info in enumerate(infos):
+        sup = info[4]
+        if sup != 0:
+            raise PngDecodeError(i, f"is not device-decodable: {PNG_SUPPORT_REASONS.get(sup, sup)} "
+                                    f"(support code {sup})")
+    sizes = [len(b) for b in bufs]
+    offs = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
+    host = torch.empty(int(offs[-1]), dtype=torch.uint8, pin_memory=True)
+    hv = host.numpy()
+    for b, o in zip(bufs, offs[:-1]):
+        hv[o:o + len(b)] = np.frombuffer(b, dtype=np.uint8)
+    with torch.cuda.device(dev):
+        data = host.to(dev, non_blocking=True)
+        outs = [torch.empty((info[0], info[1], 3), dtype=torch.uint8, device=dev) for info in infos]
+        status = torch.empty(n, dtype=torch.int32, device=dev)
+        table = np.zeros(n, dtype=_PNG_FILE_DTYPE)
+        table["host"] = host.data_ptr() + offs[:-1]
+        table["dev"] = data.data_ptr() + offs[:-1]
+        table["nbytes"] = sizes
+        table["dst"] = [t.data_ptr() for t in outs]
+        table["H"] = [info[0] for info in infos]
+        table["W"] = [info[1] for info in infos]
+        table_p = table.ctypes.data_as(C.c_void_p)
+        wsb = lib.attwarp_png_decode_workspace_bytes(table_p, n)
+        ws = _workspace(wsb, dev)
+        check(lib.attwarp_decode_png(table_p, n, ptr(ws), ws.numel(), ptr(status), current_stream(dev)))
+        st = status.cpu().numpy()                      # synchronises: the decode (and the upload) have run
+    bad = np.nonzero(st)[0]
+    if bad.size:
+        i = int(bad[0])
+        raise PngDecodeError(i, f"is malformed: {PNG_STATUS_REASONS.get(int(st[i]), int(st[i]))} "
+                                f"(status {int(st[i])})")
+    return outs
+
+
+# --------------------------------------------------------------------------------------------
 # Attention overlay (save_warped_image's masked_overlay_save_path image)
 # --------------------------------------------------------------------------------------------
 # attwarp_overlay_image (include/attwarp.h)

@@ -458,6 +458,78 @@ size_t attwarp_jpeg_workspace_bytes(const attwarp_jpeg_image* images_host, int n
 int attwarp_decode_jpeg(const attwarp_jpeg_image* images_host, int n, void* workspace, size_t workspace_bytes,
                         int32_t* status_out, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * PNG decode of n files of any sizes in one launch, pixel for pixel as Image.open(path).convert('RGB')
+ * gives them (the reference drivers' reader), in cv2.imread's BGR order: alpha dropped, grey replicated
+ * to three channels, 1/2/4-bit grey scaled by 255/85/17, palette indices past the end of PLTE black.
+ *
+ * Device-decodable files (attwarp_png_probe's support code ATTWARP_PNG_OK): not interlaced; bit depth 8
+ * for colour types 0 (grey), 2 (RGB), 3 (palette), 4 (grey + alpha), 6 (RGBA), bit depths 1, 2, 4 for
+ * types 0 and 3; any number of consecutive IDAT chunks (empty ones too); a zlib stream without a preset
+ * dictionary, with any window size and any stored, fixed or dynamic blocks.  The CRCs of IHDR, PLTE and
+ * IEND are checked by the probe, those of the IDAT chunks and the stream's Adler-32 by the decode;
+ * ancillary chunks are skipped unchecked, and the bytes after the zlib stream and the inflated bytes
+ * after the last row are ignored, as libpng does.
+ *
+ * attwarp_png_probe: host only, no GPU.  Walks the chunks of bytes[0 .. nbytes) and fills *info.
+ *   Returns ATTWARP_ERR_INVALID_ARG for NULL pointers, else ATTWARP_OK whatever the support code.
+ * attwarp_png_decode_workspace_bytes: device scratch one call over `files` needs (the files' gathered
+ *   streams and inflated rows, a fixed scratch per CTA, the descriptor and chunk tables); 0 when a file
+ *   is not device-decodable or a pointer is NULL.
+ * attwarp_decode_png:
+ *   files      HOST array of n descriptors: host and dev both hold the file's nbytes bytes (the host
+ *              copy is parsed during the call, the device copy is read by the kernel); dst is a
+ *              DEVICE [H][W][3] uint8 buffer at any byte alignment, H and W the file's.  dev and dst
+ *              must stay valid until the stream has run the call.
+ *   status_out DEVICE int32 [n]: per file ATTWARP_PNG_ST_OK or the reason it is malformed.  The dst of
+ *              a failed file is left untouched; no pixel of it is guessed.
+ *   Argument errors (NULL, n <= 0, a size mismatch, a file that is not device-decodable: message names
+ *   the file) return before any CUDA call.  The call uploads its descriptor table from host memory:
+ *   ATTWARP_ERR_UNSUPPORTED on a stream that is being captured into a CUDA graph.
+ */
+typedef enum attwarp_png_support {
+    ATTWARP_PNG_OK = 0,
+    ATTWARP_PNG_NOT_PNG = 1,          /* no PNG signature                                         */
+    ATTWARP_PNG_TRUNCATED = 2,        /* the file ends inside a chunk or before IEND              */
+    ATTWARP_PNG_BIT_DEPTH = 3,        /* 16-bit samples                                            */
+    ATTWARP_PNG_INTERLACED = 4,       /* Adam7                                                    */
+    ATTWARP_PNG_BAD_CRITICAL = 5,     /* a bad CRC on IHDR, PLTE or IEND                          */
+    ATTWARP_PNG_STRUCTURE = 6,        /* invalid IHDR, missing or misplaced PLTE, IDAT chunks not
+                                         consecutive, unknown critical chunk, zlib header (method,
+                                         window, check bits, preset dictionary)                   */
+    ATTWARP_PNG_SIZE = 7              /* a side above 10^6 or 2^31 inflated bytes or more         */
+} attwarp_png_support;
+
+typedef enum attwarp_png_status {
+    ATTWARP_PNG_ST_OK = 0,
+    ATTWARP_PNG_ST_BLOCK_TYPE = 1,    /* deflate block type 3                                     */
+    ATTWARP_PNG_ST_BAD_CODE = 2,      /* an invalid Huffman code, code-length header or symbol    */
+    ATTWARP_PNG_ST_DISTANCE = 3,      /* a distance back past the start of the stream             */
+    ATTWARP_PNG_ST_STORED_LEN = 4,    /* a stored block whose LEN and NLEN disagree               */
+    ATTWARP_PNG_ST_SHORT_STREAM = 5,  /* the IDAT data ends before the zlib stream does           */
+    ATTWARP_PNG_ST_ADLER = 6,         /* Adler-32 mismatch                                        */
+    ATTWARP_PNG_ST_IDAT_CRC = 7,      /* an IDAT chunk's CRC-32 mismatch                          */
+    ATTWARP_PNG_ST_FILTER = 8,        /* a row filter type above 4                                */
+    ATTWARP_PNG_ST_SHORT_IMAGE = 9    /* the stream holds fewer bytes than the rows need          */
+} attwarp_png_status;
+
+typedef struct attwarp_png_info {
+    int32_t H, W, colour_type, bit_depth, support;
+} attwarp_png_info;
+
+typedef struct attwarp_png_file {      /* attwarp_png_image is the encoder's descriptor */
+    const void* host;
+    const void* dev;
+    size_t nbytes;
+    void* dst;
+    int32_t H, W;
+} attwarp_png_file;
+
+int attwarp_png_probe(const void* bytes, size_t nbytes, attwarp_png_info* info);
+size_t attwarp_png_decode_workspace_bytes(const attwarp_png_file* files_host, int n);
+int attwarp_decode_png(const attwarp_png_file* files_host, int n, void* workspace, size_t workspace_bytes,
+                       int32_t* status_out, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Stages 2-3, torch path (all float32 [B][N] row-major unless noted).
  */
